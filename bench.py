@@ -7,6 +7,7 @@ One *step* = the work of one `Solver_CCSD.SCF` iteration body (Solver_GS.py:683-
 
     python bench.py --gpus N --steps K --warmup W          # this repo's CUDA path
     python bench.py --impl reference --gpus N ...          # the reference algorithm on host cores
+    python bench.py ... --dump-outputs DIR                 # also write the last timed step's results to DIR/*.npy
 
 Prints ONE JSON line.  `value` = steps/s with everything resident in HBM; `e2e` = the same through
 the reference-facing API (`GCC.gamma/energy/tupdate/lupdate`) with HOST (pinned numpy) buffers,
@@ -492,6 +493,31 @@ def np_copy(x):
     return np.array(x, copy=True)
 
 
+DUMP_SAMPLE = 1 << 21          # elements kept of an output larger than this: 16 MB in float64
+DUMP_MAX_BYTES = 64 << 20
+DUMP_SEED = 20261020
+
+
+def dump_outputs(path, outs):
+    """Write {name: device tensor} as path/<name>.npy in float64.  An output with more than DUMP_SAMPLE elements is
+    stored as the flat elements at a fixed, seeded set of sorted indices (the same for every run at the same shape),
+    so that two builds can be compared output for output; smaller ones are stored whole, in their own shape."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    total = 0
+    for name, t in outs.items():
+        t = t.detach()
+        if t.numel() > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(DUMP_SEED).choice(t.numel(), size=DUMP_SAMPLE, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        a = t.cpu().numpy().astype(np.float64)
+        total += a.nbytes
+        if total > DUMP_MAX_BYTES:
+            raise RuntimeError("--dump-outputs: more than %d bytes" % DUMP_MAX_BYTES)
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -555,8 +581,12 @@ def run_ours(args):
     if rank == 0:
         sampler.start()
     lib.ecw_profile_enable(de._h, 0)
-    ms_dev, _ = timed(step_dev, args.steps, args.warmup)
+    ms_dev, last = timed(step_dev, args.steps, args.warmup)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(zip(("gamma", "energy", "tupdate_t1", "tupdate_t2", "lupdate_l1",
+                                                  "lupdate_l2"), last)))
+    del last
 
     # ---- the functions of one evaluation on their own, and the updates with the L1 term (extra key "parts")
     try:
@@ -793,7 +823,14 @@ def main():
     ap.add_argument("--config5", action="store_true", help="add the sharded (60,800) vvvv ladder as extra key config5 (default: at 8 GPUs)")
     ap.add_argument("--gemm", default=None, choices=["int8", "dmma"], help="GEMM engine (default: int8)")
     ap.add_argument("--int8-digits", type=int, default=None, help="base-256 digits of the INT8 engine (default: from the integral magnitudes, 6 for the benchmark)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (rdm1, energy, T1/T2 and L1/L2 updates) as DIR/<name>.npy, "
+                         "float64; outputs above %d elements as a fixed seeded sample of it (64 MB at most in all)" % DUMP_SAMPLE)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps this repo's path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,7 +1,8 @@
-"""Load the UNMODIFIED reference modules from /root/reference behind the pyscf
-stub.  TEST INFRASTRUCTURE ONLY (used by oracle/make_golden.py and by the
-`not gpu` tests that pin the numpy restatement); it is unavailable on the GPU
-box, where only the committed fixtures under tests/golden/ are used.
+"""Load the UNMODIFIED reference modules from a checkout of the reference (directory
+ECW_REFERENCE_DIR) behind the pyscf stub.  Used by the oracle/make_golden*.py
+scripts that write the fixtures under tests/golden/ (and by __graft_entry__.build()
+as an import check when a checkout is present); the tests read those fixtures and
+need no reference checkout.
 """
 import importlib
 import os

@@ -4,8 +4,8 @@
             Vexp[0,0] = L (rdm1_exp - rdm1), Delta = sum|diff| / sum|rdm1_exp|, vmax = max|diff|.
 `scf_loop`: Solver_GS.Solver_CCSD.SCF (Solver_GS.py:621-742), DIIS through oracle/pyscf_stub's restatement of
             pyscf.lib.diis, for any object with the GCC method surface.
-Pinned against the unmodified reference by tests/test_oracle_pins_solver.py (live reference in the build container,
-tests/golden/solver_ccsd_*.npz everywhere).
+Pinned against the unmodified reference's runs stored in tests/golden/solver_ccsd_*.npz by
+tests/test_oracle_pins_solver.py.
 """
 import numpy as np
 

@@ -68,3 +68,21 @@ def test_cpu_leg_is_a_measurement_with_the_extrapolation_labelled(monkeypatch):
     assert ss["shape"] == [16, 96] and ss["cpu_evals_s"] == 0.05 and ss["gpu_e2e_evals_s"] == 50.0 and ss["ratio"] == 1000.0
     assert cb["extrapolated_evals_per_sec_at_bench_shape"] < 1e-3 * cb["value"] and "NOT a measurement" in cb["extrapolation"]
     assert [x["shape"] for x in cb["same_shape_all"]] == [[10, 48], [16, 96]]
+
+
+def test_dump_outputs_fixed_sample(tmp_path, monkeypatch):
+    """--dump-outputs: small outputs whole, large ones as the same seeded sample every run, float64 .npy files."""
+    import numpy as np
+    import torch
+    import bench
+    monkeypatch.setattr(bench, "DUMP_SAMPLE", 100)
+    big = torch.arange(1000, dtype=torch.float64).reshape(10, 10, 10)
+    outs = {"gamma": torch.ones(5, 5, dtype=torch.float64), "energy": torch.tensor(-1.5, dtype=torch.float64), "t2": big}
+    bench.dump_outputs(str(tmp_path / "a"), outs)
+    bench.dump_outputs(str(tmp_path / "b"), outs)
+    for name in outs:
+        a, b = np.load(tmp_path / "a" / (name + ".npy")), np.load(tmp_path / "b" / (name + ".npy"))
+        assert a.dtype == np.float64 and np.array_equal(a, b)
+    t2 = np.load(tmp_path / "a" / "t2.npy")
+    assert t2.shape == (100,) and np.all(np.diff(t2) > 0)          # distinct sorted flat indices of arange
+    assert np.load(tmp_path / "a" / "energy.npy") == -1.5 and np.load(tmp_path / "a" / "gamma.npy").shape == (5, 5)

@@ -5,7 +5,6 @@ import numpy as np
 import pytest
 
 from helpers import load_golden
-from oracle import ref_loader
 from oracle.make_golden_exp import CALLS, run
 from oracle.make_golden_h2o import H2O
 
@@ -48,23 +47,6 @@ def test_exp_matches_reference_for_every_target(water):
         assert want.shape == got.shape, k
         assert np.abs(want - got).max() <= 1e-11 * max(1.0, np.abs(want).max()), k
     assert len(CALLS) == 7 and float(g["w_11_Delta"]) > 0
-
-
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present (GPU box)")
-def test_exp_matches_live_reference(water):
-    from ecw_cc_b200 import exp_pot, utilities
-    mol, er = water
-    ref_exp, ref_util = ref_loader.load("exp_pot", "utilities")
-    a = run(ref_exp.Exp, mol, er.mo_coeff_g, ref_util)
-    b = run(exp_pot.Exp, mol, er.mo_coeff_g, utilities)
-    for k in a:
-        assert np.abs(np.asarray(a[k], dtype=float) - np.asarray(b[k], dtype=float)).max() <= 1e-11 * max(
-            1.0, np.abs(np.asarray(a[k], dtype=float)).max()), k
-    # helpers of the excited-state solver
-    for nst, kidx in (([2, 0], [0, 2]), ([1, 1], None), ([3, 2], [0, 1, 0, 0, 1])):
-        x = ref_util.koopman_init_guess(er.mo_energy, er.mo_occ, nst, koop_idx=kidx)
-        y = utilities.koopman_init_guess(er.mo_energy, er.mo_occ, nst, koop_idx=kidx)
-        assert all(np.array_equal(p, q) for p, q in zip(x[0], y[0])) and list(x[1]) == list(y[1])
 
 
 def test_errors():

@@ -1,24 +1,20 @@
-"""Pin the CPU oracle: against the golden vectors produced by the reference
-itself (always), and against the live reference + its raw-equation second
-implementation when /root/reference is present (build container only)."""
+"""Pin the CPU oracle against the golden vectors produced by the unmodified reference
+(oracle/make_golden.py), including its raw-equation second implementation."""
 import numpy as np
 import pytest
 
 from helpers import load_golden, MODES
-from oracle import synth, ref_loader
+from oracle import synth
 from oracle.ccsd_np import OracleGCC, soft_threshold
 from oracle import refactored_np as R
 
 TOL = 1e-13
 
 
-@pytest.mark.parametrize("name", ["ccsd_o4v6.npz", "ccsd_o5v8.npz"])
-def test_oracle_matches_golden(name):
-    g = load_golden(name)
+def _assert_matches_golden(cc, g):
+    """tupdate / lupdate in every mode with both Fock matrices, energy and rdm1 of `cc` against the golden `g`."""
     o, v = int(g["nocc"]), int(g["nvir"])
-    er = synth.SynthEris(o, v)
     t1, t2, l1, l2 = synth.amplitudes(o, v)
-    cc = OracleGCC(er)
     for fname, fsp in (("sym", synth.fsp(o, v)), ("ns", g["fsp_ns"])):
         for tag, alpha, eq in MODES:
             a, b = cc.tupdate(t1, t2, fsp=fsp, alpha=alpha, equation=eq)
@@ -29,6 +25,15 @@ def test_oracle_matches_golden(name):
             assert np.abs(b - g["L2_%s_%s" % (fname, tag)]).max() < TOL
         assert abs(cc.energy(t1, t2, fsp) - float(g["E_%s" % fname])) < TOL
     assert np.abs(cc.gamma(t1, t2, l1, l2) - g["gamma"]).max() < TOL
+
+
+@pytest.mark.parametrize("name", ["ccsd_o4v6.npz", "ccsd_o5v8.npz"])
+def test_oracle_matches_golden(name):
+    g = load_golden(name)
+    o, v = int(g["nocc"]), int(g["nvir"])
+    t1, t2, l1, l2 = synth.amplitudes(o, v)
+    cc = OracleGCC(synth.SynthEris(o, v))
+    _assert_matches_golden(cc, g)
     # identity the reference itself checks (CCSD.py:675-699): factorised == raw equations
     a, b = cc.tupdate(t1, t2, equation=True)
     assert np.abs(a - g["rawT1"]).max() < 1e-12 and np.abs(b - g["rawT2"]).max() < 1e-12
@@ -77,27 +82,8 @@ def test_quirks():
     assert abs(np.trace(g) - o) < 1e-12 and np.abs(g - g.T).max() < 1e-15
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present (GPU box)")
-@pytest.mark.parametrize("ov", [(4, 6), (6, 9)])
-def test_oracle_matches_live_reference(ov):
-    o, v = ov
-    CCSD, U, RAW = ref_loader.load("CCSD", "utilities", "CC_raw_equations")
-    er = synth.SynthEris(o, v)
-    t1, t2, l1, l2 = synth.amplitudes(o, v)
-    fsp = synth.fsp(o, v)
-    ref, orc, orf = CCSD.GCC(er), OracleGCC(er), OracleGCC(er, faithful=True)
-    for tag, alpha, eq in MODES:
-        for cc in (orc, orf):
-            a, b = ref.tupdate(t1, t2, fsp=fsp, alpha=alpha, equation=eq)
-            c, d = cc.tupdate(t1, t2, fsp=fsp, alpha=alpha, equation=eq)
-            assert np.abs(a - c).max() < TOL and np.abs(b - d).max() < TOL
-            a, b = ref.lupdate(t1, t2, l1, l2, fsp=fsp, alpha=alpha, equation=eq)
-            c, d = cc.lupdate(t1, t2, l1, l2, fsp=fsp, alpha=alpha, equation=eq)
-            assert np.abs(a - c).max() < TOL and np.abs(b - d).max() < TOL
-    assert np.abs(ref.gamma(t1, t2, l1, l2) - orc.gamma(t1, t2, l1, l2)).max() < TOL
-    assert abs(ref.energy(t1, t2, fsp) - orc.energy(t1, t2, fsp)) < TOL
-    rng = np.random.default_rng(0)
-    e, var = rng.standard_normal((7, 5)), rng.standard_normal((7, 5))
-    var[0] = 0.0
-    for al in (0.0, 1e-3, 0.5):
-        assert np.array_equal(U.subdiff(e, var, al), soft_threshold(e, var, al))
+@pytest.mark.parametrize("name", ["ccsd_o4v6.npz", "ccsd_o5v8.npz"])
+def test_faithful_oracle_matches_golden(name):
+    """The oracle with the reference's own einsum routing (`faithful=True`, what bench.py's CPU leg times)."""
+    g = load_golden(name)
+    _assert_matches_golden(OracleGCC(synth.SynthEris(int(g["nocc"]), int(g["nvir"])), faithful=True), g)

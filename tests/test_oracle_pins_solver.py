@@ -1,19 +1,20 @@
-"""Pins of the solver-loop restatement (oracle/solver_np.py) and of the converged-state fixtures: against the live
-unmodified reference when /root/reference exists, against tests/golden/solver_ccsd_*.npz (made by
-oracle/make_golden_solver.py from the unmodified reference solver + CCSD.GCC + exp_pot.Exp) always."""
+"""Pins of the solver-loop restatement (oracle/solver_np.py) and of the converged-state fixtures against
+tests/golden/solver_ccsd_*.npz (made by oracle/make_golden_solver.py from the unmodified reference solver + CCSD.GCC +
+exp_pot.Exp)."""
 import numpy as np
 import pytest
 
 from helpers import load_golden
-from oracle import ref_loader, synth
+from oracle import synth
 from oracle.ccsd_np import OracleGCC
 from oracle.make_golden_solver import CASES, target_rdm1
 from oracle.solver_np import ExpMat, scf_loop
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")
-def test_expmat_matches_reference_exp_pot():
-    exp_pot = ref_loader.load("exp_pot")
+def test_expmat_matches_product_exp_pot():
+    """The oracle's 'mat' target against the product's ecw_cc_b200.exp_pot.Exp (same constructor as the reference's
+    exp_pot.Exp, pinned to the reference's outputs by tests/test_exp_pot_cpu.py)."""
+    import ecw_cc_b200.exp_pot as exp_pot
     rng = np.random.default_rng(3)
     n = 10
     target = rng.standard_normal((n, n))
@@ -22,15 +23,14 @@ def test_expmat_matches_reference_exp_pot():
         rdm1 = rng.standard_normal((n, n))
         a, b = ref.Vexp_update(rdm1, rdm1, (0, 0), L=L), mine.Vexp_update(rdm1, rdm1, (0, 0), L=L)
         assert a == b and np.array_equal(ref.Vexp[0, 0], mine.Vexp[0, 0])
-        # the product-side mirror (ecw_cc_b200.exp_pot.Exp, same constructor as the reference)
-        import ecw_cc_b200.exp_pot as mirror
+        # with the Hartree-Fock property given (Delta is then relative to target - HF), and with L changed by the call
         for hf in (False, [[0.5 * target]]):
-            r2 = exp_pot.Exp(L, [[["mat", target]]], None, None, HF_prop=hf)
-            m2 = mirror.Exp(L, [[["mat", target]]], None, None, HF_prop=hf)
-            assert r2.Vexp_update(rdm1, rdm1, (0, 0)) == m2.Vexp_update(rdm1, rdm1, (0, 0))
-            assert np.array_equal(r2.Vexp[0, 0], m2.Vexp[0, 0]) and r2.L == m2.L
-            assert r2.Vexp_update(rdm1, rdm1, (0, 0), L=2 * L + 0.1) == m2.Vexp_update(rdm1, rdm1, (0, 0), L=2 * L + 0.1)
-            assert np.array_equal(r2.Vexp[0, 0], m2.Vexp[0, 0])
+            r2, m2 = exp_pot.Exp(L, [[["mat", target]]], None, None, HF_prop=hf), ExpMat(L, target)
+            scale = np.sum(abs(target)) / np.sum(abs(target - hf[0][0])) if hf else 1.0
+            for Lc in (None, 2 * L + 0.1):
+                (d, vmax), (d0, vmax0) = r2.Vexp_update(rdm1, rdm1, (0, 0), L=Lc), m2.Vexp_update(rdm1, rdm1, (0, 0), L=Lc)
+                assert vmax == vmax0 and (d == d0 if not hf else abs(d - d0 * scale) <= 1e-15 * d)
+                assert np.array_equal(r2.Vexp[0, 0], m2.Vexp[0, 0]) and r2.L == [[L]]
 
 
 @pytest.mark.parametrize("name", ["solver_ccsd_o4v6.npz", "solver_ccsd_o8v16.npz"])
