@@ -5,8 +5,8 @@ import subprocess
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libecw_b200.so")
-_SRC = ["gemm.cu", "gemm_tma.cu", "ewise.cu", "ozaki.cu", "synth.cu", "capi.cu", "plan.cpp", "ccsd_plan.cpp", "ccsd_plan_slab.cpp",
-        "ccs_plan.cpp"]
+_SRC = ["gemm.cu", "gemm_tma.cu", "ewise.cu", "ozaki.cu", "synth.cu", "ftao.cu", "capi.cu", "plan.cpp", "ccsd_plan.cpp",
+        "ccsd_plan_slab.cpp", "ccs_plan.cpp"]
 
 ECW_HAS_ALPHA = 1
 ECW_EQUATION = 2
@@ -133,6 +133,9 @@ class _Lib(object):
             "ecw_op_workspace_needed": (c_l, [c_p]),
             "ecw_conv_check": (c_i, [c_p, c_p, c_p, c_p, c_l, c_p, c_p, c_i, c_p]),
             "ecw_vexp_mat": (c_i, [c_p, c_p, c_p, c_d, c_p, c_p, c_p, c_l, c_p]),
+            "ecw_ft_aopair": (c_i, [c_p, c_l, c_p, c_i, c_p, c_l, c_p, c_p]),
+            "ecw_vexp_sf": (c_i, [c_p, c_i, c_p, c_i, c_p, c_l, c_p, c_d, c_p, c_p, c_p, c_p, c_p, c_p, c_p]),
+            "ecw_vexp_sf_workspace_bytes": (c_l, [c_i, c_i, c_l]),
             "ecw_profile_enable": (c_i, [c_p, c_i]),
             "ecw_profile_dump": (c_l, [c_p, c_p, c_l]),
         }

@@ -1152,6 +1152,76 @@ int ecw_vexp_mat(const double* rdm1, const double* target, const double* fock, d
   });
 }
 
+int ecw_ft_aopair(const double* prim, int64_t nprim, const int64_t* ao_first, int nao, const double* G, int64_t nG,
+                  double* out, void* stream) {
+  return guarded(nullptr, [&] {
+    require_device();
+    if (!prim || !ao_first || !G || !out) throw Fail("ecw_ft_aopair: null pointer");
+    if (nprim < 1 || nao < 1 || nG < 1) throw Fail("ecw_ft_aopair: empty primitive table, basis or G list");
+    ck(launch_ft_aopair(prim, nprim, ao_first, nao, G, nG, out, static_cast<cudaStream_t>(stream)), "ft_aopair");
+  });
+}
+
+namespace {
+// ecw_vexp_sf workspace: X / Y [2nao, n] | D [nao, nao] | coef [2 nG] | V_AO [nao, nao], each padded to 32 doubles
+struct SfWorkspace {
+  int64_t x, d, coef, v, total;
+  SfWorkspace(int n, int nao, int64_t nG) {
+    auto pad = [](int64_t e) { return (e + 31) / 32 * 32; };
+    x = 0;
+    d = x + pad(2LL * nao * n);
+    coef = d + pad((int64_t)nao * nao);
+    v = coef + pad(2 * nG);
+    total = v + pad((int64_t)nao * nao);
+  }
+};
+}  // namespace
+
+int64_t ecw_vexp_sf_workspace_bytes(int n, int nao, int64_t nG) {
+  if (n < 1 || nao < 1 || nG < 1) return -1;
+  return 8 * SfWorkspace(n, nao, nG).total;
+}
+
+int ecw_vexp_sf(const double* rdm1, int n, const double* mo_coeff_g, int nao, const double* ft, int64_t nG,
+                const double* F_exp, double L, const double* fock, double* vexp, double* fsp, double* F_calc,
+                double* stats2, double* workspace, void* stream) {
+  return guarded(nullptr, [&] {
+    require_device();
+    if (!rdm1 || !mo_coeff_g || !ft || !F_exp || !fock || !vexp || !fsp || !F_calc || !stats2 || !workspace)
+      throw Fail("ecw_vexp_sf: null pointer");
+    if (n < 1 || nao < 1 || nG < 1) throw Fail("ecw_vexp_sf: empty rdm1, basis or reflection list");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const SfWorkspace w(n, nao, nG);
+    double* X = workspace + w.x;                 // C_g gamma, later blockdiag(V, V) C_g
+    double* D = workspace + w.d;
+    double* coef = workspace + w.coef;
+    double* V = workspace + w.v;
+    const int64_t n2 = (int64_t)nao * nao;
+    const double* Ca = mo_coeff_g;               // alpha rows of C_g
+    const double* Cb = mo_coeff_g + (int64_t)nao * n;
+    auto gemm = [&](int ta, int tb, int64_t M, int64_t N, int64_t K, const double* A, int64_t lda, const double* B,
+                    int64_t ldb, double beta, double* C, int64_t ldc) {
+      GemmArgs g{};
+      g.A = A; g.B = B; g.C = C; g.M = M; g.N = N; g.K = K; g.lda = lda; g.ldb = ldb; g.ldc = ldc;
+      g.batch = 1; g.splitk = 1; g.kchunk = K; g.ta = ta; g.tb = tb; g.alpha = 1.0; g.beta = beta;
+      ck(launch_gemm(g, st), "vexp_sf gemm");
+    };
+    // D = C_a gamma C_a^T + C_b gamma C_b^T: the spin-summed AO density
+    gemm(0, 0, 2LL * nao, n, n, mo_coeff_g, n, rdm1, n, 0.0, X, n);
+    gemm(0, 1, nao, nao, n, X, n, Ca, n, 0.0, D, nao);
+    gemm(0, 1, nao, nao, n, X + (int64_t)nao * n, n, Cb, n, 1.0, D, nao);
+    // F_calc [Re | Im] = planes [2 nG, nao^2] . vec(D)
+    gemm(0, 0, 2 * nG, 1, n2, ft, n2, D, 1, 0.0, F_calc, 1);
+    ck(launch_sf_coef(F_exp, F_calc, L, coef, stats2, nG, st), "vexp_sf coef");
+    // V_AO = planes^T . coef,  vexp = C_g^T blockdiag(V_AO, V_AO) C_g
+    gemm(1, 0, n2, 1, 2 * nG, ft, n2, coef, 1, 0.0, V, 1);
+    gemm(0, 0, nao, n, nao, V, nao, Ca, n, 0.0, X, n);
+    gemm(0, 0, nao, n, nao, V, nao, Cb, n, 0.0, X + (int64_t)nao * n, n);
+    gemm(1, 0, n, n, 2LL * nao, mo_coeff_g, n, X, n, 0.0, vexp, n);
+    ck(launch_sf_finish(vexp, fock, fsp, stats2, (int64_t)n * n, st), "vexp_sf finish");
+  });
+}
+
 int ecw_profile_enable(ecw_ctx* c, int on) {
   if (!c) return -1;
   c->profile = on != 0;

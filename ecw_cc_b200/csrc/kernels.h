@@ -128,6 +128,17 @@ cudaError_t launch_subdiff(const double* e, const double* v, double alpha, doubl
 // conv = |a| + |b| (b null: a); scal = beta*scal + sum (conv - prev)^2 (prev null: + 0); partial: nblocks doubles
 cudaError_t launch_vexp_mat(const double* rdm1, const double* target, const double* fock, double L, double* vexp,
                             double* fsp, double* stats, int64_t n, cudaStream_t st);
+// structure-factor target (ftao.cu).  prim [nprim, 8] = {Ax, Ay, Az, alpha, coef, lx, ly, lz} per primitive Cartesian
+// Gaussian (l <= 2 per direction), the primitives of AO mu at rows ao_first[mu] .. ao_first[mu+1]-1; G [nG, 3] in
+// bohr^-1; out [2][nG][nao][nao] = Re and Im planes of int phi_mu phi_nu exp(+i G.r)
+cudaError_t launch_ft_aopair(const double* prim, int64_t nprim, const int64_t* ao_first, int nao, const double* G,
+                             int64_t nG, double* out, cudaStream_t st);
+// coef [2][nG] = L (F_exp - F_calc) (Re, Im planes), stats[0] = sum_h |F_exp(h) - F_calc(h)|
+cudaError_t launch_sf_coef(const double* F_exp, const double* F_calc, double L, double* coef, double* stats, int64_t nG,
+                           cudaStream_t st);
+// fsp = fock - vexp, stats[1] = max |vexp|
+cudaError_t launch_sf_finish(const double* vexp, const double* fock, double* fsp, double* stats, int64_t n2,
+                             cudaStream_t st);
 cudaError_t launch_conv(const double* a, const double* b, const double* prev, double* conv, int64_t n, double* partial,
                         int nblocks, double* scal, double beta, cudaStream_t st);
 cudaError_t launch_dot(const double* a, const double* b, int64_t n, double* partial, int nblocks, double* scal,

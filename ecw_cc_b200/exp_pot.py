@@ -3,31 +3,43 @@ dress the Fock matrix of the ECW fit, their relative deviations Delta, and the w
 
 Targets (exp_pot.py:131-345): 'mat' (ground or excited state rdm1), 'trmat' (left/right transition rdm1), 'Ek', 'v1e',
 'dip' (state properties), 'DEk..' (kinetic-energy difference to the ground state, acts on Vexp[0, 0]) and 'trdip'
-(squared transition dipole, acts on Vexp[0, n] / Vexp[n, 0]).  The structure-factor target 'F' needs Fourier-transformed
-AO pairs (PySCF `ft_ao`) and is not provided.  Property targets take their AO integrals from `mol`, which may be a PySCF
-`Mole` or `ecw_cc_b200.molint.Molecule` (same `intor_symmetric` / `with_common_orig` / `atom_charges` / `atom_coords`).
+(squared transition dipole, acts on Vexp[0, n] / Vexp[n, 0]) and 'F' (X-ray structure factors, any diagonal state).
+Property targets take their AO integrals from `mol`, which may be a PySCF `Mole` or `ecw_cc_b200.molint.Molecule` (same
+`intor_symmetric` / `with_common_orig` / `atom_charges` / `atom_coords`); 'F' needs a `molint.Molecule`.
 
-Scope: only the 'mat' ground-state target is part of the product (SURVEY §8 f-2; `mat_update_device`, `ecw_vexp_mat`).
+'F' = ['F', F_exp, hkl, cell]: N_h structure factors (complex, or real = phase 0), integer Miller indices [N_h, 3] and
+orthorhombic cell lengths (a, b, c) in Angstrom; G_h = 2 pi (h/a, k/b, l/c).  The reference's own 'F' branch needs PySCF
+and is not pinned; the target is defined by the penalty it minimises, P = (w/2) sum_h |F_exp(h) - F_calc(h)|^2 with
+F_calc(h) = sum_mu,nu D_mu,nu A_mu,nu(G_h), A = `molint.ft_aopair` (exp(+i G.r)), D = C_g rdm1 C_g^T spin-summed.  The
+potential is -dP/drdm1 = w sum_h Re[conj(dF_h) C_g^T blockdiag(A_h, A_h) C_g]: on purpose NOT the `convert_aoint`
+convention (C^-1 A C^-T, |diff|) of the other property targets, since there is no reference behaviour to mirror and the
+fit needs the true gradient.  Delta = sum_h |dF_h| / sum_h |F_exp(h)| (HF_prop: / sum_h |F_exp - F_HF|), vmax =
+max |V_F|, and ['F', F_calc] goes to `prop_calc`.
+
+Scope: the 'mat' ground-state target is part of the product (SURVEY §8 f-2; `mat_update_device`, `ecw_vexp_mat`),
+and so is the 'F' ground-state target (`sf_update_device`, `ecw_ft_aopair`, `ecw_vexp_sf`).
 The other targets are n x n host code kept as test HARNESS (callers of the path, SURVEY §2 "out of scope"): they let the
 excited-state configuration of BASELINE.json be driven on a box without PySCF, and are pinned to the reference class
 in tests/test_exp_pot_cpu.py.
 
 n x n work on the host, except for the case `Main.CCSD_GS` runs — one density-matrix target for the ground state —
-which `mat_update_device` evaluates on the GPU (`ecw_vexp_mat`): the device-resident solver (`ecw_cc_b200.Solver_CCSD`)
+which `mat_update_device` evaluates on the GPU (`ecw_vexp_mat`), and one structure-factor target for the ground state,
+which `sf_update_device` evaluates there (`ecw_ft_aopair` builds the AO-pair planes once, `ecw_vexp_sf` forms the
+potential per iteration): the device-resident solver (`ecw_cc_b200.Solver_CCSD`)
 then moves only scalars per iteration; for every other target it sends the rdm1 (n x n) to the host once per iteration
 and takes the dressed Fock back (3 MB of PCIe traffic per iteration at (40,400)).
 """
 import numpy as np
 
-from . import utilities
+from . import molint, utilities
 
 
 class Exp(object):
     def __init__(self, L, exp_data, mol=None, mo_coeff=None, Ek_exp_GS=None, Ek_HF_GS=None, HF_prop=False):
         """Same signature as the reference (exp_pot.py:11).  exp_data = [[GS targets], [ES1 targets], ...], a target
         being ['mat', rdm1], ['trmat', (left, right)], ['Ek', x], ['v1e', x], ['dip', [x, y, z]], ['trdip', [x, y, z]],
-        ['DEk..', x]; mo_coeff in spin-orbital (G) format; HF_prop in the layout of exp_data switches Delta to the
-        deviation relative to |exp - HF|."""
+        ['DEk..', x], ['F', F_exp, hkl, cell]; mo_coeff in spin-orbital (G) format; HF_prop in the layout of exp_data
+        switches Delta to the deviation relative to |exp - HF|."""
         self.nbr_states = len(exp_data)
         self.exp_data = exp_data
         self.mol, self.mo_coeff = mol, mo_coeff
@@ -39,11 +51,13 @@ class Exp(object):
         self.Ek_int = self.dip_int = self.v1e_int = self.F_int = None
         self.dic_int = {}
         self.prop_names = []
-        for st in exp_data:
-            for prop in st:
+        self.sf = {}                                                # 'F' data per (state, target index)
+        for k, st in enumerate(exp_data):
+            for i, prop in enumerate(st):
                 name = prop[0]
                 if name == 'F':
-                    raise NotImplementedError("the structure-factor target 'F' needs PySCF's ft_ao")
+                    self.sf[k, i] = self._sf_setup(prop, mol, mo_coeff, self.HF_prop[k][i])
+                    continue
                 if name not in ('mat', 'trmat') and mol is None:
                     raise ValueError("target %r needs AO integrals: pass mol (PySCF Mole or molint.Molecule)" % (name,))
                 if 'dip' in name and self.dip_int is None:          # 'dip' and 'trdip' (exp_pot.py:90-98)
@@ -67,6 +81,34 @@ class Exp(object):
         self.Ek_calc_GS = None
         self.Delta_Ek_GS = None
         self.Vexp = np.full((self.nbr_states, self.nbr_states), None)
+
+    # -- the structure-factor target --------------------------------------------------------------------------------
+    def _sf_setup(self, prop, mol, mo_coeff, hf):
+        """Validate ['F', F_exp, hkl, cell] and derive the scattering vectors G_h = 2 pi (h/a, k/b, l/c) in bohr^-1.
+        The AO-pair transforms are built on first use: on the host by `Vexp_update`, on the device by
+        `sf_update_device`."""
+        if mol is None or not isinstance(mol, molint.Molecule):
+            raise NotImplementedError("the structure-factor target 'F' needs the AO pairs of an ecw_cc_b200.molint."
+                                      "Molecule" + ("" if mol is None else " (a PySCF Mole is not supported)"))
+        if len(prop) != 4:
+            raise ValueError("the structure-factor target is ['F', F_exp, hkl, cell]")
+        F_exp = np.asarray(prop[1])
+        if F_exp.ndim != 1 or F_exp.size == 0 or not np.issubdtype(F_exp.dtype, np.number) \
+                or not np.all(np.isfinite(F_exp)):
+            raise ValueError("'F' target: F_exp must be a non-empty 1-D array of finite (real or complex) values")
+        hkl = np.asarray(prop[2])
+        if hkl.shape != (F_exp.size, 3) or not np.issubdtype(hkl.dtype, np.number) or not np.all(np.isfinite(hkl)) \
+                or np.any(hkl != np.round(hkl)):
+            raise ValueError("'F' target: hkl must be an (N_h, 3) array of integer Miller indices, N_h = len(F_exp)")
+        cell = np.asarray(prop[3], dtype=np.float64)
+        if cell.shape != (3,) or not np.all(np.isfinite(cell)) or np.any(cell <= 0):
+            raise ValueError("'F' target: cell must be three positive orthorhombic cell lengths (a, b, c), Angstrom")
+        if mo_coeff is None or np.shape(mo_coeff)[0] != 2 * mol.nao:
+            raise ValueError("'F' target: mo_coeff in spin-orbital (G) format, [2 nao, n], is required")
+        F_exp = F_exp.astype(np.complex128)
+        G = 2 * np.pi * hkl.astype(np.float64) / cell / molint.ANGSTROM
+        ref = F_exp if hf is None else F_exp - np.asarray(hf, dtype=np.complex128)
+        return {"F_exp": F_exp, "G": G, "norm": float(np.sum(np.abs(ref))), "A": None}
 
     # -- weights (exp_pot.py:459-490) -------------------------------------------------------------------------------
     def L_check(self, L):
@@ -179,6 +221,21 @@ class Exp(object):
                     self.Vexp[n, m] += w * diff
                     vmax += np.max(np.abs(diff))
                 self.prop_calc.append([name, calc])
+            if name == 'F' and n == m:
+                sf = self.sf[st, i]
+                if sf["A"] is None:
+                    sf["A"] = molint.ft_aopair(self.mol, sf["G"])
+                A, C = sf["A"], self.mo_coeff
+                nao = A.shape[1]
+                D = utilities.convert_g_to_ru_rdm1(C @ rdm1 @ C.T)[0]
+                calc = np.einsum('hij,ij->h', A, D)
+                dF = sf["F_exp"] - calc
+                v_ao = w * np.einsum('h,hij->ij', np.conj(dF), A).real
+                diff = C[:nao].T @ v_ao @ C[:nao] + C[nao:].T @ v_ao @ C[nao:]
+                self.Vexp[n, n] += diff
+                Delta += np.sum(np.abs(dF)) / sf["norm"]
+                vmax += np.max(np.abs(diff))
+                self.prop_calc.append([name, calc])
         return Delta, vmax
 
     # -- the 'mat' ground-state target without leaving the GPU (SURVEY §8f-2) ------------------------------------------
@@ -219,8 +276,91 @@ class Exp(object):
         s = st["stats"].cpu()
         return float(s[0]) / st["norm"], float(s[1]), fsp
 
+    # -- the structure-factor ground-state target without leaving the GPU ---------------------------------------------
+    def device_sf_ready(self):
+        """True when Vexp[0, 0] is exactly one structure-factor target: then `sf_update_device` forms the potential and
+        the dressed Fock matrix on the device."""
+        return bool(self.prop_names) and self.prop_names[0] == ['F'] and self.Ek_exp_GS is None
+
+    def sf_update_device(self, rdm1_dev, fock_dev, L=None):
+        """Device version of `Vexp_update(rdm1, rdm1, (0, 0), L)` + `fsp = fock - Vexp[0, 0]` for one 'F' target through
+        `ecw_vexp_sf`: returns (Delta, vmax, fsp) with fsp a device tensor; only the two reduction results come to the
+        host.  The first call builds the AO-pair planes on the device (`ecw_ft_aopair`, 2 N_h nao^2 doubles) and
+        uploads mo_coeff; both stay there.  Afterwards `self.Vexp[0, 0]` holds the DEVICE potential and `prop_calc`
+        the device F_calc ([2, N_h]: Re, Im); `sync_host()` turns both into what the host path leaves there."""
+        import torch
+        from ._lib import lib, EcwError
+        if not self.device_sf_ready():
+            raise EcwError("sf_update_device needs a single 'F' ground-state target")
+        L = self.L if L is None else self.L_check(L)
+        dev = rdm1_dev.device
+        sf = self.sf[0, 0]
+        C = np.ascontiguousarray(self.mo_coeff, dtype=np.float64)
+        nao, n = C.shape[0] // 2, C.shape[1]
+        nG = len(sf["G"])
+        st = getattr(self, "_sf_dev", None)
+        if st is None or st["device"] != dev:
+            ws = lib.ecw_vexp_sf_workspace_bytes(n, nao, nG)
+            if ws < 0:
+                raise EcwError("ecw_vexp_sf_workspace_bytes failed")
+            fe = np.stack([sf["F_exp"].real, sf["F_exp"].imag])
+            st = {"device": dev, "ft": ft_aopair_device(self.mol, sf["G"], dev), "C": torch.from_numpy(C).to(dev),
+                  "F_exp": torch.from_numpy(np.ascontiguousarray(fe)).to(dev),
+                  "vexp": torch.empty((n, n), dtype=torch.float64, device=dev),
+                  "F_calc": torch.empty((2, nG), dtype=torch.float64, device=dev),
+                  "stats": torch.zeros(2, dtype=torch.float64, device=dev),
+                  "ws": torch.empty((ws + 7) // 8, dtype=torch.float64, device=dev)}
+            self._sf_dev = st
+        for x in (rdm1_dev, fock_dev):
+            if tuple(x.shape) != (n, n) or not x.is_contiguous() or x.dtype != torch.float64 or x.device != dev:
+                raise ValueError("rdm1 and fock must be contiguous float64 (n, n) matrices on one device, n = mo_coeff "
+                                 "columns")
+        fsp = torch.empty_like(rdm1_dev)
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        rc = lib.ecw_vexp_sf(rdm1_dev.data_ptr(), n, st["C"].data_ptr(), nao, st["ft"].data_ptr(), nG,
+                             st["F_exp"].data_ptr(), float(L[0][0]), fock_dev.data_ptr(), st["vexp"].data_ptr(),
+                             fsp.data_ptr(), st["F_calc"].data_ptr(), st["stats"].data_ptr(), st["ws"].data_ptr(),
+                             stream)
+        if rc != 0:
+            raise EcwError("ecw_vexp_sf failed")
+        self.Vexp[0, 0] = st["vexp"]
+        self.prop_calc = [['F', st["F_calc"]]]
+        s = st["stats"].cpu()
+        return float(s[0]) / sf["norm"], float(s[1]), fsp
+
     def sync_host(self):
-        """Replace a device-resident Vexp[0, 0] by its numpy copy."""
+        """Replace a device-resident Vexp[0, 0] (and a device F_calc in `prop_calc`) by numpy copies."""
         v = self.Vexp[0, 0]
         if v is not None and not isinstance(v, np.ndarray) and hasattr(v, "cpu"):
             self.Vexp[0, 0] = v.cpu().numpy()
+        for pc in self.prop_calc:
+            if pc[0] == 'F' and not isinstance(pc[1], np.ndarray) and hasattr(pc[1], "cpu"):
+                f = pc[1].cpu().numpy()
+                pc[1] = f[0] + 1j * f[1]
+
+
+def ft_aopair_device(mol, G, device):
+    """`molint.ft_aopair(mol, G)` on the GPU (`ecw_ft_aopair`): a float64 tensor [2, nG, nao, nao] holding the real
+    and imaginary planes.  G: [nG, 3] scattering vectors in bohr^-1."""
+    import torch
+    from ._lib import lib, EcwError
+    G = np.ascontiguousarray(np.atleast_2d(np.asarray(G, dtype=np.float64)))
+    if G.ndim != 2 or G.shape[1] != 3 or len(G) == 0:
+        raise ValueError("G must be a non-empty [nG, 3] array of scattering vectors")
+    ao = np.asarray(mol.ao)
+    if np.any(np.diff(ao) < 0) or ao[0] != 0 or ao[-1] != mol.nao - 1:
+        raise ValueError("the primitives of each AO must be contiguous (molint.Molecule.ao non-decreasing)")
+    if np.any(mol.lmn > 2) or np.any(mol.lmn < 0):
+        raise ValueError("ecw_ft_aopair takes Cartesian powers up to 2 per direction (s, p, d)")
+    if not torch.cuda.is_available():
+        raise EcwError("no CUDA device: ecw_ft_aopair has no CPU implementation (molint.ft_aopair is the host path)")
+    prim = np.ascontiguousarray(np.concatenate([mol.cen, mol.ex[:, None], mol.coef[:, None], mol.lmn], axis=1),
+                                dtype=np.float64)
+    ao_first = np.searchsorted(ao, np.arange(mol.nao + 1)).astype(np.int64)
+    t_prim, t_first, t_G = (torch.from_numpy(x).to(device) for x in (prim, ao_first, G))
+    out = torch.empty((2, len(G), mol.nao, mol.nao), dtype=torch.float64, device=device)
+    rc = lib.ecw_ft_aopair(t_prim.data_ptr(), len(prim), t_first.data_ptr(), mol.nao, t_G.data_ptr(), len(G),
+                           out.data_ptr(), torch.cuda.current_stream(out.device).cuda_stream)
+    if rc != 0:
+        raise EcwError("ecw_ft_aopair failed")
+    return out

@@ -368,6 +368,57 @@ def dipole_integrals(mol, origin=(0., 0., 0.)):
     return np.stack(out)
 
 
+def ft_aopair(mol, G):
+    """Fourier-transformed AO pairs A_mu,nu(G) = int phi_mu phi_nu exp(+i G.r) d^3r (crystallographic sign), complex
+    [nG, nao, nao], for scattering vectors G [nG, 3] in bohr^-1.  Symmetric in mu nu; A(0) is the overlap matrix.
+    One primitive pair (exponents a, b, p = a + b, centre P) contributes, exactly,
+        (pi/p)^(3/2) exp(-|G|^2/4p) exp(i G.P) prod_d sum_t E_t^(d) (i G_d)^t
+    with the 1-D Hermite coefficients E_t of `_hermite_E` (the Fourier transform of the Hermite Gaussian of order t is
+    (i G_d)^t times that of order 0).  This is the host path of the structure-factor target of `exp_pot.Exp` and the
+    reference the device kernel (`ecw_ft_aopair`) is tested against."""
+    G = np.atleast_2d(np.asarray(G, dtype=np.float64))
+    if G.ndim != 2 or G.shape[1] != 3:
+        raise ValueError("G must be an [nG, 3] array of scattering vectors")
+    I, J, M = _pairs(mol)
+    a, b = mol.ex[I], mol.ex[J]
+    p = a + b
+    mu = a * b / p
+    A, B = mol.cen[I], mol.cen[J]
+    P = (a[:, None] * A + b[:, None] * B) / p[:, None]
+    la, lb = mol.lmn[I], mol.lmn[J]
+    lm = mol.lmax
+    re = np.ones((len(G), len(p)))
+    im = np.zeros((len(G), len(p)))
+    for d in range(3):
+        E = _hermite_E(lm, lm, p, P[:, d] - A[:, d], P[:, d] - B[:, d], mu, A[:, d] - B[:, d])
+        et = np.zeros((2 * lm + 1, len(p)))                      # E_t^{la_d, lb_d} per pair
+        for i in range(lm + 1):
+            for j in range(lm + 1):
+                m = (la[:, d] == i) & (lb[:, d] == j)
+                for t in range(i + j + 1):
+                    et[t, m] = E[i][j][t][m]
+        g = G[:, d:d + 1]
+        pr, pi = np.zeros_like(re), np.zeros_like(im)            # sum_t E_t (i g)^t
+        for t in range(2 * lm + 1):
+            c = et[t][None, :] * g ** t
+            if t % 4 == 0:
+                pr += c
+            elif t % 4 == 1:
+                pi += c
+            elif t % 4 == 2:
+                pr -= c
+            else:
+                pi -= c
+        re, im = re * pr - im * pi, re * pi + im * pr
+    amp = mol.coef[I] * mol.coef[J] * (np.pi / p) ** 1.5 * np.exp(-(G ** 2).sum(1)[:, None] / (4 * p[None, :]))
+    ph = G @ P.T
+    c, s = np.cos(ph), np.sin(ph)
+    vr = amp * (re * c - im * s)
+    vi = amp * (re * s + im * c)
+    nao = mol.nao
+    return ((vr @ M) + 1j * (vi @ M)).reshape(len(G), nao, nao)
+
+
 def rhf(mol, ints=None, conv=1e-11, maxiter=100):
     """Closed-shell SCF with DIIS.  Returns (E_HF, mo_energy, mo_coeff, ints)."""
     S, T, V, eri = ints if ints is not None else integrals(mol)

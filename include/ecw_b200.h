@@ -189,6 +189,25 @@ int ecw_conv_check(const double* a, const double* b, const double* prev, double*
 int ecw_vexp_mat(const double* rdm1, const double* target, const double* fock, double L, double* vexp, double* fsp,
                  double* stats2, int64_t n, void* stream);
 
+/* Structure-factor ('F') target.  ecw_ft_aopair fills out[2][nG][nao][nao] (Re plane, then Im plane) with the
+ * Fourier-transformed AO pairs A_mu,nu(G) = int phi_mu phi_nu exp(+i G.r) d^3r for the scattering vectors G[nG,3]
+ * (bohr^-1).  prim[nprim,8] = {Ax, Ay, Az, alpha, coef, lx, ly, lz} lists primitive Cartesian Gaussians (bohr; coef
+ * includes normalisation and contraction; l <= 2 per direction), those of AO mu at rows ao_first[mu] ..
+ * ao_first[mu+1]-1 (ao_first[nao+1], int64).  FP64, fixed summation order: two calls give identical bits.  A malformed
+ * table yields NaN elements.  All pointers are device pointers. */
+int ecw_ft_aopair(const double* prim, int64_t nprim, const int64_t* ao_first, int nao, const double* G, int64_t nG,
+                  double* out, void* stream);
+/* One iteration of the 'F' potential, ground state: D = C_a gamma C_a^T + C_b gamma C_b^T (rdm1 gamma [n,n] in
+ * spin-orbital MOs, mo_coeff_g [2nao,n] with alpha rows first), F_calc[2][nG] = sum_mu,nu D_mu,nu A_mu,nu(G_h) (Re, Im),
+ * dF = F_exp - F_calc (F_exp[2][nG]), vexp = L sum_h Re[conj(dF_h) C_g^T blockdiag(A_h, A_h) C_g] (= -dP/dgamma of
+ * P = L/2 sum_h |dF_h|^2), fsp = fock - vexp; stats2[0] = sum_h |dF_h|, stats2[1] = max |vexp|.  ft: the planes of
+ * ecw_ft_aopair.  workspace: ecw_vexp_sf_workspace_bytes(n, nao, nG) bytes of device memory.  Device pointers;
+ * stream-ordered, no synchronisation; fixed reduction order. */
+int ecw_vexp_sf(const double* rdm1, int n, const double* mo_coeff_g, int nao, const double* ft, int64_t nG,
+                const double* F_exp, double L, const double* fock, double* vexp, double* fsp, double* F_calc,
+                double* stats2, double* workspace, void* stream);
+int64_t ecw_vexp_sf_workspace_bytes(int n, int nao, int64_t nG);
+
 /* ---- primitive device ops ---------------------------------------------------------
  * The CCS class (CCS.py:197-1518: T1inter/tsupdate/L1inter/lsupdate/R1inter/rsupdate/es_L1inter/
  * es_lsupdate/R0inter/L0inter/*_fromE/gamma_*) and the GCC intermediate getters (cc_Fvv, cc_Woooo,
