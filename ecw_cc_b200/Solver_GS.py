@@ -2,8 +2,8 @@
 (Solver_GS.py:522-742): same constructor and `SCF` signatures, same iteration order, same convergence bookkeeping
 (Q7: `Dconv` stays 1.0 on iteration 0; divergence threshold 1.0) and the same return tuple — but the o^2v^2 amplitudes
 never leave the GPU.  With `ecw_cc_b200.exp_pot.Exp` and a single density-matrix target (what `Main.CCSD_GS` fits), or a
-single structure-factor target, the potential and the dressed Fock matrix are formed on the device too (`ecw_vexp_mat`,
-`ecw_vexp_sf`) and only scalars cross PCIe; with
+single structure-factor or amplitude target, the potential and the dressed Fock matrix are formed on the device too
+(`ecw_vexp_mat`, `ecw_vexp_sf`, `ecw_vexp_sfobs`) and only scalars cross PCIe; with
 any other `VX_exp` object (e.g. the unchanged reference `exp_pot.Exp`, exp_pot.py:131-345) the rdm1 (n x n) goes to the
 host once per iteration and the dressed Fock comes back.  The convergence vector and its norm are formed on the device
 (`ecw_conv_check`).
@@ -117,15 +117,17 @@ class Solver_CCSD(object):
         if 'tl' in diis:
             tl_diis = DIIS(mycc._dev_ops())
             tl_diis.space, tl_diis.min_space = self.maxdiis, 2
-        # a single density-matrix target (ecw_vexp_mat) or a single structure-factor target (ecw_vexp_sf) of our own Exp
-        # class is evaluated on the device: then nothing but scalars crosses PCIe inside the loop.  Any other potential
-        # object, and DIIS on the rdm1, take the host route.
+        # a single density-matrix target (ecw_vexp_mat), structure-factor target (ecw_vexp_sf) or amplitude target
+        # (ecw_vexp_sfobs) of our own Exp class is evaluated on the device: then nothing but scalars crosses PCIe inside
+        # the loop.  Any other potential object, and DIIS on the rdm1, take the host route.
         dev_update = None
         if adiis is None:
             if getattr(VXexp, "device_mat_ready", lambda: False)():
                 dev_update = VXexp.mat_update_device
             elif getattr(VXexp, "device_sf_ready", lambda: False)():
                 dev_update = VXexp.sf_update_device
+            elif getattr(VXexp, "device_fobs_ready", lambda: False)():
+                dev_update = VXexp.fobs_update_device
         on_device = dev_update is not None
         fock_dev = mycc.eris.fock_dev if on_device else None
         rdm1_dev = None

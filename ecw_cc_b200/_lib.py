@@ -136,6 +136,10 @@ class _Lib(object):
             "ecw_ft_aopair": (c_i, [c_p, c_l, c_p, c_i, c_p, c_l, c_p, c_p]),
             "ecw_vexp_sf": (c_i, [c_p, c_i, c_p, c_i, c_p, c_l, c_p, c_d, c_p, c_p, c_p, c_p, c_p, c_p, c_p]),
             "ecw_vexp_sf_workspace_bytes": (c_l, [c_i, c_i, c_l]),
+            "ecw_ft_aopair_cryst": (c_i, [c_p, c_l, c_p, c_p, c_i, c_p, c_i, c_p, c_p, c_i, c_l, c_p, c_p]),
+            "ecw_vexp_sfobs": (c_i, [c_p, c_i, c_p, c_i, c_p, c_l, c_p, c_p, c_d, c_d, c_p, c_p, c_p, c_p, c_p, c_p,
+                                     c_p]),
+            "ecw_vexp_sfobs_workspace_bytes": (c_l, [c_i, c_i, c_l]),
             "ecw_profile_enable": (c_i, [c_p, c_i]),
             "ecw_profile_dump": (c_l, [c_p, c_p, c_l]),
         }

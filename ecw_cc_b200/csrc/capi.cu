@@ -1182,6 +1182,47 @@ int64_t ecw_vexp_sf_workspace_bytes(int n, int nao, int64_t nG) {
   return 8 * SfWorkspace(n, nao, nG).total;
 }
 
+extern "C++" {
+namespace {
+// The pipeline shared by the 'F' and 'Fobs' potentials: D = C_a gamma C_a^T + C_b gamma C_b^T, F_calc = planes . vec(D),
+// coef_step(F_calc, coef) forms the GEMV coefficients [2 nG], V_AO = planes^T . coef, vexp = C_g^T blockdiag(V_AO,
+// V_AO) C_g, fsp = fock - vexp and stats[1] = max |vexp|.  Stream-ordered, no synchronisation.
+template <typename CoefStep>
+void vexp_planes(const double* rdm1, int n, const double* mo_coeff_g, int nao, const double* ft, int64_t nG,
+                 const double* fock, double* vexp, double* fsp, double* F_calc, double* stats, double* workspace,
+                 cudaStream_t st, CoefStep coef_step) {
+  const SfWorkspace w(n, nao, nG);
+  double* X = workspace + w.x;                 // C_g gamma, later blockdiag(V, V) C_g
+  double* D = workspace + w.d;
+  double* coef = workspace + w.coef;
+  double* V = workspace + w.v;
+  const int64_t n2 = (int64_t)nao * nao;
+  const double* Ca = mo_coeff_g;               // alpha rows of C_g
+  const double* Cb = mo_coeff_g + (int64_t)nao * n;
+  auto gemm = [&](int ta, int tb, int64_t M, int64_t N, int64_t K, const double* A, int64_t lda, const double* B,
+                  int64_t ldb, double beta, double* C, int64_t ldc) {
+    GemmArgs g{};
+    g.A = A; g.B = B; g.C = C; g.M = M; g.N = N; g.K = K; g.lda = lda; g.ldb = ldb; g.ldc = ldc;
+    g.batch = 1; g.splitk = 1; g.kchunk = K; g.ta = ta; g.tb = tb; g.alpha = 1.0; g.beta = beta;
+    ck(launch_gemm(g, st), "vexp_sf gemm");
+  };
+  // D = C_a gamma C_a^T + C_b gamma C_b^T: the spin-summed AO density
+  gemm(0, 0, 2LL * nao, n, n, mo_coeff_g, n, rdm1, n, 0.0, X, n);
+  gemm(0, 1, nao, nao, n, X, n, Ca, n, 0.0, D, nao);
+  gemm(0, 1, nao, nao, n, X + (int64_t)nao * n, n, Cb, n, 1.0, D, nao);
+  // F_calc [Re | Im] = planes [2 nG, nao^2] . vec(D)
+  gemm(0, 0, 2 * nG, 1, n2, ft, n2, D, 1, 0.0, F_calc, 1);
+  coef_step(F_calc, coef);
+  // V_AO = planes^T . coef,  vexp = C_g^T blockdiag(V_AO, V_AO) C_g
+  gemm(1, 0, n2, 1, 2 * nG, ft, n2, coef, 1, 0.0, V, 1);
+  gemm(0, 0, nao, n, nao, V, nao, Ca, n, 0.0, X, n);
+  gemm(0, 0, nao, n, nao, V, nao, Cb, n, 0.0, X + (int64_t)nao * n, n);
+  gemm(1, 0, n, n, 2LL * nao, mo_coeff_g, n, X, n, 0.0, vexp, n);
+  ck(launch_sf_finish(vexp, fock, fsp, stats, (int64_t)n * n, st), "vexp_sf finish");
+}
+}  // namespace
+}  // extern "C++"
+
 int ecw_vexp_sf(const double* rdm1, int n, const double* mo_coeff_g, int nao, const double* ft, int64_t nG,
                 const double* F_exp, double L, const double* fock, double* vexp, double* fsp, double* F_calc,
                 double* stats2, double* workspace, void* stream) {
@@ -1191,34 +1232,42 @@ int ecw_vexp_sf(const double* rdm1, int n, const double* mo_coeff_g, int nao, co
       throw Fail("ecw_vexp_sf: null pointer");
     if (n < 1 || nao < 1 || nG < 1) throw Fail("ecw_vexp_sf: empty rdm1, basis or reflection list");
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const SfWorkspace w(n, nao, nG);
-    double* X = workspace + w.x;                 // C_g gamma, later blockdiag(V, V) C_g
-    double* D = workspace + w.d;
-    double* coef = workspace + w.coef;
-    double* V = workspace + w.v;
-    const int64_t n2 = (int64_t)nao * nao;
-    const double* Ca = mo_coeff_g;               // alpha rows of C_g
-    const double* Cb = mo_coeff_g + (int64_t)nao * n;
-    auto gemm = [&](int ta, int tb, int64_t M, int64_t N, int64_t K, const double* A, int64_t lda, const double* B,
-                    int64_t ldb, double beta, double* C, int64_t ldc) {
-      GemmArgs g{};
-      g.A = A; g.B = B; g.C = C; g.M = M; g.N = N; g.K = K; g.lda = lda; g.ldb = ldb; g.ldc = ldc;
-      g.batch = 1; g.splitk = 1; g.kchunk = K; g.ta = ta; g.tb = tb; g.alpha = 1.0; g.beta = beta;
-      ck(launch_gemm(g, st), "vexp_sf gemm");
-    };
-    // D = C_a gamma C_a^T + C_b gamma C_b^T: the spin-summed AO density
-    gemm(0, 0, 2LL * nao, n, n, mo_coeff_g, n, rdm1, n, 0.0, X, n);
-    gemm(0, 1, nao, nao, n, X, n, Ca, n, 0.0, D, nao);
-    gemm(0, 1, nao, nao, n, X + (int64_t)nao * n, n, Cb, n, 1.0, D, nao);
-    // F_calc [Re | Im] = planes [2 nG, nao^2] . vec(D)
-    gemm(0, 0, 2 * nG, 1, n2, ft, n2, D, 1, 0.0, F_calc, 1);
-    ck(launch_sf_coef(F_exp, F_calc, L, coef, stats2, nG, st), "vexp_sf coef");
-    // V_AO = planes^T . coef,  vexp = C_g^T blockdiag(V_AO, V_AO) C_g
-    gemm(1, 0, n2, 1, 2 * nG, ft, n2, coef, 1, 0.0, V, 1);
-    gemm(0, 0, nao, n, nao, V, nao, Ca, n, 0.0, X, n);
-    gemm(0, 0, nao, n, nao, V, nao, Cb, n, 0.0, X + (int64_t)nao * n, n);
-    gemm(1, 0, n, n, 2LL * nao, mo_coeff_g, n, X, n, 0.0, vexp, n);
-    ck(launch_sf_finish(vexp, fock, fsp, stats2, (int64_t)n * n, st), "vexp_sf finish");
+    vexp_planes(rdm1, n, mo_coeff_g, nao, ft, nG, fock, vexp, fsp, F_calc, stats2, workspace, st,
+                [&](const double* fc, double* coef) {
+                  ck(launch_sf_coef(F_exp, fc, L, coef, stats2, nG, st), "vexp_sf coef");
+                });
+  });
+}
+
+int ecw_ft_aopair_cryst(const double* prim, int64_t nprim, const int64_t* ao_first, const int64_t* ao_atom, int nao,
+                        const double* U, int natom, const double* Gs, const double* phase, int nsym, int64_t nG,
+                        double* out, void* stream) {
+  return guarded(nullptr, [&] {
+    require_device();
+    if (!prim || !ao_first || !ao_atom || !U || !Gs || !phase || !out) throw Fail("ecw_ft_aopair_cryst: null pointer");
+    if (nprim < 1 || nao < 1 || nG < 1 || natom < 1) throw Fail("ecw_ft_aopair_cryst: empty table, basis or hkl list");
+    if (nsym < 1 || nsym > 192) throw Fail("ecw_ft_aopair_cryst: nsym must lie in 1..192");
+    ck(launch_ft_aopair_cryst(prim, nprim, ao_first, ao_atom, nao, U, natom, Gs, phase, nsym, nG, out,
+                              static_cast<cudaStream_t>(stream)), "ft_aopair_cryst");
+  });
+}
+
+int64_t ecw_vexp_sfobs_workspace_bytes(int n, int nao, int64_t nG) { return ecw_vexp_sf_workspace_bytes(n, nao, nG); }
+
+int ecw_vexp_sfobs(const double* rdm1, int n, const double* mo_coeff_g, int nao, const double* ft, int64_t nG,
+                   const double* F_obs, const double* weight, double k_fixed, double L, const double* fock, double* vexp,
+                   double* fsp, double* F_calc, double* stats4, double* workspace, void* stream) {
+  return guarded(nullptr, [&] {
+    require_device();
+    if (!rdm1 || !mo_coeff_g || !ft || !F_obs || !weight || !fock || !vexp || !fsp || !F_calc || !stats4 || !workspace)
+      throw Fail("ecw_vexp_sfobs: null pointer");
+    if (n < 1 || nao < 1 || nG < 1) throw Fail("ecw_vexp_sfobs: empty rdm1, basis or reflection list");
+    if (!(k_fixed > 0.0) && nG < 2) throw Fail("ecw_vexp_sfobs: a refined scale needs at least two reflections");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    vexp_planes(rdm1, n, mo_coeff_g, nao, ft, nG, fock, vexp, fsp, F_calc, stats4, workspace, st,
+                [&](const double* fc, double* coef) {
+                  ck(launch_sfobs_coef(F_obs, weight, fc, L, k_fixed, coef, stats4, nG, st), "vexp_sfobs coef");
+                });
   });
 }
 

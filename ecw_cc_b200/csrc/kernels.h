@@ -136,6 +136,16 @@ cudaError_t launch_ft_aopair(const double* prim, int64_t nprim, const int64_t* a
 // coef [2][nG] = L (F_exp - F_calc) (Re, Im planes), stats[0] = sum_h |F_exp(h) - F_calc(h)|
 cudaError_t launch_sf_coef(const double* F_exp, const double* F_calc, double L, double* coef, double* stats, int64_t nG,
                            cudaStream_t st);
+// amplitude ('Fobs') target.  Symmetrised, smeared planes B(h) = sum_s exp(2 pi i h.t_s) T(G_hs) A(G_hs), out as for
+// launch_ft_aopair; ao_atom [nao] (int64), U [natom][6] = Cartesian ADP (xx, yy, zz, xy, xz, yz) in bohr^2, Gs
+// [nG][nsym][3] = G_{R_s^T h} in bohr^-1, phase [nG][nsym][2] = (cos, sin) of 2 pi h.t_s; 1 <= nsym <= 192
+cudaError_t launch_ft_aopair_cryst(const double* prim, int64_t nprim, const int64_t* ao_first, const int64_t* ao_atom,
+                                   int nao, const double* U, int natom, const double* Gs, const double* phase, int nsym,
+                                   int64_t nG, double* out, cudaStream_t st);
+// scale k (k_fixed > 0: fixed, else refined), coef [2][nG] of the amplitude potential, stats[0] = sum |k|Fc| - Fo|,
+// stats[2] = k, stats[3] = chi^2 (w = 1/sigma^2 per reflection)
+cudaError_t launch_sfobs_coef(const double* F_obs, const double* w, const double* F_calc, double L, double k_fixed,
+                              double* coef, double* stats, int64_t nG, cudaStream_t st);
 // fsp = fock - vexp, stats[1] = max |vexp|
 cudaError_t launch_sf_finish(const double* vexp, const double* fock, double* fsp, double* stats, int64_t n2,
                              cudaStream_t st);

@@ -8,10 +8,14 @@ not the path.  Basis sets embedded for H, C, N, O: the 6-31G family — 6-31G, 6
 (Pople's standard polarisation / diffuse exponents; five spherical d functions per shell, PySCF's default) — and
 cc-pVDZ for H, C, O.  Anchor: E_HF(H2O/6-31G) = -75.9839 (ECW_CC/__init__.py:39).
 """
+import re
+from fractions import Fraction
+
 import numpy as np
 from scipy.special import hyp1f1
 
 ANGSTROM = 1.0 / 0.52917721092                 # bohr per Angstrom (the value PySCF uses)
+FOBS_ZERO = 1e-12                              # 'Fobs': |F_calc| <= FOBS_ZERO max |F_calc| counts as zero
 
 # 6-31G: per element a list of (kind, exponents, s coefficients, p coefficients)
 BASIS_631G = {
@@ -109,9 +113,9 @@ class Molecule(object):
         if self.nelec % 2:
             raise NotImplementedError("closed shells only (RHF)")
         # primitive Cartesian Gaussians: centre, exponent, (lx,ly,lz), coefficient incl. normalisation, AO index
-        cen, ex, lmn, coef, ao = [], [], [], [], []
+        cen, ex, lmn, coef, ao, ao_atom = [], [], [], [], [], []
         nao = 0
-        for z, r in zip(self.Z, self.R):
+        for iat, (z, r) in enumerate(zip(self.Z, self.R)):
             for kind, exps, cs, cp in basis_shells(basis, int(z)):
                 parts = {"S": ((0, cs),), "P": ((1, cp),), "SP": ((0, cs), (1, cp)), "D": ((2, cp),)}[kind]
                 for ang, cc in parts:
@@ -124,9 +128,11 @@ class Molecule(object):
                             norm = (2 * a / np.pi) ** 0.75 * (2 * np.sqrt(a)) ** ang      # s / p / xy-type d norm
                             for l3, f in comp:
                                 cen.append(r); ex.append(a); lmn.append(l3); coef.append(c * norm * f); ao.append(nao)
+                        ao_atom.append(iat)
                         nao += 1
         self.cen, self.ex = np.array(cen), np.array(ex)
         self.lmn, self.coef, self.ao = np.array(lmn), np.array(coef), np.array(ao)
+        self.ao_atom = np.array(ao_atom, dtype=np.int64)            # atom of every AO
         self.nao = nao
         self.lmax = int(self.lmn.sum(1).max())
         # Tables of general contractions (cc-pVDZ) list contracted functions that are not unit normalised: rescale
@@ -417,6 +423,173 @@ def ft_aopair(mol, G):
     vi = amp * (re * s + im * c)
     nao = mol.nao
     return ((vr @ M) + 1j * (vi @ M)).reshape(len(G), nao, nao)
+
+
+_SYMOP_TERM = re.compile(r"([+-])((?:\d+(?:\.\d*)?|\.\d+)(?:/\d+)?)?\*?([xyz])?")
+
+
+def parse_symop(op):
+    """One symmetry operation x' = R x + t in fractional coordinates, from a CIF `_space_group_symop_operation_xyz`
+    string ('x,y,z', '-x,y+1/2,-z+1/2', 'x-y,x,z+1/6', ...) or an (R, t) pair.  R must be an integer matrix with
+    det +-1.  Returns (R int [3, 3], t float [3])."""
+    if isinstance(op, str):
+        parts = op.replace(" ", "").lower().split(",")
+        if len(parts) != 3:
+            raise ValueError("symmetry operation %r: three comma-separated components expected" % (op,))
+        R, t = np.zeros((3, 3)), np.zeros(3)
+        for d, s in enumerate(parts):
+            s = s if s[:1] in ("+", "-") else "+" + s
+            pos = 0
+            while pos < len(s):
+                m = _SYMOP_TERM.match(s, pos)
+                if m is None or (m.group(2) is None and m.group(3) is None):
+                    raise ValueError("symmetry operation %r: cannot read %r" % (op, s[pos:]))
+                v = float(Fraction(m.group(2))) if m.group(2) else 1.0
+                v = -v if m.group(1) == "-" else v
+                if m.group(3):
+                    R[d, "xyz".index(m.group(3))] += v
+                else:
+                    t[d] += v
+                pos = m.end()
+    else:
+        try:
+            R, t = op
+            R, t = np.asarray(R, dtype=np.float64), np.asarray(t, dtype=np.float64)
+        except (TypeError, ValueError):
+            raise ValueError("symmetry operation %r: a CIF xyz string or an (R, t) pair expected" % (op,))
+        if R.shape != (3, 3) or t.shape != (3,) or not np.all(np.isfinite(R)) or not np.all(np.isfinite(t)):
+            raise ValueError("symmetry operation: R must be 3 x 3 and t of length 3, finite")
+    if np.any(R != np.round(R)):
+        raise ValueError("symmetry operation %r: R must be an integer matrix" % (op,))
+    R = np.round(R).astype(np.int64)
+    if abs(round(np.linalg.det(R))) != 1:
+        raise ValueError("symmetry operation %r: det R must be +-1" % (op,))
+    return R, t
+
+
+def symop_string(R, t):
+    """The CIF xyz string of (R, t): the inverse of `parse_symop` for the standard strings."""
+    out = []
+    for d in range(3):
+        s = ""
+        for e in range(3):
+            c = int(R[d][e])
+            if c:
+                s += ("+" if c > 0 else "-") + ("" if abs(c) == 1 else str(abs(c))) + "xyz"[e]
+        f = Fraction(float(t[d])).limit_denominator(48)
+        if f:
+            s += ("+" if f > 0 else "-") + str(abs(f))
+        out.append(s.lstrip("+") or "0")
+    return ",".join(out)
+
+
+class Crystal(object):
+    """A molecular crystal for the amplitude target 'Fobs' of `exp_pot.Exp`.
+
+    cell: (a, b, c) in Angstrom (orthorhombic) or (a, b, c, alpha, beta, gamma) in Angstrom and degrees.  The lattice
+    matrix M has the lattice vectors as columns in the standard orthogonalisation (a along x, b in the xy plane):
+        M = [[a, b cos g, c cos b], [0, b sin g, c (cos a - cos b cos g) / sin g], [0, 0, V / (a b sin g)]]
+    and the molecule's Cartesian coordinates (`Molecule`, Angstrom) are taken in this frame (`cartesian` converts
+    fractional coordinates).  The scattering vector of reflection h is G_h = 2 pi M^-T h.
+
+    symops: operations x' = R x + t in fractional coordinates, CIF xyz strings or (R, t) pairs (`parse_symop`); the
+    default is the identity.  The list must hold exactly the operations that generate the DISTINCT copies of the
+    molecule in the cell, centring translations included: for a molecule on a special position give only the coset
+    representatives.  One molecule in the asymmetric unit (Z' = 1).
+
+    adp: None, or one entry per atom of the molecule: None (no smearing), a scalar U_iso, or a 3 x 3 Cartesian U tensor
+    in the frame above (not the crystal-axis U_ij of a CIF), Angstrom^2."""
+
+    def __init__(self, cell, symops=("x,y,z",), adp=None):
+        cell = np.asarray(cell, dtype=np.float64)
+        if cell.shape not in ((3,), (6,)) or not np.all(np.isfinite(cell)) or np.any(cell[:3] <= 0):
+            raise ValueError("cell: (a, b, c) or (a, b, c, alpha, beta, gamma), positive lengths in Angstrom")
+        ang = cell[3:] if len(cell) == 6 else np.full(3, 90.0)
+        if np.any(ang <= 0) or np.any(ang >= 180):
+            raise ValueError("cell angles must lie strictly between 0 and 180 degrees")
+
+        def cos_sin(x):                                             # exact 0 / 1 at 90 degrees
+            return (0.0, 1.0) if x == 90.0 else (np.cos(np.deg2rad(x)), np.sin(np.deg2rad(x)))
+        (ca, _), (cb, _), (cg, sg) = (cos_sin(x) for x in ang)
+        vf = 1.0 - ca * ca - cb * cb - cg * cg + 2.0 * ca * cb * cg
+        if vf <= 0:
+            raise ValueError("cell angles do not describe a cell of positive volume")
+        a, b, c = cell[:3]
+        self.cell = cell
+        self.M = np.array([[a, b * cg, c * cb], [0.0, b * sg, c * (ca - cb * cg) / sg], [0.0, 0.0, c * np.sqrt(vf) / sg]])
+        self.volume = float(a * b * c * np.sqrt(vf))
+        self.ops = [parse_symop(op) for op in ([symops] if isinstance(symops, str) else symops)]
+        if not self.ops:
+            raise ValueError("symops: at least one operation")
+        self.adp = None if adp is None else [self._adp_entry(u) for u in adp]
+
+    @staticmethod
+    def _adp_entry(u):
+        if u is None:
+            return np.zeros((3, 3))
+        u = np.asarray(u, dtype=np.float64)
+        if u.ndim == 0:
+            u = float(u) * np.eye(3)
+        if u.shape != (3, 3) or not np.all(np.isfinite(u)) or np.abs(u - u.T).max() > 1e-12 * max(1.0, np.abs(u).max()):
+            raise ValueError("adp: each entry is None, a scalar U_iso or a symmetric 3 x 3 Cartesian tensor (A^2)")
+        if np.linalg.eigvalsh(u).min() < -1e-12 * max(1.0, np.abs(u).max()):
+            raise ValueError("adp: U must be positive semi-definite")
+        return 0.5 * (u + u.T)
+
+    @property
+    def nsym(self):
+        return len(self.ops)
+
+    def cartesian(self, frac):
+        """Fractional coordinates [..., 3] -> Cartesian Angstrom in the frame of M."""
+        return np.asarray(frac, dtype=np.float64) @ self.M.T
+
+    def G(self, hkl):
+        """G_h = 2 pi M^-T h in bohr^-1, [..., 3] (M^T is lower triangular: forward substitution, which gives
+        2 pi (h/a, k/b, l/c) bit for bit in an orthorhombic cell)."""
+        x = 2 * np.pi * np.asarray(hkl, dtype=np.float64)
+        M = self.M
+        g0 = x[..., 0] / M[0, 0]
+        g1 = (x[..., 1] - M[0, 1] * g0) / M[1, 1]
+        g2 = (x[..., 2] - M[0, 2] * g0 - M[1, 2] * g1) / M[2, 2]
+        return np.stack([g0, g1, g2], axis=-1) / ANGSTROM
+
+    def adp_bohr(self, natom):
+        """Cartesian U per atom in bohr^2, [natom, 3, 3] (zeros without ADPs)."""
+        if self.adp is None:
+            return np.zeros((natom, 3, 3))
+        if len(self.adp) != natom:
+            raise ValueError("adp: %d entries for a molecule of %d atoms" % (len(self.adp), natom))
+        return np.array(self.adp) * ANGSTROM ** 2
+
+    def tables(self, hkl):
+        """What the symmetrised planes need per (h, s), [N_h, nsym, ...]: the rotated vectors G_{h_s}, h_s = R_s^T h
+        (bohr^-1), and the phases (cos, sin) of 2 pi h.t_s (h.t_s reduced mod 1 first)."""
+        h = np.asarray(hkl, dtype=np.float64).reshape(-1, 3)
+        R = np.array([r for r, _ in self.ops], dtype=np.float64)
+        t = np.array([t for _, t in self.ops])
+        Gs = self.G(np.einsum("sdk,hd->hsk", R, h))
+        ph = 2 * np.pi * np.mod(h @ t.T, 1.0)
+        return Gs, np.stack([np.cos(ph), np.sin(ph)], axis=-1)
+
+
+def ft_aopair_cryst(mol, crystal, hkl):
+    """Symmetrised, thermally smeared AO-pair transforms, complex [N_h, nao, nao]:
+        B_mu,nu(h) = sum_s exp(+2 pi i h.t_s) T_mu,nu(G_{h_s}) A_mu,nu(G_{h_s}),   h_s = R_s^T h,
+    A = `ft_aopair`, T_mu,nu(G) = (T_A(G) + T_B(G)) / 2 for mu on atom A and nu on atom B, T_A(G) = exp(-G^T U_A G / 2).
+    For a one-centre pair T is the exact Debye-Waller factor of a rigidly displaced atom; for a two-centre pair the
+    arithmetic mean is a convention.  F_calc(h) = sum D_mu,nu B_mu,nu(h) is then the structure factor of the unit cell
+    (all copies of the molecule, smeared).  Host path of the 'Fobs' target and reference of `ecw_ft_aopair_cryst`."""
+    Gs, ph = crystal.tables(hkl)
+    U = crystal.adp_bohr(len(mol.Z))
+    at = mol.ao_atom
+    out = np.zeros((len(Gs), mol.nao, mol.nao), dtype=np.complex128)
+    for s in range(crystal.nsym):
+        G = Gs[:, s]
+        T = np.exp(-0.5 * np.einsum("hi,aij,hj->ha", G, U, G))      # [N_h, natom]
+        Tp = 0.5 * (T[:, at][:, :, None] + T[:, at][:, None, :])
+        out += (ph[:, s, 0] + 1j * ph[:, s, 1])[:, None, None] * Tp * ft_aopair(mol, G)
+    return out
 
 
 def rhf(mol, ints=None, conv=1e-11, maxiter=100):

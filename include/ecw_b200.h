@@ -208,6 +208,29 @@ int ecw_vexp_sf(const double* rdm1, int n, const double* mo_coeff_g, int nao, co
                 double* stats2, double* workspace, void* stream);
 int64_t ecw_vexp_sf_workspace_bytes(int n, int nao, int64_t nG);
 
+/* Amplitude ('Fobs') target: measured |F_obs| with weights 1/sigma^2, a unit cell of nsym copies of the molecule and
+ * thermal smearing.  ecw_ft_aopair_cryst fills out[2][nG][nao][nao] with the symmetrised, smeared planes
+ *   B_mu,nu(h) = sum_s exp(+2 pi i h.t_s) T_mu,nu(G_hs) A_mu,nu(G_hs),   T_mu,nu = (T_A + T_B)/2, T_A(G) = exp(-G^T U_A G/2)
+ * (A as for ecw_ft_aopair; mu on atom A, nu on atom B).  prim / ao_first as for ecw_ft_aopair; ao_atom[nao] (int64) is
+ * the atom of each AO; U[natom][6] = Cartesian ADP (xx, yy, zz, xy, xz, yz) in bohr^2; Gs[nG][nsym][3] = G_{R_s^T h} in
+ * bohr^-1 and phase[nG][nsym][2] = (cos, sin) of 2 pi h.t_s, tabulated by the caller; 1 <= nsym <= 192.  FP64, fixed
+ * summation order (operations in list order), identical bits call to call; a malformed table yields NaN elements. */
+int ecw_ft_aopair_cryst(const double* prim, int64_t nprim, const int64_t* ao_first, const int64_t* ao_atom, int nao,
+                        const double* U, int natom, const double* Gs, const double* phase, int nsym, int64_t nG,
+                        double* out, void* stream);
+/* One iteration of the 'Fobs' potential, ground state: D and F_calc[2][nG] as for ecw_vexp_sf (ft: the planes of
+ * ecw_ft_aopair_cryst), a_h = |F_calc(h)|, w = weight[nG] (1/sigma^2).  Scale k = k_fixed if k_fixed > 0 (N_p = 0), else
+ * refined, k = sum w F_obs a / sum w a^2 (N_p = 1, needs nG >= 2).  chi^2 = sum w (k a - F_obs)^2 / (nG - N_p), the
+ * penalty P = L chi^2, vexp = sum_h Re[conj(c_h) C_g^T blockdiag(B_h, B_h) C_g] with c_h = 2 L k / (nG - N_p) w_h (F_obs
+ * - k a_h) F_calc(h) / a_h, c_h = 0 where a_h <= 1e-12 max a (a cusp of |F|, the direction there is rounding noise)
+ * (= -dP/dgamma at fixed k; also at the refined k, where dP/dk = 0), fsp = fock - vexp.  stats4 = [sum_h |k a_h - F_obs(h)|, max |vexp|, k, chi^2].  workspace:
+ * ecw_vexp_sfobs_workspace_bytes(n, nao, nG) bytes.  Device pointers; stream-ordered, no synchronisation; fixed
+ * reduction order. */
+int ecw_vexp_sfobs(const double* rdm1, int n, const double* mo_coeff_g, int nao, const double* ft, int64_t nG,
+                   const double* F_obs, const double* weight, double k_fixed, double L, const double* fock, double* vexp,
+                   double* fsp, double* F_calc, double* stats4, double* workspace, void* stream);
+int64_t ecw_vexp_sfobs_workspace_bytes(int n, int nao, int64_t nG);
+
 /* ---- primitive device ops ---------------------------------------------------------
  * The CCS class (CCS.py:197-1518: T1inter/tsupdate/L1inter/lsupdate/R1inter/rsupdate/es_L1inter/
  * es_lsupdate/R0inter/L0inter/*_fromE/gamma_*) and the GCC intermediate getters (cc_Fvv, cc_Woooo,
