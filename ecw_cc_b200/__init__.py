@@ -15,5 +15,6 @@ from .Solver_GS import Solver_CCSD  # noqa: F401
 from .harness import Solver_CCS, Solver_ES  # noqa: F401  (test harness: callers of the path, see harness/__init__.py)
 from . import exp_pot  # noqa: F401
 from . import molint  # noqa: F401
+from . import maps  # noqa: F401
 
 __all__ = ["GCC", "Gccs", "Solver_CCSD", "Solver_CCS", "Solver_ES", "DevOps", "DeviceEris", "subdiff", "gamma_CCSD", "build", "lib", "EcwError"]

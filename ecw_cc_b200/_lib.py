@@ -5,7 +5,7 @@ import subprocess
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libecw_b200.so")
-_SRC = ["gemm.cu", "gemm_tma.cu", "ewise.cu", "ozaki.cu", "synth.cu", "ftao.cu", "capi.cu", "plan.cpp", "ccsd_plan.cpp",
+_SRC = ["gemm.cu", "gemm_tma.cu", "ewise.cu", "ozaki.cu", "synth.cu", "ftao.cu", "maps.cu", "capi.cu", "plan.cpp", "ccsd_plan.cpp",
         "ccsd_plan_slab.cpp", "ccs_plan.cpp"]
 
 ECW_HAS_ALPHA = 1
@@ -140,6 +140,9 @@ class _Lib(object):
             "ecw_vexp_sfobs": (c_i, [c_p, c_i, c_p, c_i, c_p, c_l, c_p, c_p, c_d, c_d, c_p, c_p, c_p, c_p, c_p, c_p,
                                      c_p]),
             "ecw_vexp_sfobs_workspace_bytes": (c_l, [c_i, c_i, c_l]),
+            "ecw_density_grid": (c_i, [c_p, c_l, c_p, c_i, c_p, ctypes.POINTER(c_d), c_i, c_i, c_i, c_p, c_p, c_p]),
+            "ecw_density_grid_workspace_bytes": (c_l, [c_i, c_l]),
+            "ecw_fourier_map": (c_i, [c_p, c_p, c_l, c_d, c_d, c_i, c_i, c_i, c_p, c_p]),
             "ecw_profile_enable": (c_i, [c_p, c_i]),
             "ecw_profile_dump": (c_l, [c_p, c_p, c_l]),
         }

@@ -5,6 +5,7 @@
 #include <dlfcn.h>
 
 #include <algorithm>
+#include <cmath>
 #include <cstring>
 #include <map>
 #include <memory>
@@ -1268,6 +1269,40 @@ int ecw_vexp_sfobs(const double* rdm1, int n, const double* mo_coeff_g, int nao,
                 [&](const double* fc, double* coef) {
                   ck(launch_sfobs_coef(F_obs, weight, fc, L, k_fixed, coef, stats4, nG, st), "vexp_sfobs coef");
                 });
+  });
+}
+
+int64_t ecw_density_grid_workspace_bytes(int nao, int64_t npts) {
+  if (nao < 1 || npts < 1) return -1;
+  return 8 * density_grid_workspace_elems(nao, npts);
+}
+
+int ecw_density_grid(const double* prim, int64_t nprim, const int64_t* ao_first, int nao, const double* dm,
+                     const double* box, int n1, int n2, int n3, double* out, double* workspace, void* stream) {
+  return guarded(nullptr, [&] {
+    require_device();
+    if (!prim || !ao_first || !dm || !box || !out || !workspace) throw Fail("ecw_density_grid: null pointer");
+    if (nprim < 1 || nao < 1) throw Fail("ecw_density_grid: empty primitive table or basis");
+    if (n1 < 1 || n2 < 1 || n3 < 1) throw Fail("ecw_density_grid: grid dimensions must be positive");
+    for (int c = 0; c < 12; ++c)
+      if (!std::isfinite(box[c])) throw Fail("ecw_density_grid: origin and axes must be finite");
+    ck(launch_density_grid(prim, nprim, ao_first, nao, dm, box, n1, n2, n3, out, workspace,
+                           static_cast<cudaStream_t>(stream)), "density_grid");
+  });
+}
+
+int ecw_fourier_map(const int64_t* hkl_half, const double* coef, int64_t N, double F000, double volume_bohr3, int n1,
+                    int n2, int n3, double* out, void* stream) {
+  return guarded(nullptr, [&] {
+    require_device();
+    if (!out || (N > 0 && (!hkl_half || !coef))) throw Fail("ecw_fourier_map: null pointer");
+    if (N < 0) throw Fail("ecw_fourier_map: negative reflection count");
+    if (n1 < 1 || n2 < 1 || n3 < 1 || n1 > FM_MAX_N || n2 > FM_MAX_N || n3 > FM_MAX_N)
+      throw Fail("ecw_fourier_map: grid dimensions must lie in 1..512");
+    if (!(volume_bohr3 > 0.0) || !std::isfinite(volume_bohr3) || !std::isfinite(F000))
+      throw Fail("ecw_fourier_map: the volume must be positive and F000 finite");
+    ck(launch_fourier_map(hkl_half, coef, N, F000, volume_bohr3, n1, n2, n3, out, static_cast<cudaStream_t>(stream)),
+       "fourier_map");
   });
 }
 

@@ -149,6 +149,21 @@ cudaError_t launch_sfobs_coef(const double* F_obs, const double* w, const double
 // fsp = fock - vexp, stats[1] = max |vexp|
 cudaError_t launch_sf_finish(const double* vexp, const double* fock, double* fsp, double* stats, int64_t n2,
                              cudaStream_t st);
+// density maps (maps.cu).  rho on the box grid r_ijk = origin + i a1 + j a2 + k a3, box[12] (host) = origin, a1, a2, a3
+// in bohr, out [n1][n2][n3] (k fastest); dm [nao][nao] is the AO density (need not be symmetric), prim / ao_first as for
+// launch_ft_aopair.  Points go in chunks of DG_CHUNK: Phi [chunk][nao] by ao_values_kernel, X = Phi D by launch_gemm,
+// rho_p = sum_mu X_p,mu Phi_p,mu; workspace: density_grid_workspace_elems(nao, npts) doubles (Phi and X)
+constexpr int64_t DG_CHUNK = 32768;
+int64_t density_grid_chunk(int64_t npts);
+int64_t density_grid_workspace_elems(int nao, int64_t npts);
+cudaError_t launch_density_grid(const double* prim, int64_t nprim, const int64_t* ao_first, int nao, const double* dm,
+                                const double* box, int n1, int n2, int n3, double* out, double* workspace,
+                                cudaStream_t st);
+// rho(x_ijk) = (F000 + 2 sum_h (Re F_h cos 2 pi h.x + Im F_h sin 2 pi h.x)) / volume at x_ijk = (i/n1, j/n2, k/n3) for
+// the half set hkl [N][3] (int64), coef [2][N] (Re, Im); out [n1][n2][n3]; 1 <= n_d <= FM_MAX_N
+constexpr int FM_MAX_N = 512;
+cudaError_t launch_fourier_map(const int64_t* hkl, const double* coef, int64_t N, double F000, double volume, int n1,
+                               int n2, int n3, double* out, cudaStream_t st);
 cudaError_t launch_conv(const double* a, const double* b, const double* prev, double* conv, int64_t n, double* partial,
                         int nblocks, double* scal, double beta, cudaStream_t st);
 cudaError_t launch_dot(const double* a, const double* b, int64_t n, double* partial, int nblocks, double* scal,

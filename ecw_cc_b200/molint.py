@@ -483,6 +483,20 @@ def symop_string(R, t):
     return ",".join(out)
 
 
+def check_group(ops, tol=1e-9):
+    """Raise ValueError unless the operations (R, t) are closed under composition modulo lattice translations:
+    (R_s R_u, R_s t_u + t_s mod 1) must be in the list for every s, u (t to `tol`)."""
+    R = np.array([r for r, _ in ops])
+    t = np.array([t for _, t in ops], dtype=np.float64)
+    for Rs, ts in zip(R, t):
+        for Ru, tu in zip(R, t):
+            dt = np.mod(Rs @ tu + ts - t + 0.5, 1.0) - 0.5
+            if not np.any(np.all(R == Rs @ Ru, axis=(1, 2)) & np.all(np.abs(dt) <= tol, axis=1)):
+                raise ValueError("the symmetry operations are not closed under composition (%s after %s is missing): "
+                                 "for a molecule on a special position the crystal lists only coset representatives; "
+                                 "pass the full space group as group=" % (symop_string(Rs, ts), symop_string(Ru, tu)))
+
+
 class Crystal(object):
     """A molecular crystal for the amplitude target 'Fobs' of `exp_pot.Exp`.
 
@@ -554,6 +568,48 @@ class Crystal(object):
         g2 = (x[..., 2] - M[0, 2] * g0 - M[1, 2] * g1) / M[2, 2]
         return np.stack([g0, g1, g2], axis=-1) / ANGSTROM
 
+    @property
+    def volume_bohr3(self):
+        return self.volume * ANGSTROM ** 3
+
+    def expand(self, hkl, F, group=None):
+        """Unique (or unmerged) structure factors -> the half set of the full sphere, for Fourier maps.
+
+        Every F(h) contributes F(R_u^T h) = exp(-2 pi i h.t_u) F(h) for each operation u and, by Friedel's law,
+        F(-R_u^T h) = conj of that.  Each coefficient of the expanded set is the mean of all contributions landing on
+        it: equivalents and Friedel mates are averaged, systematically absent reflections cancel to zero (to rounding)
+        and a consistent set such as F_calc comes out unchanged.  The operations (this crystal's, or `group`: symmetry
+        operations as for `Crystal`) must form a group modulo lattice translations; that is checked, to 1e-9 in t.
+        Returns (hkl_half int64 [M, 3], F_half complex [M], F000 float): h > 0, or h = 0 and k > 0, or h = k = 0 and
+        l > 0, in lexicographic order; F000 is the real part of the mean at (0, 0, 0) (0 when no input lands there)."""
+        hkl = np.asarray(hkl)
+        F = np.asarray(F)
+        if hkl.ndim != 2 or hkl.shape[1] != 3 or not np.issubdtype(hkl.dtype, np.number) \
+                or not np.all(np.isfinite(hkl)) or np.any(hkl != np.round(hkl)):
+            raise ValueError("hkl must be an (N_h, 3) array of integer Miller indices")
+        if F.shape != (len(hkl),) or not np.issubdtype(F.dtype, np.number) or not np.all(np.isfinite(F)):
+            raise ValueError("F must hold N_h finite (real or complex) structure factors, N_h = len(hkl)")
+        ops = self.ops if group is None else [parse_symop(op) for op in ([group] if isinstance(group, str) else group)]
+        if not ops:
+            raise ValueError("group: at least one operation")
+        check_group(ops)
+        R = np.array([r for r, _ in ops])
+        t = np.array([t for _, t in ops])
+        h = np.round(hkl).astype(np.int64)
+        hs = np.einsum("sdk,hd->hsk", R, h).reshape(-1, 3)          # R_u^T h
+        ph = 2 * np.pi * np.mod(h @ t.T, 1.0)
+        v = ((np.cos(ph) - 1j * np.sin(ph)) * F.astype(np.complex128)[:, None]).ravel()
+        keys, inv = np.unique(np.concatenate([hs, -hs]), axis=0, return_inverse=True)
+        inv = inv.ravel()
+        s = np.zeros(len(keys), dtype=np.complex128)
+        np.add.at(s, inv, np.concatenate([v, np.conj(v)]))
+        mean = s / np.bincount(inv, minlength=len(keys))
+        zero = np.all(keys == 0, axis=1)
+        F000 = float(mean[zero][0].real) if zero.any() else 0.0
+        half = (keys[:, 0] > 0) | ((keys[:, 0] == 0) & (keys[:, 1] > 0)) | \
+               ((keys[:, 0] == 0) & (keys[:, 1] == 0) & (keys[:, 2] > 0))
+        return keys[half], mean[half], F000
+
     def adp_bohr(self, natom):
         """Cartesian U per atom in bohr^2, [natom, 3, 3] (zeros without ADPs)."""
         if self.adp is None:
@@ -590,6 +646,64 @@ def ft_aopair_cryst(mol, crystal, hkl):
         Tp = 0.5 * (T[:, at][:, :, None] + T[:, at][:, None, :])
         out += (ph[:, s, 0] + 1j * ph[:, s, 1])[:, None, None] * Tp * ft_aopair(mol, G)
     return out
+
+
+def ao_values(mol, points):
+    """AO values phi_mu(r), [P, nao], at points [P, 3] in bohr: phi_mu(r) = sum_{p in mu} coef_p (x-A_x)^l (y-A_y)^m
+    (z-A_z)^n exp(-alpha_p |r-A|^2), each AO's primitives added in table order with no screening.  The reference of
+    the AO-value kernel of `ecw_density_grid`."""
+    r = np.atleast_2d(np.asarray(points, dtype=np.float64))
+    if r.ndim != 2 or r.shape[1] != 3:
+        raise ValueError("points must be a [P, 3] array (bohr)")
+    out = np.zeros((len(r), mol.nao))
+    for q in range(len(mol.ex)):
+        d = r - mol.cen[q]
+        r2 = d[:, 0] * d[:, 0] + d[:, 1] * d[:, 1] + d[:, 2] * d[:, 2]
+        lx, ly, lz = mol.lmn[q]
+        out[:, mol.ao[q]] += mol.coef[q] * d[:, 0] ** lx * d[:, 1] ** ly * d[:, 2] ** lz * np.exp(-mol.ex[q] * r2)
+    return out
+
+
+def density_points(mol, dm, points, chunk=65536):
+    """rho(r) = sum_mu,nu dm_mu,nu phi_mu(r) phi_nu(r) in e/bohr^3 at points [P, 3] (bohr), for an AO density dm
+    [nao, nao] (need not be symmetric).  The reference of `ecw_density_grid`."""
+    dm = np.asarray(dm, dtype=np.float64)
+    if dm.shape != (mol.nao, mol.nao):
+        raise ValueError("dm must be an (nao, nao) AO density matrix")
+    r = np.atleast_2d(np.asarray(points, dtype=np.float64))
+    out = np.empty(len(r))
+    for p0 in range(0, len(r), chunk):
+        phi = ao_values(mol, r[p0:p0 + chunk])
+        out[p0:p0 + chunk] = ((phi @ dm) * phi).sum(1)
+    return out
+
+
+def fourier_synthesis(hkl_half, F_half, F000, volume_bohr3, shape, chunk=256):
+    """rho(x_ijk) = (F000 + 2 sum_h (Re F_h cos 2 pi h.x + Im F_h sin 2 pi h.x)) / V at x_ijk = (i/n1, j/n2, k/n3), a
+    direct sum over the half set (the Friedel mates are implied): the inverse of the exp(+i G.r) sign of `ft_aopair`.
+    The phases are exact: (h_d i_d) mod n_d in integers, then a table of 2 pi m / n_d.  Returns [n1, n2, n3]."""
+    shape = tuple(int(n) for n in shape)
+    h = np.asarray(hkl_half, dtype=np.int64).reshape(-1, 3)
+    F = np.asarray(F_half, dtype=np.complex128).reshape(-1)
+    tabs = [np.exp(2j * np.pi * np.arange(n) / n) for n in shape]
+    acc = np.zeros(shape)
+    for c0 in range(0, len(h), chunk):
+        hc = h[c0:c0 + chunk]
+        e = [tabs[d][np.mod(hc[:, d:d + 1] * np.arange(shape[d]), shape[d])] for d in range(3)]
+        e12 = np.conj(F[c0:c0 + chunk])[:, None, None] * e[0][:, :, None] * e[1][:, None, :]
+        acc += np.einsum("cij,ck->ijk", e12, e[2]).real             # Re[conj(F) exp(2 pi i h.x)]
+    return (F000 + 2 * acc) / volume_bohr3
+
+
+def fourier_map(crystal, hkl, F, shape, group=None):
+    """Fourier map (1/V) sum_h F(h) exp(-2 pi i h.x) in e/bohr^3 on the [n1, n2, n3] fractional grid of `crystal`, from
+    structure factors F of the reflections hkl expanded to the full sphere by `crystal.expand(hkl, F, group)`.  A direct
+    sum for small grids: the reference of `ecw_fourier_map`."""
+    shape = tuple(int(n) for n in shape)
+    if len(shape) != 3 or min(shape) < 1:
+        raise ValueError("shape must be three positive grid dimensions")
+    hh, Fh, F000 = crystal.expand(hkl, F, group)
+    return fourier_synthesis(hh, Fh, F000, crystal.volume_bohr3, shape)
 
 
 def rhf(mol, ints=None, conv=1e-11, maxiter=100):

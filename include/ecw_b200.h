@@ -231,6 +231,25 @@ int ecw_vexp_sfobs(const double* rdm1, int n, const double* mo_coeff_g, int nao,
                    double* fsp, double* F_calc, double* stats4, double* workspace, void* stream);
 int64_t ecw_vexp_sfobs_workspace_bytes(int n, int nao, int64_t nG);
 
+/* Density maps.  ecw_density_grid fills out[n1][n2][n3] (k fastest, the cube-file order) with
+ *   rho(r_ijk) = sum_mu,nu dm[mu][nu] phi_mu(r_ijk) phi_nu(r_ijk),   r_ijk = origin + i a1 + j a2 + k a3,
+ * box[12] = {origin, a1, a2, a3} in bohr (a HOST array), dm[nao][nao] the AO density (need not be symmetric), prim /
+ * ao_first as for ecw_ft_aopair.  Points are processed in chunks of 32768: the AO values Phi[chunk][nao] (a fixed-order
+ * sum over each AO's primitives, no screening), X = Phi dm (FP64 GEMM), rho_p = sum_mu X_p,mu Phi_p,mu (fixed order).
+ * workspace: ecw_density_grid_workspace_bytes(nao, n1 n2 n3) bytes of device memory.  Identical bits call to call; a
+ * malformed table yields NaN.  Device pointers except box; stream-ordered, no synchronisation. */
+int ecw_density_grid(const double* prim, int64_t nprim, const int64_t* ao_first, int nao, const double* dm,
+                     const double* box, int n1, int n2, int n3, double* out, double* workspace, void* stream);
+int64_t ecw_density_grid_workspace_bytes(int nao, int64_t npts);
+/* Fourier synthesis on the fractional grid x_ijk = (i/n1, j/n2, k/n3) of a unit cell, out[n1][n2][n3]:
+ *   rho(x) = (F000 + 2 sum_h (Re F_h cos 2 pi h.x + Im F_h sin 2 pi h.x)) / volume_bohr3
+ * over the half set hkl_half[N][3] (int64; the Friedel mate -h of each is implied) with coef[2][N] = (Re F, Im F): the
+ * inverse of the exp(+i G.r) convention of ecw_ft_aopair.  The phase is exact, (h_d i_d) mod n_d in integers and a
+ * table of 2 pi m / n_d per axis; 1 <= n_d <= 512, N >= 0.  Fixed summation order, identical bits call to call.  Device
+ * pointers; stream-ordered, no synchronisation. */
+int ecw_fourier_map(const int64_t* hkl_half, const double* coef, int64_t N, double F000, double volume_bohr3, int n1,
+                    int n2, int n3, double* out, void* stream);
+
 /* ---- primitive device ops ---------------------------------------------------------
  * The CCS class (CCS.py:197-1518: T1inter/tsupdate/L1inter/lsupdate/R1inter/rsupdate/es_L1inter/
  * es_lsupdate/R0inter/L0inter/*_fromE/gamma_*) and the GCC intermediate getters (cc_Fvv, cc_Woooo,
