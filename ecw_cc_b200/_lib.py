@@ -79,7 +79,6 @@ class _Lib(object):
             "ecw_ctx_get_gemm": (c_i, [c_p]),
             "ecw_int8_error_bound": (c_i, [c_p, ctypes.POINTER(c_d), c_p]),
             "ecw_ctx_set_engine_override": (c_i, [c_p, c_i]),
-            "ecw_ctx_set_plan_variant": (c_i, [c_p, c_i]),
             "ecw_ctx_set_int8_splitk": (c_i, [c_p, c_l]),
             "ecw_ccs_t1inter": (c_i, [c_p, c_p, c_p, c_p, c_p]),
             "ecw_ccs_l1inter": (c_i, [c_p, c_p, c_p, c_i, c_p, c_p, c_p, c_p]),

@@ -552,13 +552,6 @@ int ecw_ctx_set_engine_override(ecw_ctx* c, int force_dmma) {
   return 0;
 }
 
-int ecw_ctx_set_plan_variant(ecw_ctx* c, int legacy_packed) {
-  if (!c) return -1;
-  c->z.legacy_packed = legacy_packed != 0;
-  drop_plans(c);
-  return 0;
-}
-
 int ecw_int8_error_bound(ecw_ctx* c, double* bound_out, void* stream) {
   return guarded(c, [&] {
     require_device();

@@ -1,4 +1,7 @@
-// ccsd_plan.cpp — plan builders for the spin-orbital CCSD residual path.
+// ccsd_plan.cpp — plan builders for the spin-orbital CCSD residual path: the
+// general T / Lambda variants (amplitudes not assumed antisymmetric), the rdm1
+// (gamma) and the energy.  The T / Lambda plans for antisymmetric amplitudes
+// are built in ccsd_plan_slab.cpp.
 //
 // Each builder states the reference equations as binary contractions over the
 // constant integral layouts of the eris container; the contraction list is
@@ -11,8 +14,8 @@
 //     Woooo (coefficient 1/4 -> 1/2), its t1.ovvv part becomes Y[ijma].t1;
 //   * wvvvo (CCSD.py:602-605) is never formed: each of its four pieces is
 //     contracted with l2 first;
-//   * the two particle-particle ladders and all o^4 terms run on
-//     antisymmetry-packed pairs  p(a<b) = b(b-1)/2 + a;
+//   * the two particle-particle ladders and the hole-hole ladder contract
+//     antisymmetry-packed integral pairs  p(a<b) = b(b-1)/2 + a;
 //   * ring terms run in the particle-hole layout X[(ia),(jb)].
 #include "ccsd_plan_detail.h"
 
@@ -29,357 +32,6 @@ void build_ccsd_energy(Plan& P, const Sizes& z) {
   P.axpby(1.0, s.fov, 0.0, f);
   emit_energy(P, s, f, 0);
   P.release(f);
-}
-
-// Round-1 lowering of the packed path (amplitudes and o^2v^2 intermediates replicated on every rank); kept behind
-// Sizes::legacy_packed (ecw_ctx_set_plan_variant) for A/B measurements against ccsd_plan_slab.cpp.
-void build_ccsd_tupdate_v1(Plan& P, const Sizes& z, int has_alpha, int equation) {
-  z.apply(P);
-  Slots s(z);
-  const int64_t o = s.o, v = s.v, po = s.po, pv = s.pv;
-  const bool shift = !equation && !has_alpha;  // CCSD.py:283-285
-  const Tensor &t1 = s.t1, &t2 = s.t2, &r1 = s.out1, &r2 = s.out2;
-
-  Tensor tau = P.tmp({o, o, v, v});
-  P.tau(t2, t1, 1.0, 1.0, tau);                                   // make_tau, CCSD.py:346-353
-  Tensor tau_p = P.tmp({po, pv});
-  P.pack(1.0, tau, 3, 0.0, tau_p);
-  P.release(tau);
-  Tensor ttl = P.tmp({o, o, v, v});
-  P.tau(t2, t1, 0.5, 0.5, ttl);                                   // tau_tilde (fac=0.5)
-  Tensor t2ph = P.tmp({o, v, o, v});
-  P.permute(1.0, t2, "ijab", 0.0, t2ph, "iajb", "t2 ph layout");
-
-  // one-body intermediates, CCSD.py:355-387
-  Tensor Fov = P.tmp({o, v});
-  P.axpby(1.0, s.fov, 0.0, Fov);
-  P.contract(1.0, s.oovv_ph, "menf", t1, "nf", 1.0, Fov, "me", "cc_Fov");
-  Tensor Fvv = P.tmp({v, v});
-  P.axpby(1.0, s.fvv, 0.0, Fvv);
-  P.contract(-0.5, s.fov, "me", t1, "ma", 1.0, Fvv, "ae", "cc_Fvv");
-  P.contract_split(-1.0, s.ovvv, "maef", t1, "mf", Fvv, "ae", 'm', "cc_Fvv vovv");
-  P.contract(-0.5, ttl, "mnfa", s.oovv, "mnfe", 1.0, Fvv, "ae", "cc_Fvv tau~");
-  Tensor Foo = P.tmp({o, o});
-  P.axpby(1.0, s.foo, 0.0, Foo);
-  P.contract(0.5, s.fov, "me", t1, "ie", 1.0, Foo, "mi", "cc_Foo");
-  P.contract(1.0, s.ooov, "mnie", t1, "ne", 1.0, Foo, "mi", "cc_Foo ooov");
-  P.contract(0.5, s.oovv, "mnef", ttl, "inef", 1.0, Foo, "mi", "cc_Foo tau~");
-  P.release(ttl);
-  if (shift) {
-    P.diag_add(Fvv, -1.0, s.fock, o);
-    P.diag_add(Foo, -1.0, s.fock, 0);
-  }
-
-  // T1 residual, CCSD.py:288-294
-  P.axpby(1.0, s.fov, 0.0, r1);
-  P.contract(1.0, t1, "ie", Fvv, "ae", 1.0, r1, "ia");
-  P.contract(-1.0, Foo, "mi", t1, "ma", 1.0, r1, "ia");
-  P.contract(1.0, t2ph, "iame", Fov, "me", 1.0, r1, "ia");
-  P.contract(-1.0, s.ovov_ph, "ianf", t1, "nf", 1.0, r1, "ia");
-  if (ovvv_fast(P)) emit_pair_ovvv(P, s, -0.5, t2, r1, "T1 ovvv");
-  else P.contract_split(-0.5, t2, "imef", s.ovvv, "maef", r1, "ia", 'm', "T1 ovvv");
-  P.contract(0.5, t2, "mnea", s.ooov, "mnie", 1.0, r1, "ia");
-
-  // T2 residual, CCSD.py:297-314
-  Tensor x = P.tmp({o, o, v, v});
-  Tensor F1 = P.tmp({v, v});
-  P.axpby(1.0, Fvv, 0.0, F1);
-  P.contract(-0.5, t1, "mb", Fov, "me", 1.0, F1, "be");
-  P.contract(1.0, t2, "ijae", F1, "be", 0.0, x, "ijab");
-  P.axpby(1.0, s.oovv, 0.0, r2);
-  P.axpby(1.0, x, 1.0, r2);
-  P.permute(-1.0, x, "ijba", 1.0, r2, "ijab");
-  P.release(F1);
-  Tensor F2 = P.tmp({o, o});
-  P.axpby(1.0, Foo, 0.0, F2);
-  P.contract(0.5, t1, "je", Fov, "me", 1.0, F2, "mj");
-  P.contract(1.0, F2, "mj", t2, "imab", 0.0, x, "ijab");
-  P.axpby(-1.0, x, 1.0, r2);
-  P.permute(1.0, x, "jiab", 1.0, r2, "ijab");
-  P.release(F2);
-
-  // packed accumulator [ij_p, ab_p]: hh ladder + pp ladder + (t1.ovvv part of Wvvvv)
-  Tensor w4 = P.tmp({o, o, o, o});
-  P.contract(1.0, s.ooov, "mnie", t1, "je", 0.0, w4, "mnij");
-  Tensor Woo_p = P.tmp({po, po});
-  P.axpby(1.0, s.oooo_p, 0.0, Woo_p);
-  P.pack(1.0, w4, 3 | 4, 1.0, Woo_p);
-  P.release(w4);
-  P.contract(1.0, s.oovv_p, "mf", tau_p, "if", 1.0, Woo_p, "mi", "Woooo tau.oovv (K3 folded)");
-  Tensor acc_p = P.tmp({po, pv});
-  P.contract(1.0, Woo_p, "mi", tau_p, "ma", 0.0, acc_p, "ia", "hh ladder");
-  P.release(Woo_p);
-  ladder_dist(P, s, tau_p, acc_p, 1.0, "K1 pp ladder");
-  Tensor Z = P.tmp({po, v, v});
-  if (P.world == 1) {
-    Tensor Y_p = P.tmp({po, o * v});
-    P.contract(-2.0, tau_p, "if", s.ovvv_p2, "qf", 0.0, Y_p, "iq", "R9 Y[ijma]");
-    P.contract(1.0, reshape(Y_p, {po, o, v}), "pma", t1, "mb", 0.0, Z, "pab");
-    P.release(Y_p);
-  } else {
-    Tensor YT = P.tmp_lead_padded({o, v, po});      // Y[ij,m,a] stored [m,a,ij], distributed over m
-    P.contract_lead_dist(-2.0, s.ovvv_p, "maf", tau_p, "if", YT, "mai", "R9 Y[ijma]");
-    P.contract(1.0, YT, "map", t1, "mb", 0.0, Z, "pab");
-    P.release(YT);
-  }
-  P.release(tau_p);
-  P.pack(-0.5, reshape(Z, {po, 1, v, v}), 2 | 4, 1.0, acc_p);
-  P.release(Z);
-  P.unpack(1.0, acc_p, 3, 1.0, r2);
-  P.release(acc_p);
-
-  // ring, CCSD.py:306-310 with Wovvo (CCSD.py:404-413) as W'[(me),(jb)]
-  Tensor Wph = P.tmp_lead_padded({o, v, o, v});
-  emit_wovvo(P, s, t1, t2ph, 0.5, Wph);
-  Tensor ring = P.tmp_lead_padded({o, v, o, v});
-  P.contract_lead_dist(1.0, t2ph, "iame", Wph, "mejb", ring, "iajb", "R2 ring");
-  P.release(Wph);
-  Tensor Q = P.tmp({o, v, o, o});
-  P.contract(1.0, s.ovov_ph, "jbme", t1, "ie", 0.0, Q, "jbmi");
-  P.contract(1.0, t1, "ma", Q, "jbmi", 1.0, ring, "iajb");
-  P.release(Q);
-  add_antisym_ph(P, ring, x, r2);
-  P.release(ring);
-  P.release(t2ph);
-
-  emit_t1_ovvv_term(P, s, t1, x, r2);
-  P.contract(1.0, t1, "ma", s.ooov, "ijmb", 0.0, x, "ijab");
-  P.axpby(-1.0, x, 1.0, r2);
-  P.permute(1.0, x, "ijba", 1.0, r2, "ijab");
-  P.release(x);
-  P.release(Fov);
-  P.release(Fvv);
-  P.release(Foo);
-
-  P.finish(r1, t1, s.fock, (int)o, 2, has_alpha, equation, 0.0, r1);
-  P.finish(r2, t2, s.fock, (int)o, 4, has_alpha, equation, 0.0, r2);
-}
-
-void build_ccsd_lupdate_v1(Plan& P, const Sizes& z, int has_alpha, int equation) {
-  z.apply(P);
-  Slots s(z);
-  const int64_t o = s.o, v = s.v, po = s.po, pv = s.pv;
-  const bool shift = !equation && !has_alpha;  // CCSD.py:449-456 (Q2)
-  const Tensor &t1 = s.t1, &t2 = s.t2, &l1 = s.l1, &l2 = s.l2, &r1 = s.out1, &r2 = s.out2;
-
-  Tensor tau = P.tmp({o, o, v, v});
-  P.tau(t2, t1, 1.0, 1.0, tau);     // antisymmetric part of CCSD.py:565 (all uses contract an antisymmetric pair)
-  Tensor tau_p = P.tmp({po, pv});
-  P.pack(1.0, tau, 3, 0.0, tau_p);
-  Tensor l2_p = P.tmp({po, pv});
-  P.pack(1.0, l2, 3, 0.0, l2_p);
-  Tensor t2ph = P.tmp({o, v, o, v});
-  P.permute(1.0, t2, "ijab", 0.0, t2ph, "iajb", "t2 ph layout");
-  Tensor l2ph = P.tmp({o, v, o, v});
-  P.permute(1.0, l2, "ijab", 0.0, l2ph, "iajb", "l2 ph layout");
-
-  // ---- Linter, CCSD.py:543-623
-  Tensor Fov = P.tmp({o, v});   // = fov1 (:474) = tmp (:504) = (:580)
-  P.axpby(1.0, s.fov, 0.0, Fov);
-  P.contract(1.0, s.oovv_ph, "menf", t1, "nf", 1.0, Fov, "me");
-  Tensor v1 = P.tmp({v, v});
-  P.axpby(1.0, s.fvv, 0.0, v1);
-  P.contract(-1.0, s.fov, "ja", t1, "jb", 1.0, v1, "ba");
-  P.contract_split(-1.0, s.ovvv, "jbac", t1, "jc", v1, "ba", 'j', "v1 ovvv");
-  P.contract(-0.5, tau, "jkcb", s.oovv, "jkca", 1.0, v1, "ba");
-  Tensor v2 = P.tmp({o, o});
-  P.axpby(1.0, s.foo, 0.0, v2);
-  P.contract(1.0, s.fov, "ib", t1, "jb", 1.0, v2, "ij");
-  P.contract(-1.0, s.ooov, "kijb", t1, "kb", 1.0, v2, "ij");
-  P.contract(0.5, s.oovv, "ikbc", tau, "jkbc", 1.0, v2, "ij");
-  P.release(tau);
-
-  Tensor v4ph = P.tmp_lead_padded({o, v, o, v});   // [(kc),(jb)] = v4[j,c,b,k]
-  P.contract_lead_dist(1.0, t2ph, "kcld", s.oovv_ph, "ldjb", v4ph, "kcjb", "R3 v4");
-  P.axpby(-1.0, s.ovov_ph, 1.0, v4ph);
-
-  Tensor v5T = P.tmp({o, v});          // v5T[j,b] = v5[b,j]
-  P.permute(1.0, s.fvo, "bj", 0.0, v5T, "jb");
-  P.contract(1.0, t2ph, "jbkc", s.fov, "kc", 1.0, v5T, "jb");
-  Tensor q = P.tmp({o, o});
-  P.contract(1.0, Fov, "kc", t1, "jc", 0.0, q, "kj");
-  P.contract(1.0, q, "kj", t1, "kb", 1.0, v5T, "jb");
-  P.release(q);
-  P.contract(0.5, s.ooov, "kljc", t2, "klcb", 1.0, v5T, "jb");
-  if (ovvv_fast(P)) emit_pair_ovvv(P, s, -0.5, t2, v5T, "v5 ovvv");
-  else P.contract_split(-0.5, t2, "jkdc", s.ovvv, "kbdc", v5T, "jb", 'k', "v5 ovvv");
-
-  Tensor w3T = P.tmp({o, v});          // w3T[k,c] = w3[c,k]
-  P.axpby(1.0, v5T, 0.0, w3T);
-  P.release(v5T);
-  P.contract(1.0, v4ph, "kcjb", t1, "jb", 1.0, w3T, "kc");
-  P.contract(1.0, t1, "kb", v1, "cb", 1.0, w3T, "kc");
-  P.contract(-1.0, v2, "jk", t1, "jc", 1.0, w3T, "kc");
-
-  // hole-hole pieces, packed [ij_p, kl_p]
-  Tensor woo_p = P.tmp({po, po});
-  P.axpby(0.5, s.oooo_p, 0.0, woo_p);
-  P.contract(0.5, s.oovv_p, "if", tau_p, "kf", 1.0, woo_p, "ik", "v3");
-  Tensor y4 = P.tmp({o, o, o, o});
-  P.contract(1.0, s.ooov, "jilc", t1, "kc", 0.0, y4, "jilk");
-  P.pack(0.5, y4, 3 | 4, 1.0, woo_p);
-  P.release(y4);
-  Tensor lt_p = P.tmp({po, po});
-  P.contract(2.0, l2_p, "if", tau_p, "kf", 0.0, lt_p, "ik", "l2.tau");
-
-  // t1[lc] (oovv[ljbd] t1[kd] - ooov[ljkb]) (CCSD.py:593-597): operands combined first, one K = nocc update of wph
-  Tensor S = P.tmp({o, o, o, v});
-  P.axpby(-1.0, s.ooov, 0.0, S);
-  P.contract(1.0, s.oovv, "ljbd", t1, "kd", 1.0, S, "ljkb");
-  Tensor wph = P.tmp({o, v, o, v});    // wovvo as [(kc),(jb)]
-  P.axpby(1.0, v4ph, 0.0, wph);
-  P.contract(1.0, t1, "lc", S, "ljkb", 1.0, wph, "kcjb");
-  P.release(S);
-  if (P.world == 1) {
-    P.contract(1.0, s.ovvv, "jcbd", t1, "kd", 1.0, wph, "kcjb");
-  } else {
-    Tensor wj = P.tmp_lead_padded({o, v, v, o});
-    P.contract_lead_dist(1.0, s.ovvv, "jcbd", t1, "kd", wj, "jcbk", "wovvo ovvv.t1 (distributed over j)");
-    P.permute(1.0, wj, "jcbk", 1.0, wph, "kcjb");
-    P.release(wj);
-  }
-
-  Tensor wo_p = P.tmp_lead_padded({o, v, po});
-  P.contract_lead_dist(0.5, s.ovvv_p, "icf", tau_p, "kf", wo_p, "ick", "R4 wovoo");
-  P.release(tau_p);
-  Tensor wovoo = P.tmp({o, v, o, o});
-  P.unpack(1.0, reshape(wo_p, {o * v, po}), 2, 0.0, wovoo);
-  P.release(wo_p);
-  P.permute(0.5, s.ooov, "jkic", 1.0, wovoo, "icjk");
-  P.contract(1.0, v4ph, "kcib", t1, "jb", 1.0, wovoo, "icjk");
-  P.contract(-1.0, t2ph, "kclb", s.ooov, "lijb", 1.0, wovoo, "icjk", "wovoo ooov.t2");
-
-  // ---- m3, CCSD.py:461-470, packed [ij_p, ab_p]
-  Tensor m3_p = P.tmp({po, pv});
-  P.contract(2.0, woo_p, "ik", l2_p, "ka", 0.0, m3_p, "ia", "l2.woooo");
-  P.release(woo_p);
-  P.contract(0.5, lt_p, "ik", s.oovv_p, "ka", 1.0, m3_p, "ia");
-  Tensor l2t1 = P.tmp({o, o, v, o});
-  P.contract(1.0, l2, "ijcd", t1, "kd", 0.0, l2t1, "ijck");
-  Tensor a_full = P.tmp({o, o, o, v});
-  P.permute(1.0, l2t1, "ijck", 0.0, a_full, "ijkc");
-  Tensor a_p = P.tmp({po, o * v});
-  P.pack(1.0, reshape(a_full, {o, o, o * v, 1}), 1, 0.0, a_p);
-  P.release(a_full);
-  if (P.world == 1) {
-    P.contract(1.0, a_p, "pq", s.ovvv_p2, "qa", 1.0, m3_p, "pa", "R6 ovvv.(l2 t1)");
-  } else {
-    Tensor r6 = P.tmp_lead_padded({po, pv});
-    P.contract_lead_dist(1.0, a_p, "pq", s.ovvv_p2, "qa", r6, "pa", "R6 ovvv.(l2 t1)");
-    P.axpby(1.0, r6, 1.0, m3_p);
-    P.release(r6);
-  }
-  P.release(a_p);
-  ladder_dist(P, s, l2_p, m3_p, 1.0, "K2 pp ladder");
-  P.release(l2_p);
-  Tensor m3 = P.tmp({o, o, v, v});
-  P.unpack(1.0, m3_p, 3, 0.0, m3);
-  P.release(m3_p);
-
-  Tensor m_vv = P.tmp({v, v});
-  P.contract(0.5, t2, "klcb", l2, "klca", 0.0, m_vv, "ba");
-  Tensor m_oo = P.tmp({o, o});
-  P.contract(0.5, l2, "kicd", t2, "kjcd", 0.0, m_oo, "ij");
-  Tensor x_vv = P.tmp({v, v});
-  P.axpby(1.0, m_vv, 0.0, x_vv);
-  P.contract(1.0, l1, "ka", t1, "kb", 1.0, x_vv, "ba");
-  Tensor x_oo = P.tmp({o, o});
-  P.axpby(1.0, m_oo, 0.0, x_oo);
-  P.contract(1.0, l1, "ic", t1, "kc", 1.0, x_oo, "ik");
-  if (shift) {  // after w3 (which uses the unshifted v1, v2)
-    P.diag_add(v1, -1.0, s.fock, o);
-    P.diag_add(v2, -1.0, s.fock, 0);
-  }
-
-  // ---- L2 residual, CCSD.py:472-488
-  P.axpby(1.0, s.oovv, 0.0, r2);
-  P.axpby(1.0, m3, 1.0, r2);
-  Tensor ring = P.tmp_lead_padded({o, v, o, v});
-  P.contract_lead_dist(1.0, l2ph, "iakc", wph, "kcjb", ring, "iajb", "R7 ring");
-  P.release(wph);
-  P.contract(1.0, l1, "ia", Fov, "jb", 1.0, ring, "iajb");
-  Tensor y = P.tmp({o, o, v, v});
-  add_antisym_ph(P, ring, y, r2);
-  P.release(ring);
-  P.contract(1.0, l1, "ka", s.ooov, "ijkb", 0.0, y, "ijab");
-  P.contract(-1.0, l2, "ijac", v1, "cb", 1.0, y, "ijab");
-  P.contract(-1.0, s.oovv, "ijbc", x_vv, "ca", 1.0, y, "ijab");     // oovv[ijcb] = -oovv[ijbc] (Eris.py:128)
-  P.axpby(-1.0, y, 1.0, r2);
-  P.permute(1.0, y, "ijba", 1.0, r2, "ijab");
-  if (ovvv_fast(P)) {
-    // y[pqrs] = sum_c l1[qc] ovvv[pcrs]: yp[q,p,rs_p] from the planes, expanded with the (p,q) view of y
-    Tensor yp = P.tmp({o * o, s.pv});
-    emit_t1_ovvv_packed(P, s, 1.0, l1, yp, "l1.ovvv (packed pair, INT8)");
-    Tensor yT = y;
-    std::swap(yT.str[0], yT.str[1]);
-    P.unpack(1.0, yp, 2, 0.0, yT);
-    P.release(yp);
-  } else if (P.world == 1) {
-    P.contract(1.0, l1, "qc", s.ovvv, "pcrs", 0.0, y, "pqrs");
-  } else {
-    Tensor yp = P.tmp_lead_padded({o, o, v, v});
-    P.contract_lead_dist(1.0, s.ovvv, "pcrs", l1, "qc", yp, "pqrs", "l1.ovvv (distributed over p)");
-    P.axpby(1.0, yp, 0.0, y);
-    P.release(yp);
-  }
-  P.contract(1.0, v2, "qk", l2, "kprs", 1.0, y, "pqrs");
-  P.contract(-1.0, x_oo, "pk", s.oovv, "kqrs", 1.0, y, "pqrs");
-  P.axpby(1.0, y, 1.0, r2);
-  P.permute(-1.0, y, "qprs", 1.0, r2, "pqrs");
-  P.release(y);
-
-  // ---- L1 residual, CCSD.py:490-506
-  P.axpby(1.0, s.fov, 0.0, r1);
-  P.contract(-1.0, s.ovov_ph, "jbia", l1, "jb", 1.0, r1, "ia");
-  P.contract(1.0, l1, "ib", v1, "ba", 1.0, r1, "ia");
-  P.contract(-1.0, v2, "ij", l1, "ja", 1.0, r1, "ia");
-  P.contract(-1.0, wovoo, "icjk", l2, "kjca", 1.0, r1, "ia");
-  P.release(wovoo);
-  // -(l2 . wvvvo) with wvvvo never formed (four pieces):
-  P.contract(1.0, l2t1, "ikcj", v4ph, "kcja", 1.0, r1, "ia", "wvvvo: v4.t1");
-  P.release(l2t1);
-  P.release(v4ph);
-  Tensor lt = P.tmp({o, o, o, o});
-  P.unpack(1.0, lt_p, 3, 0.0, lt);
-  P.release(lt_p);
-  P.contract(-0.25, lt, "ikjl", s.ooov, "jlka", 1.0, r1, "ia", "wvvvo: ooov.tau");
-  P.release(lt);
-  if (ovvv_fast(P)) emit_pair_ovvv(P, s, -0.5, l2, r1, "wvvvo: ovvv");
-  else P.contract_split(-0.5, l2, "ikbc", s.ovvv, "kabc", r1, "ia", 'k', "wvvvo: ovvv");
-  Tensor Xph = P.tmp_lead_padded({o, v, o, v});
-  P.contract_lead_dist(1.0, l2ph, "ibjc", t2ph, "jckd", Xph, "ibkd", "R8 l2.t2");
-  P.contract_split(1.0, Xph, "ibkd", s.ovvv, "kbda", r1, "ia", 'k', "wvvvo: ovvv.t2 (K4 refactored)");
-  P.release(Xph);
-  P.contract(1.0, m3, "ijab", t1, "jb", 1.0, r1, "ia");
-  P.release(m3);
-  P.contract(1.0, l2ph, "iajb", w3T, "jb", 1.0, r1, "ia");
-  P.release(l2ph);
-  Tensor zz = P.tmp({o, v});
-  P.axpby(1.0, t1, 0.0, zz);
-  P.contract(1.0, t2ph, "jbkc", l1, "kc", 1.0, zz, "jb");
-  P.release(t2ph);
-  P.contract(-1.0, x_vv, "bd", t1, "jd", 1.0, zz, "jb");
-  P.contract(-1.0, m_oo, "lj", t1, "lb", 1.0, zz, "jb");
-  P.contract(1.0, s.oovv_ph, "iajb", zz, "jb", 1.0, r1, "ia");
-  P.release(zz);
-  P.contract_split(-1.0, s.ovvv, "icba", x_vv, "bc", r1, "ia", 'c', "L1 ovvv.x_vv");
-  P.contract(-1.0, s.ooov, "jika", x_oo, "kj", 1.0, r1, "ia");
-  P.contract(-1.0, m_oo, "ik", Fov, "ka", 1.0, r1, "ia");
-  P.contract(-1.0, m_vv, "ca", Fov, "ic", 1.0, r1, "ia");
-
-  if (shift) {  // energy term, CCSD.py:509-510
-    Tensor f = P.tmp({o, v});
-    P.axpby(1.0, s.fov, 0.0, f);
-    emit_energy(P, s, f, 0);
-    P.release(f);
-    P.scale_dev(r1, 1.0, -1.0, 0);
-    P.scale_dev(r2, 1.0, -1.0, 0);
-  }
-  P.release(Fov); P.release(v1); P.release(v2); P.release(w3T);
-  P.release(m_vv); P.release(m_oo); P.release(x_vv); P.release(x_oo);
-
-  P.finish(r1, l1, s.fock, (int)o, 2, has_alpha, equation, 0.0, r1);
-  P.finish(r2, l2, s.fock, (int)o, 4, has_alpha, equation, 0.0, r2);
 }
 
 // ======================================================================

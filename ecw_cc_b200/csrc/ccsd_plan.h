@@ -18,9 +18,6 @@ struct Sizes {
   // their per-call cuts and the ovvv-streaming terms with a contracted or free antisymmetric pair run on the INT8
   // pipe as batched products (needs nocc % 8 == 0 and nvir % 8 == 0: sub-blocks start on 8-row groups)
   bool ovvv_planes = false;
-  // packed-path lowering: false = ccsd_plan_slab.cpp (o^2v^2 work on slabs of the leading occupied index, fused
-  // antisymmetriser), true = the round-1 builders (ccsd_plan.cpp, *_v1) — kept for A/B measurements and tests
-  bool legacy_packed = false;
   int64_t cut_cache_min_elems = 1 << 20;   // operands at least this large keep their digit planes for a second use
   void apply(Plan& P) const {
     P.rank = rank; P.world = world;
@@ -36,8 +33,6 @@ struct Sizes {
 // (CCSD.py:248, :419): has_alpha <=> `alpha is not None`, equation <=> `equation=True`.
 void build_ccsd_tupdate(Plan& P, const Sizes& z, int has_alpha, int equation);
 void build_ccsd_lupdate(Plan& P, const Sizes& z, int has_alpha, int equation);
-void build_ccsd_tupdate_v1(Plan& P, const Sizes& z, int has_alpha, int equation);
-void build_ccsd_lupdate_v1(Plan& P, const Sizes& z, int has_alpha, int equation);
 // general variants: amplitudes not assumed antisymmetric (only the integrals are)
 void build_ccsd_tupdate_general(Plan& P, const Sizes& z, int has_alpha, int equation);
 void build_ccsd_lupdate_general(Plan& P, const Sizes& z, int has_alpha, int equation);

@@ -66,8 +66,8 @@ inline void emit_energy(Plan& P, const Slots& s, const Tensor& fov_dense, int k)
   P.release(G);
 }
 
-// Wph[(me),(jb)] = Wovvo[m,b,e,j] (CCSD.py:404-413) for the rows m in [m0, m0+nm); `t2x`/`c2` give the
-// t2 operand of the o^3v^3 term: (t2ph, +1/2) on the packed path, (t2ph2, -1/2) on the general path.
+// Wph[(me),(jb)] = Wovvo[m,b,e,j] (CCSD.py:404-413) for the rows m in [m0, m0+nm); `t2x`/`c2` are the
+// t2 operand of the o^3v^3 term and its coefficient (the general path passes t2ph2, -1/2).
 inline void emit_wovvo_rows(Plan& P, const Slots& s, const Tensor& t1, const Tensor& t2x, double c2, const Tensor& Wph,
                      int64_t m0, int64_t nm) {
   const int64_t o = s.o, v = s.v;

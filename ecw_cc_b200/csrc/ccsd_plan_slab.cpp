@@ -1,9 +1,8 @@
-// ccsd_plan_slab.cpp — the packed (antisymmetric-amplitude) T and Lambda plans, round-2 lowering.
+// ccsd_plan_slab.cpp — the packed (antisymmetric-amplitude) T and Lambda plans.
 //
-// Same equations as the round-1 builders (reference: CCSD.py:248-338 tupdate, :346-413 T intermediates, :419-535
-// lupdate, :543-623 Linter; identities of oracle/refactored_np.py), organised so that every o^2v^2-sized piece of work
-// is done on a SLAB — the rows [i0, i0+ni) of the leading occupied index that belong to this rank — and only small or
-// packed tensors are replicated:
+// The contractions of oracle/refactored_np.py (reference: CCSD.py:248-338 tupdate, :346-413 T intermediates, :419-535
+// lupdate, :543-623 Linter), organised so that every o^2v^2-sized piece of work is done on a SLAB — the rows
+// [i0, i0+ni) of the leading occupied index that belong to this rank — and only small or packed tensors are replicated:
 //
 //   * The amplitudes are replicated INPUTS, so any layout or slice of them (t2ph, l2ph, packed pairs, slabs) is
 //     produced locally at HBM speed; nothing of them is ever exchanged.
@@ -98,7 +97,6 @@ void t1_ovvv_rows(Plan& P, const Slots& s, double alpha, const Tensor& amp1, con
 
 // ======================================================================================================= T1 / T2
 void build_ccsd_tupdate(Plan& P, const Sizes& z, int has_alpha, int equation) {
-  if (z.legacy_packed) { build_ccsd_tupdate_v1(P, z, has_alpha, equation); return; }
   z.apply(P);
   Slots s(z);
   const int64_t o = s.o, v = s.v, po = s.po, pv = s.pv;
@@ -309,7 +307,6 @@ void build_ccsd_tupdate(Plan& P, const Sizes& z, int has_alpha, int equation) {
 
 // ======================================================================================================= L1 / L2
 void build_ccsd_lupdate(Plan& P, const Sizes& z, int has_alpha, int equation) {
-  if (z.legacy_packed) { build_ccsd_lupdate_v1(P, z, has_alpha, equation); return; }
   z.apply(P);
   Slots s(z);
   const int64_t o = s.o, v = s.v, po = s.po, pv = s.pv;

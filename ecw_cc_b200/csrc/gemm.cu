@@ -415,11 +415,11 @@ int gemm_pick_config(int64_t M, int64_t N, int64_t K) {
   // 12: 48x128  13: 128x48 — one tile covers a whole occupied index of up to 48 (no operand re-read)
   // 14: 40x40  15: 48x48 — both extents an occupied index
   // 16: 128x40 — N an occupied index of 33..40 (ovvv.t1 products: no DMMA work on padding columns)
-  // 17: 40x200 — measured slower than 48x128 for ovvv.t2 (5 warps per SM do not cover the loads); kept for A/B only
-  // 22: 40x80 — like 17 measured slower than 48x128 on ovvv.t2 (16.2 vs 12.5 ms): five-warp CTAs; A/B only
   // 18: 40x128  19: 80x80, both with BK = 8 and six stages — short-K rank updates (see below)
   // (tried and dropped: issuing the old-C loads of a short-K tile before the operand wait — 2-3x slower, gemm per-op
   //  logs profiles/r2_perop_dmma_variants.md)
+  // (tried and dropped: 40x200 and 40x80 tiles for ovvv.t2 — five-warp CTAs do not cover the loads, slower than 48x128:
+  //  17.6 vs 13.2 ms and 16.2 vs 12.5 ms; the 40x200 run is in profiles/r2_perop_dmma_variants.md)
   if (N <= 8) return 3;
   auto padded = [](int64_t x, int64_t b) { return (x + b - 1) / b * b; };
   if (K > 0 && K <= 40 && K % 8 == 0 && N >= 80) {
@@ -447,9 +447,10 @@ int gemm_pick_config(int64_t M, int64_t N, int64_t K) {
 }
 
 void gemm_tile_of(int64_t M, int64_t N, int64_t K, int* bm, int* bn) {
-  static const int dims[23][2] = {{128, 128}, {32, 128}, {128, 32}, {128, 8}, {64, 64}, {128, 128}, {128, 128}, {128, 128},
-                                  {128, 128}, {128, 128}, {112, 128}, {96, 128}, {48, 128}, {128, 48}, {40, 40}, {48, 48},
-                                  {128, 40}, {40, 200}, {40, 128}, {80, 80}, {128, 128}, {112, 128}, {40, 80}};
+  // indexed by the configurations gemm_pick_config returns; {0, 0}: numbers it never returns
+  static const int dims[20][2] = {{0, 0}, {32, 128}, {128, 32}, {128, 8}, {64, 64}, {0, 0}, {0, 0}, {0, 0},
+                                  {128, 128}, {0, 0}, {112, 128}, {96, 128}, {48, 128}, {128, 48}, {40, 40}, {48, 48},
+                                  {128, 40}, {0, 0}, {40, 128}, {80, 80}};
   const int cfg = gemm_pick_config(M, N, K);
   *bm = dims[cfg][0];
   *bn = dims[cfg][1];
@@ -471,13 +472,8 @@ cudaError_t launch_gemm(const GemmArgs& args, cudaStream_t st, int force_cfg) {
     return launch_gemv(p, st);
   int cfg = force_cfg >= 0 ? force_cfg : gemm_pick_config(p.M, p.N, p.kchunk);
   // large aligned problems: TMA producer + mbarrier ring + DMMA consumers (gemm_tma.cu)
-#ifdef ECW_OZ_EXPERIMENT
-  static const bool no_tma = getenv("ECW_NO_TMA") != nullptr;      // experiment builds only (tools/)
-#else
-  constexpr bool no_tma = false;
-#endif
   const bool tma_cfg = cfg == 20 || cfg == 21;
-  if (tma_cfg || (force_cfg < 0 && !no_tma && (cfg == 8 || cfg == 10 || cfg == 11))) {
+  if (tma_cfg || (force_cfg < 0 && (cfg == 8 || cfg == 10 || cfg == 11))) {
     if (gemm_tma_eligible(p)) {
       int tcfg = tma_cfg ? cfg : ((cfg != 8 && p.ta == 0) ? 21 : 20);
       cudaError_t e = launch_gemm_tma(p, st, tcfg);
@@ -487,16 +483,11 @@ cudaError_t launch_gemm(const GemmArgs& args, cudaStream_t st, int force_cfg) {
     if (tma_cfg) cfg = 8;
   }
   switch (cfg) {
-    case 0: return launch_cfg<128, 128, 32, 32, 16, 4, 0>(p, st);
     case 1: return launch_cfg<32, 128, 16, 32, 16, 4, 0>(p, st);
     case 2: return launch_cfg<128, 32, 32, 16, 16, 4, 0>(p, st);
     case 3: return launch_cfg<128, 8, 16, 8, 16, 4, 0>(p, st);
     case 4: return launch_cfg<64, 64, 32, 16, 16, 4, 0>(p, st);
-    case 5: return launch_cfg<128, 128, 64, 32, 16, 4, 0>(p, st);
-    case 6: return launch_cfg<128, 128, 64, 32, 16, 4, 1>(p, st);
-    case 7: return launch_cfg<128, 128, 64, 32, 32, 3, 1>(p, st);
     case 8: return launch_cfg<128, 128, 32, 32, 16, 4, 1>(p, st);
-    case 9: return launch_cfg<128, 128, 32, 32, 32, 3, 1>(p, st);
     case 10: return launch_cfg<112, 128, 56, 32, 16, 4, 1>(p, st);
     case 12: return launch_cfg<48, 128, 48, 16, 16, 4, 1>(p, st);
     case 13: return launch_cfg<128, 48, 32, 24, 16, 4, 1>(p, st);
@@ -504,10 +495,8 @@ cudaError_t launch_gemm(const GemmArgs& args, cudaStream_t st, int force_cfg) {
     case 14: return launch_cfg<40, 40, 40, 8, 16, 4, 1>(p, st);
     case 15: return launch_cfg<48, 48, 48, 8, 16, 4, 1>(p, st);
     case 16: return launch_cfg<128, 40, 32, 40, 16, 4, 1>(p, st);
-    case 17: return launch_cfg<40, 200, 40, 40, 16, 3, 1>(p, st);
     case 18: return launch_cfg<40, 128, 40, 16, 8, 6, 1>(p, st);
     case 19: return launch_cfg<80, 80, 40, 40, 8, 6, 1>(p, st);
-    case 22: return launch_cfg<40, 80, 40, 16, 16, 4, 1>(p, st);
     default: return cudaErrorInvalidValue;
   }
 }

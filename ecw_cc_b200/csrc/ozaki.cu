@@ -39,13 +39,12 @@
 //                    N = TN (NS-p) columns (split at 256);
 //   warps 2-5      : epilogue — tcgen05.ld the NS accumulators, Horner in FP64, rank-one terms, scales,
 //                    alpha/beta, store (coalesced across lanes when the tile rows are contiguous in C).
-// Measured limiter (tools/oz_experiment.py, profiles/r1_oz_limiter.md): a stage is 39.9 KB and 840 clk of MMA
+// Measured limiter (profiles/r1_oz_limiter.md): a stage is 39.9 KB and 840 clk of MMA
 // (47 B/clk); an SM ingests ~32.6 B/clk from L2 whatever the path (bulk TMA, cp.async, both), so the main loop
 // runs at 1224 clk per stage = 69 % of the pipe; without loads it reaches 87 %.  TMEM (NS accumulators x TN
 // columns <= 512) is what keeps the tile, and with it the bytes per MAC, from growing.
 #include <cuda.h>
 #include <cstdio>
-#include <cstdlib>
 
 #include "kernels.h"
 
@@ -141,10 +140,6 @@ struct OzGemmParams {
   uint32_t lbo, sbo;     // descriptor strides (bytes)
   // batch b = 0..batch-1 of independent products (OzBatch, kernels.h)
   OzBatch bt;
-#ifdef ECW_OZ_EXPERIMENT
-  int debug;             // tools/oz_experiment.py only (never in the product build): bit 0 = the producer skips the
-                         // loads (MMA on stale data), bit 1 / 2 = A / B planes only, bit 4 = 15 of the 21 products
-#endif
 };
 
 // tile columns: NS accumulators of TN int32 columns must fit the 512 TMEM columns; every MMA needs N % 16 == 0
@@ -230,18 +225,6 @@ __global__ void __launch_bounds__(192, 1) ozaki_gemm_kernel(OzGemmParams p) {
           const uint32_t st = it % STAGES, use = it / STAGES;
           mbar_wait(&empty[st], (use & 1) ^ 1);
           unsigned char* s = smem + st * Cfg::STAGE;
-#ifdef ECW_OZ_EXPERIMENT
-          if (p.debug & 1) { mbar_arrive(&full[st]); continue; }
-          if (p.debug & 6) {           // experiments: bit 1 = A planes only, bit 2 = B planes only
-            mbar_expect_tx(&full[st], NS * ((p.debug & 2) ? Cfg::A_PLANE : Cfg::B_PLANE));
-#pragma unroll
-            for (int d = 0; d < NS; ++d) {
-              if (p.debug & 2) bulk_load(s + d * Cfg::A_PLANE, ga + ((int64_t)kb * NS + d) * a_slab, Cfg::A_PLANE, &full[st]);
-              else bulk_load(s + NS * Cfg::A_PLANE + d * Cfg::B_PLANE, gb + ((int64_t)kb * NS + d) * b_slab, Cfg::B_PLANE, &full[st]);
-            }
-            continue;
-          }
-#endif
           mbar_expect_tx(&full[st], Cfg::STAGE);
 #pragma unroll
           for (int d = 0; d < NS; ++d) {
@@ -276,9 +259,6 @@ __global__ void __launch_bounds__(192, 1) ozaki_gemm_kernel(OzGemmParams p) {
             // pd .. NS-1, which are contiguous too.  One MMA per <= 256 columns.
 #pragma unroll
             for (int pd = 0; pd < NS; ++pd) {
-#ifdef ECW_OZ_EXPERIMENT
-              if ((p.debug & 16) && pd >= 3) continue;        // experiment: 15 of the 21 products
-#endif
               const uint64_t adesc = desc0 | (uint64_t)(((sa + pd * Cfg::A_PLANE) >> 4) & 0x3fff);
               const int ncols = TN * (NS - pd);
 #pragma unroll
@@ -698,10 +678,6 @@ cudaError_t launch_ozaki_gemm_batched(const int8_t* pa, const double* sa, int64_
   p.bt = bt;
   if (bt.batch < 1 || ((bt.a_row0 | bt.a_rowb | bt.b_row0 | bt.b_rowb) & 7)) return cudaErrorInvalidValue;
   if (sm_count <= 0) sm_count = 148;
-#ifdef ECW_OZ_EXPERIMENT
-  if (const char* e = getenv("ECW_OZ_DEBUG")) p.debug = atoi(e);
-  if (const char* e = getenv("ECW_OZ_GRID")) sm_count = atoi(e);
-#endif
   switch (ns) {
     case 3: return launch_gemm_ns<3>(p, st, sm_count);
     case 4: return launch_gemm_ns<4>(p, st, sm_count);

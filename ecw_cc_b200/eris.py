@@ -106,9 +106,6 @@ class DeviceEris(object):
             raise EcwError("ecw_ctx_create failed")
         if self.world > 1 and lib.ecw_ctx_set_shard(self._h, self.rank, self.world) != 0:
             raise EcwError("ecw_ctx_set_shard failed")
-        # experiments: ECW_PLAN_VARIANT=legacy selects the round-1 lowering of the packed plans (include/ecw_b200.h)
-        if os.environ.get("ECW_PLAN_VARIANT", "") == "legacy":
-            self.check(lib.ecw_ctx_set_plan_variant(self._h, 1), "ecw_ctx_set_plan_variant")
         self.int8_digits, self.int8_min_flops = _gemm_config(gemm, int8_digits, int8_min_flops, self.nvir, eri_max)
         self.check(lib.ecw_ctx_set_gemm(self._h, self.int8_digits, self.int8_min_flops), "ecw_ctx_set_gemm")
         # constant digit planes of ovvv_p (both orientations): sub-blocks of a plane set start on 8-row groups

@@ -82,10 +82,6 @@ int ecw_ctx_get_gemm(ecw_ctx* ctx);
  * exceeds its tolerance (ecw_cc_b200/eris.py: INT8_TOL); 0 restores the configured engine. */
 int ecw_int8_error_bound(ecw_ctx* ctx, double* bound_out, void* stream);
 int ecw_ctx_set_engine_override(ecw_ctx* ctx, int force_dmma);
-/* Lowering of the antisymmetric-amplitude (packed) T / Lambda plans: 0 (default) = o^2v^2 work on slabs of the leading
- * occupied index with one fused antisymmetriser (csrc/ccsd_plan_slab.cpp), 1 = the round-1 lowering with replicated
- * intermediates (csrc/ccsd_plan.cpp) — kept for A/B measurements. */
-int ecw_ctx_set_plan_variant(ecw_ctx* ctx, int legacy_packed);
 /* INT8 products with fewer output tiles than SMs and a contraction length >= min_k (a multiple of 32) are cut into
  * equal K chunks, one product each, summed in a fixed order (default 65536; <= 0: never). */
 int ecw_ctx_set_int8_splitk(ecw_ctx* ctx, int64_t min_k);
@@ -309,7 +305,9 @@ double ecw_plan_flops(ecw_ctx* ctx, const char* func, int mode_flags);
 int64_t ecw_plan_launches(ecw_ctx* ctx, const char* func, int mode_flags);
 /* Raw FP64 tensor-core GEMM: C = alpha op(A) op(B) + beta C (row-major C);
  * ta/tb: 0 = A is [M,K] / B is [K,N] row-major, 1 = transposed storage.
- * cfg < 0 picks the tile configuration automatically. */
+ * cfg < 0 picks the tile configuration automatically; cfg = 1-4, 8, 10-16, 18 or 19 forces one of the DMMA tiles
+ * the picker chooses from (csrc/gemm.cu, gemm_pick_config), 20 / 21 the TMA-fed 128x128 / 112x128 tiles (the 128x128
+ * DMMA tile where TMA does not apply).  Any other cfg returns non-zero without launching. */
 int ecw_dgemm(int ta, int tb, int64_t M, int64_t N, int64_t K, double alpha, const double* A, int64_t lda,
               const double* B, int64_t ldb, double beta, double* C, int64_t ldc, int cfg, void* stream);
 /* FP64 GEMM on the INT8 tcgen05 tensor pipe (csrc/ozaki.cu: operands cut into base-256 int8 digits).

@@ -23,7 +23,7 @@ def _dev(x):
     return torch.from_numpy(np.ascontiguousarray(x)).cuda()
 
 
-@pytest.mark.parametrize("cfg", [-1, 0, 1, 2, 3, 4, 5, 6, 7, 8, 9, 10, 11, 12, 13, 14, 15, 16, 17, 18, 19, 20, 21, 22])
+@pytest.mark.parametrize("cfg", [-1, 1, 2, 3, 4, 8, 10, 11, 12, 13, 14, 15, 16, 18, 19, 20, 21])
 @pytest.mark.parametrize("ta,tb", [(0, 0), (0, 1), (1, 0), (1, 1)])
 def test_dgemm_all_layouts(ecw, cfg, ta, tb):
     import torch
@@ -43,6 +43,19 @@ def test_dgemm_all_layouts(ecw, cfg, ta, tb):
         assert rc == 0
         err = np.abs(dC.cpu().numpy() - ref).max()
         assert err < 1e-11 * max(1.0, K ** 0.5), (M, N, K, err)
+
+
+def test_dgemm_refuses_unknown_config(ecw):
+    """Configuration numbers without a tile (those the picker never chooses) are refused, and C is left untouched."""
+    import torch
+    M, N, K = 40, 400, 64
+    dA, dB = _dev(np.ones((M, K))), _dev(np.ones((K, N)))
+    dC = _dev(np.full((M, N), 3.0))
+    for cfg in (0, 5, 6, 7, 9, 17, 22):
+        rc = ecw.lib.ecw_dgemm(0, 0, M, N, K, 1.0, dA.data_ptr(), K, dB.data_ptr(), N, 0.0, dC.data_ptr(), N, cfg,
+                               torch.cuda.current_stream().cuda_stream)
+        assert rc != 0, cfg
+    assert bool((dC == 3.0).all())
 
 
 def test_dgemm_strided_views(ecw):

@@ -242,22 +242,3 @@ def test_non_finite_amplitudes_propagate(ecw, engine):
         assert np.isnan(b).any() and np.isnan(a).any()
         assert np.isnan(cc.gamma(t1, x, l1, l2)).any()
 
-
-def test_slab_lowering_equals_round1_lowering(ecw, monkeypatch):
-    """The packed plans of csrc/ccsd_plan_slab.cpp (slabs + fused antisymmetriser) against the round-1 builders kept
-    behind ecw_ctx_set_plan_variant, same inputs, at a size with many tiles: equal to rounding."""
-    import torch
-    o, v = 16, 96
-    res = {}
-    for variant in ("", "legacy"):
-        monkeypatch.setenv("ECW_PLAN_VARIANT", variant)
-        de = ecw.DeviceEris.synthetic(o, v, gemm="dmma")
-        cc = ecw.GCC(de)
-        t1, t2 = de.synth_tensor("t1", (o, v)), de.synth_tensor("t2", (o, o, v, v))
-        l1, l2 = de.synth_tensor("l1", (o, v)), de.synth_tensor("l2", (o, o, v, v))
-        fsp = de.synth_tensor("fsp", (o + v, o + v))
-        res[variant] = cc.tupdate(t1, t2, fsp=fsp) + cc.lupdate(t1, t2, l1, l2, fsp=fsp, alpha=1e-3)
-        n_asym = cc.plan_json("tupdate").count('"asym4"')
-        assert n_asym == (0 if variant else 1)
-    for x, y in zip(res[""], res["legacy"]):
-        assert float((x - y).abs().max()) < 1e-12
