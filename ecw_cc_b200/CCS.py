@@ -18,7 +18,7 @@ device, so the update that follows does not upload them again.
 import numpy as np
 
 from ._lib import lib, EcwError, ECW_HAS_ALPHA, ECW_SUBDIFF_SINGLES
-from .devops import DevOps, _scalar
+from .devops import ArgBlocks, _scalar
 from .eris import DeviceEris
 
 
@@ -48,26 +48,15 @@ class Gccs(object):
         self.fock = np.asarray(eris.fock) if fock is None else fock  # CCS.py:212-215
         self.nocc = eris.nocc
         self.nvir = self.fock.shape[0] - self.nocc
-        self.ops = DevOps(eris)
-        o, v = self.nocc, self.nvir
-        b = eris.buf
-        self._ooov = b["ooov"][: o * o * o * v].view(o, o, o, v)
-        self._oovv = b["oovv"][: o * o * v * v].view(o, o, v, v)
-        self._ovvv = b["ovvv"][: o * v * v * v].view(o, v, v, v)
-        self._ovov_ph = b["ovov_ph"][: o * v * o * v].view(o, v, o, v)
+        self.ops = eris.ops
+        self._blocks = None           # ArgBlocks of _inter
         if fock is not None:
             eris.set_fock(fock)
 
     # ------------------------------------------------------------------ helpers
-    def _f(self, fsp):
-        """Device copy of the one-body operator and its four blocks (views)."""
-        o = self.nocc
-        F = self.eris.fock_dev if fsp is None else self.ops.to_dev(fsp)
-        return F[:o, :o], F[:o, o:], F[o:, :o], F[o:, o:]
-
     def _G(self, ts):
         """G[jb] = sum_kc ts[kc] oovv[jkbc]"""
-        return self.ops.contract('kc,jkbc->jb', ts, self._oovv)
+        return self.ops.contract('kc,jkbc->jb', ts, self.eris.block("oovv"))
 
     def _w_dev(self, inter, idx, shape):
         """Device copy of the o^2v^2 member of an intermediate tuple (cached when it is ours)."""
@@ -82,6 +71,17 @@ class Gccs(object):
         t.dev = {"W": W_dev, "host_id": id(host_items[w_index])}
         return t
 
+    def _q6(self, Fv_h, Fo_h):
+        """Q6: an update subtracts the Fock diagonal from the vv and oo blocks of its intermediate tuple IN PLACE, so
+        the caller's arrays change as in the reference.  Returns the shifted device copies."""
+        ops = self.ops
+        Fv, Fo = ops.to_dev(Fv_h), ops.to_dev(Fo_h)
+        ops.diag_shift(Fv, -1.0, self.nocc)
+        ops.diag_shift(Fo, -1.0, 0)
+        Fv_h[...] = ops.to_host(Fv)
+        Fo_h[...] = ops.to_host(Fo)
+        return Fv, Fo
+
     def _inter(self, func, ts, fsp, vm=None, e_term=True):
         """One of the four intermediate builders as ONE call of the C ABI (ecw_ccs_t1inter / l1inter / r1inter /
         esl1inter: a cached plan, replayed as a CUDA graph).  The arguments go through persistent device blocks so that
@@ -89,19 +89,16 @@ class Gccs(object):
         or None, scalar or None) — F and X are views of the persistent blocks (read them before the next call), W is a
         fresh tensor (it is cached for the update that follows)."""
         ops = self.ops
-        torch = ops.torch
         e = self.eris
         o, v = self.nocc, self.nvir
         n = o + v
-        st = getattr(self, "_ccs_blocks", None)
+        st = self._blocks
         if st is None:
-            mk = lambda *shape: torch.empty(shape, dtype=torch.float64, device=e.device)      # noqa: E731
-            st = self._ccs_blocks = dict(ts=mk(o, v), fsp=mk(n, n), vm=mk(n, n), F=mk(n, n), W=mk(v, o, o, v), X=mk(o, v),
-                                         e=mk(1))
-        st["ts"].copy_(ops.to_dev(ts))
-        st["fsp"].copy_(e.fock_dev if fsp is None else ops.to_dev(fsp))
+            st = self._blocks = ArgBlocks(e.device, ts=(o, v), fsp=(n, n), vm=(n, n), F=(n, n), W=(v, o, o, v),
+                                          X=(o, v), e=(1,))
+        st.put(ts=ops.to_dev(ts), fsp=e.fock_dev if fsp is None else ops.to_dev(fsp))
         if vm is not None:
-            st["vm"].copy_(ops.to_dev(vm))
+            st.put(vm=ops.to_dev(vm))
         p = lambda k: st[k].data_ptr()                                                           # noqa: E731
         if func == "t1":
             e.execute("ccs_t1inter", 0, lambda: lib.ecw_ccs_t1inter(e._h, p("ts"), p("fsp"), p("F"), e.stream()),
@@ -124,7 +121,7 @@ class Gccs(object):
         ops = self.ops
         o = self.nocc
         d_ts = ops.to_dev(ts)
-        foo, fov, fvo, fvv = self._f(fsp)
+        foo, fov, fvo, fvv = self.eris.fock_blocks(fsp)
         e = ops.dot(fov, d_ts) + 0.5 * ops.dot(d_ts, self._G(d_ts))
         if rsn is not None:
             for rs, v, r0 in zip(rsn, vn, r0n):
@@ -171,12 +168,8 @@ class Gccs(object):
         o, v = self.nocc, self.nvir
         Fab_h, Fji_h, Fai_h = T1inter
         d_ts = ops.to_dev(ts)
-        Fab, Fji, Fai = ops.to_dev(Fab_h), ops.to_dev(Fji_h), ops.to_dev(Fai_h)
-        ops.diag_shift(Fab, -1.0, o)                       # in place, CCS.py:307-308 (Q6)
-        ops.diag_shift(Fji, -1.0, 0)
-        Fab_h[...] = ops.to_host(Fab)
-        Fji_h[...] = ops.to_host(Fji)
-        new = self._t1(d_ts, Fab, Fji, Fai)
+        Fab, Fji = self._q6(Fab_h, Fji_h)                  # CCS.py:307-308
+        new = self._t1(d_ts, Fab, Fji, ops.to_dev(Fai_h))
         if rsn is not None:                                # ES coupling, CCS.py:316-347
             if r0n is None:
                 raise ValueError('if Vexp are to be calculated, list of r0 amp must be given')
@@ -240,13 +233,9 @@ class Gccs(object):
         o, v = self.nocc, self.nvir
         Fia_h, Fba_h, Fij_h, W_h, E = L1inter
         d_ts, d_ls = ops.to_dev(ts), ops.to_dev(ls)
-        Fia, Fba, Fij = ops.to_dev(Fia_h), ops.to_dev(Fba_h), ops.to_dev(Fij_h)
         W = self._w_dev(L1inter, 3, (v, o, o, v))
-        ops.diag_shift(Fba, -1.0, o)                       # in place, CCS.py:529-530 (Q6)
-        ops.diag_shift(Fij, -1.0, 0)
-        Fba_h[...] = ops.to_host(Fba)
-        Fij_h[...] = ops.to_host(Fij)
-        new = self._l1(d_ls, Fia, Fba, Fij, W, _scalar(E))
+        Fba, Fij = self._q6(Fba_h, Fij_h)                  # CCS.py:529-530
+        new = self._l1(d_ls, ops.to_dev(Fia_h), Fba, Fij, W, _scalar(E))
         if rsn is not None:                                # CCS.py:539-579
             if len(lsn) != len(rsn) or len(vn) != len(rsn):
                 raise ValueError('v0n, l and r list must be of same length')
@@ -297,16 +286,18 @@ class Gccs(object):
         ops.contract('akic,kc->ia', W, d_rs, out=R, beta=1.0)
         return R
 
-    def _r1full(self, rs, r0, Rinter):
+    def _es1full(self, core, amp, amp0, inter, shifted=None):
+        """core(amp, Fv, Fo, W) + amp F + amp0 Zia + P for an excited-state intermediate tuple (Fv, Fo, W, F, Zia, P:
+        R1inter / es_L1inter); shifted: the device Fv, Fo of an update (_q6).  Returns it and the device amp."""
         ops = self.ops
         o, v = self.nocc, self.nvir
-        Fab, Fji, W_h, F, Zia, Pia = Rinter
-        d_rs = ops.to_dev(rs)
-        R = self._r1core(d_rs, ops.to_dev(Fab), ops.to_dev(Fji), self._w_dev(Rinter, 2, (v, o, o, v)))
-        ops.scale_add(R, d_rs, _scalar(F))
-        ops.scale_add(R, ops.to_dev(Zia), _scalar(r0))
-        ops.scale_add(R, ops.to_dev(Pia), 1.0)
-        return R, d_rs
+        d = ops.to_dev(amp)
+        Fv, Fo = shifted or (ops.to_dev(inter[0]), ops.to_dev(inter[1]))
+        R = core(d, Fv, Fo, self._w_dev(inter, 2, (v, o, o, v)))
+        ops.scale_add(R, d, _scalar(inter[3]))
+        ops.scale_add(R, ops.to_dev(inter[4]), _scalar(amp0))
+        ops.scale_add(R, ops.to_dev(inter[5]), 1.0)
+        return R, d
 
     def Extract_Em_r(self, rs, r0, Rinter, ov=None):       # CCS.py:874-906
         ops = self.ops
@@ -315,24 +306,13 @@ class Gccs(object):
             o, v = np.unravel_index(np.argmax(abs(rs), axis=None), rs.shape)
         else:
             o, v = ov
-        R, d_rs = self._r1full(rs, r0, Rinter)
+        R, _ = self._es1full(self._r1core, rs, r0, Rinter)
         q = ops.to_host(R)
         return _like_amp0(q[o, v] / rs[o, v], r0), o, v
 
     def rsupdate(self, rs, r0, Rinter, Em, force_alpha=True):   # CCS.py:908-943
         ops = self.ops
-        o, v = self.nocc, self.nvir
-        Fab_h, Fji_h, W_h, F, Zia, Pia = Rinter
-        d_rs = ops.to_dev(rs)
-        Fab, Fji = ops.to_dev(Fab_h), ops.to_dev(Fji_h)
-        ops.diag_shift(Fab, -1.0, o)                       # CCS.py:927-928 (Q6)
-        ops.diag_shift(Fji, -1.0, 0)
-        Fab_h[...] = ops.to_host(Fab)
-        Fji_h[...] = ops.to_host(Fji)
-        R = self._r1core(d_rs, Fab, Fji, self._w_dev(Rinter, 2, (v, o, o, v)))
-        ops.scale_add(R, d_rs, _scalar(F))
-        ops.scale_add(R, ops.to_dev(Zia), _scalar(r0))
-        ops.scale_add(R, ops.to_dev(Pia), 1.0)
+        R, d_rs = self._es1full(self._r1core, rs, r0, Rinter, self._q6(Rinter[0], Rinter[1]))   # CCS.py:927-928
         new = ops.denom(R, d_rs, shift=float(np.asarray(Em).reshape(-1)[0]))
         if force_alpha:
             ops.fill(new[0::2, :], 0.0)                    # force alpha transition (Q9)
@@ -350,16 +330,16 @@ class Gccs(object):
         return rov / ls[o, v]
 
     def R1eq(self, rs, r0, Rinter):                        # CCS.py:965-985
-        R, _ = self._r1full(rs, r0, Rinter)
+        R, _ = self._es1full(self._r1core, rs, r0, Rinter)
         return self.ops.to_host(R)
 
     def R0inter(self, ts, fsp, vm):                        # CCS.py:987-1034
         ops = self.ops
         o = self.nocc
         d_ts = ops.to_dev(ts)
-        foo, fov, fvo, fvv = self._f(self.fock if fsp is None else fsp)
+        foo, fov, fvo, fvv = self.eris.fock_blocks(self.fock if fsp is None else fsp)
         Fjb = ops.copy(fov)
-        ops.contract('kc,kjcb->jb', d_ts, self._oovv, out=Fjb, beta=1.0)
+        ops.contract('kc,kjcb->jb', d_ts, self.eris.block("oovv"), out=Fjb, beta=1.0)
         E = ops.dot(d_ts, fov) + 0.5 * ops.dot(d_ts, self._G(d_ts))
         d_v = ops.to_dev(vm)
         P = ops.trace(d_v[:o, :o]) + ops.dot(d_ts, d_v[:o, o:])
@@ -373,7 +353,7 @@ class Gccs(object):
         f = self.fock if fsp is None else fsp
         Rinter = self.R1inter(ts, f, vm)
         Fjb, Z, P = self.R0inter(ts, f, vm)
-        R, d_rs = self._r1full(r1, 0.0, Rinter)            # Fab.r1 - Fji.r1 + W.r1 + r1 F + Pia  (r0 = 0: no Zia term)
+        R, d_rs = self._es1full(self._r1core, r1, 0.0, Rinter)  # Fab.r1 - Fji.r1 + W.r1 + r1 F + Pia (r0 = 0: no Zia term)
         R1 = self.ops.to_host(R)
         Zia = np.asarray(Rinter[4])
         c = -self.ops.dot(d_rs, self.ops.to_dev(Fjb)) - P
@@ -404,7 +384,7 @@ class Gccs(object):
         ops = self.ops
         o = self.nocc
         d_t, d_r = ops.to_dev(t1), ops.to_dev(r1)
-        foo, fov, fvo, fvv = self._f(self.fock if fsp is None else fsp)
+        foo, fov, fvo, fvv = self.eris.fock_blocks(self.fock if fsp is None else fsp)
         G = self._G(d_t)
         d = En - ops.dot(d_t, fov) - 0.5 * ops.dot(d_t, G)
         r0 = ops.dot(d_r, fov) + ops.dot(d_r, G)           # 'kc,jb,jkbc' = r1 . G (oovv[jkbc] = oovv[kjcb])
@@ -423,20 +403,20 @@ class Gccs(object):
         return self._pack(host, W, 2)
 
     def L0inter(self, ts, fsp, vm):                        # CCS.py:1236-1286
-        ops = self.ops
+        ops, B = self.ops, self.eris.block
         o = self.nocc
         d_ts = ops.to_dev(ts)
-        foo, fov, fvo, fvv = self._f(self.fock if fsp is None else fsp)
+        foo, fov, fvo, fvv = self.eris.fock_blocks(self.fock if fsp is None else fsp)
         Fbj = ops.copy(fvo)
         ops.contract('kb,kj->bj', d_ts, foo, alpha=-1.0, out=Fbj, beta=1.0)
         ops.contract('ja,ba->bj', d_ts, fvv, out=Fbj, beta=1.0)
         q = ops.contract('kb,kc->bc', d_ts, fov)                                             # 'jc,kb,kc->bj'
         ops.contract('jc,bc->bj', d_ts, q, alpha=-1.0, out=Fbj, beta=1.0)
-        x = ops.copy(self._ovov_ph, 'jbkc->kbcj', alpha=-1.0)                                 # ovvo[kbcj] = -ovov[kbjc]
-        a = ops.contract('lb,lkcd->bkcd', d_ts, self._oovv)                                  # 'lb,jd,lkcd->kbcj'
+        x = ops.copy(B("ovov_ph"), 'jbkc->kbcj', alpha=-1.0)                                  # ovvo[kbcj] = -ovov[kbjc]
+        a = ops.contract('lb,lkcd->bkcd', d_ts, B("oovv"))                                   # 'lb,jd,lkcd->kbcj'
         ops.contract('jd,bkcd->kbcj', d_ts, a, out=x, beta=1.0)
-        ops.contract('lb,kljc->kbcj', d_ts, self._ooov, out=x, beta=1.0)                     # -(oovo[klcj] = -ooov[kljc])
-        ops.contract('jd,kbcd->kbcj', d_ts, self._ovvv, out=x, beta=1.0)
+        ops.contract('lb,kljc->kbcj', d_ts, B("ooov"), out=x, beta=1.0)                      # -(oovo[klcj] = -ooov[kljc])
+        ops.contract('jd,kbcd->kbcj', d_ts, B("ovvv"), out=x, beta=1.0)
         Wjb = ops.contract('kc,kbcj->jb', d_ts, x)
         Z = ops.dot(d_ts, fov) + 0.5 * ops.dot(d_ts, self._G(d_ts))
         d_v = ops.to_dev(vm)
@@ -450,24 +430,13 @@ class Gccs(object):
         ops.contract('jb,bija->ia', d_ls, W, out=L, beta=1.0)
         return L
 
-    def _esl1full(self, ls, l0, inter):
-        ops = self.ops
-        o, v = self.nocc, self.nvir
-        Fba, Fij, W_h, F, Zia, P = inter
-        d_ls = ops.to_dev(ls)
-        L = self._l1core(d_ls, ops.to_dev(Fba), ops.to_dev(Fij), self._w_dev(inter, 2, (v, o, o, v)))
-        ops.scale_add(L, d_ls, _scalar(F))
-        ops.scale_add(L, ops.to_dev(Zia), _scalar(l0))
-        ops.scale_add(L, ops.to_dev(P), 1.0)
-        return L
-
     def Extract_Em_l(self, ls, l0, L1inter, ov=None):      # CCS.py:1288-1319
         ls = np.asarray(ls)
         if ov is None:
             o, v = np.unravel_index(np.argmax(abs(ls), axis=None), ls.shape)
         else:
             o, v = ov
-        L = self.ops.to_host(self._esl1full(ls, l0, L1inter))
+        L = self.ops.to_host(self._es1full(self._l1core, ls, l0, L1inter)[0])
         return _like_amp0(L[o, v] / ls[o, v], l0), o, v
 
     def Extract_l0(self, l1, ts, fsp, vm):
@@ -476,25 +445,14 @@ class Gccs(object):
 
     def es_lsupdate(self, ls, l0, Em, L1inter, force_alpha=True):   # CCS.py:1366-1399
         ops = self.ops
-        o, v = self.nocc, self.nvir
-        Fba_h, Fij_h, W_h, F, Zia, P = L1inter
-        d_ls = ops.to_dev(ls)
-        Fba, Fij = ops.to_dev(Fba_h), ops.to_dev(Fij_h)
-        ops.diag_shift(Fba, -1.0, o)                       # CCS.py:1384-1385 (Q6)
-        ops.diag_shift(Fij, -1.0, 0)
-        Fba_h[...] = ops.to_host(Fba)
-        Fij_h[...] = ops.to_host(Fij)
-        L = self._l1core(d_ls, Fba, Fij, self._w_dev(L1inter, 2, (v, o, o, v)))
-        ops.scale_add(L, d_ls, _scalar(F))
-        ops.scale_add(L, ops.to_dev(Zia), _scalar(l0))
-        ops.scale_add(L, ops.to_dev(P), 1.0)
+        L, d_ls = self._es1full(self._l1core, ls, l0, L1inter, self._q6(L1inter[0], L1inter[1]))   # CCS.py:1384-1385
         new = ops.denom(L, d_ls, shift=float(np.asarray(Em).reshape(-1)[0]))
         if force_alpha:
             ops.fill(new[0::2, :], 0.0)
         return ops.to_host(new)
 
     def es_L1eq(self, ls, l0, es_L1inter):                 # CCS.py:1401-1421
-        return self.ops.to_host(self._esl1full(ls, l0, es_L1inter))
+        return self.ops.to_host(self._es1full(self._l1core, ls, l0, es_L1inter)[0])
 
     def l0update(self, ls, l0, Em, L0inter):               # CCS.py:1423-1439
         ops = self.ops
@@ -511,10 +469,10 @@ class Gccs(object):
         return ops.dot(d_ls, ops.to_dev(Fbj).t()) + ops.dot(d_ls, ops.to_dev(Wjb)) + l0 * El + P
 
     def l0_fromE(self, En, t1, l1, v0m, fsp=None):         # CCS.py:1459-1518
-        ops = self.ops
+        ops, B = self.ops, self.eris.block
         o = self.nocc
         d_t, d_l = ops.to_dev(t1), ops.to_dev(l1)
-        foo, fov, fvo, fvv = self._f(self.fock if fsp is None else fsp)
+        foo, fov, fvo, fvv = self.eris.fock_blocks(self.fock if fsp is None else fsp)
         G = self._G(d_t)
         shift = 0.5 * ops.dot(d_t, G)
         if isinstance(En, np.ndarray):                     # Q12: `d = En; d -= ...` (CCS.py:1488-1490) changes the
@@ -527,15 +485,15 @@ class Gccs(object):
         l0 -= ops.dot(ops.contract('jb,kb->kj', d_l, d_t), foo)                              # 'jb,kb,kj'
         q = ops.contract('kb,kc->bc', d_t, fov)                                              # 'jc,kb,kc,jb'
         l0 -= ops.dot(ops.contract('jc,bc->jb', d_t, q), d_l)
-        w = ops.contract('kc,jbkc->jb', d_t, self._ovov_ph, alpha=-1.0)                      # ovvo[kbcj] = -ovov_ph[jbkc]
+        w = ops.contract('kc,jbkc->jb', d_t, B("ovov_ph"), alpha=-1.0)                       # ovvo[kbcj] = -ovov_ph[jbkc]
         l0 += ops.dot(d_l, w)
         x = ops.contract('jb,jd->bd', d_l, d_t)
-        y = ops.contract('lc,klcd->kd', d_t, self._oovv)                                     # 'bd,kb,lc,klcd'
+        y = ops.contract('lc,klcd->kd', d_t, B("oovv"))                                      # 'bd,kb,lc,klcd'
         l0 += ops.dot(ops.contract('kb,kd->bd', d_t, y), x)
         m = ops.contract('jb,lb->jl', d_l, d_t)
-        n2 = ops.contract('kc,kljc->jl', d_t, self._ooov)                                    # -'jl,kc,klcj' oovo = +ooov
+        n2 = ops.contract('kc,kljc->jl', d_t, B("ooov"))                                     # -'jl,kc,klcj' oovo = +ooov
         l0 += ops.dot(m, n2)
-        l0 += ops.dot(ops.contract('kc,kbcd->bd', d_t, self._ovvv), x)                       # 'bd,kc,kbcd'
+        l0 += ops.dot(ops.contract('kc,kbcd->bd', d_t, B("ovvv")), x)                        # 'bd,kc,kbcd'
         if v0m is not None:
             d_v = ops.to_dev(v0m)
             l0 += ops.dot(d_t, d_v[:o, o:]) + ops.trace(d_v[:o, :o])

@@ -9,6 +9,7 @@ CUDA tensors out (device-resident mode used by bench.py's `value` leg).
 import numpy as np
 
 from ._lib import lib, EcwError, ECW_HAS_ALPHA, ECW_EQUATION, ECW_ANTISYM
+from .devops import ArgBlocks
 from .eris import DeviceEris
 
 
@@ -26,7 +27,6 @@ def _flags(alpha, equation, antisym=False):
 
 class GCC(object):
     TRACK_MIN_BYTES = 1 << 20   # smaller outputs are not worth a device copy kept alive
-    POOL_DEPTH = 4              # pinned result blocks kept per shape
     # Shapes with o^2 v^2 up to this many elements (every molecular configuration of BASELINE.json) are bound by the
     # launch rate of the several hundred kernels of an evaluation, not by their run time.  Their calls go through
     # persistent argument blocks owned by this object — inputs copied in, results copied out (device to device,
@@ -47,13 +47,17 @@ class GCC(object):
             eris = DeviceEris.from_geris(eris, device=device, rank=rank, world=world, group=group, gemm=gemm,
                                          int8_digits=int8_digits)
         self.eris = eris
+        self.ops = eris.ops
         self.nocc = eris.nocc
         if fock is None:                       # CCSD.py:196-198
             self.fock = eris.fock
         self.nvir = self.fock.shape[0] - self.nocc
+        o, v, n = self.nocc, self.nvir, self.fock.shape[0]
+        self._shapes = dict(t1=(o, v), t2=(o, o, v, v), l1=(o, v), l2=(o, o, v, v), fsp=(n, n), o1=(o, v),
+                            o2=(o, o, v, v), rdm1=(n, n), e=(1,))    # arguments and results of the four entry points
         self._pin = {}
         self._tracked = {}      # id(host array this object returned) -> (weakref, its device copy)
-        self._pool = {}         # (shape, dtype) -> pinned blocks of returned arrays the caller has dropped
+        self._blocks = None     # ArgBlocks of the small-shape route (_stage)
         self.track_outputs = bool(track_outputs)
         self.h2d_bytes = 0      # bytes staged host->device / device->host by this object
         self.d2h_bytes = 0
@@ -98,18 +102,18 @@ class GCC(object):
         return pin.to(self.eris.device, non_blocking=True), False
 
     def _to_host(self, *ts):
-        """device -> fresh numpy arrays backed by pinned memory (torch's caching host allocator).  With
-        `track_outputs` (default) the arrays are READ-ONLY and the object remembers their device copies for as long
-        as the caller keeps the arrays (weak references): passing one back costs no transfer.  (The reference
-        returns writable arrays; its solvers never write into them — `GCC(..., track_outputs=False)` restores that.)"""
+        """device -> fresh numpy arrays in pinned blocks of the context's download pool (devops.PinnedPool).  With
+        `track_outputs` (default) the arrays of TRACK_MIN_BYTES or more are READ-ONLY and the object remembers their
+        device copies for as long as the caller keeps the arrays (weak references): passing one back costs no transfer.
+        (The reference returns writable arrays; its solvers never write into them — `GCC(..., track_outputs=False)`
+        restores that.)"""
         import weakref
-        torch = self._torch()
         import time
-        outs = []
+        torch = self._torch()
+        pool = self.ops.pinned
         torch.cuda.current_stream(self.eris.device).synchronize()          # the results are complete
         t0 = time.perf_counter()
-        for t in ts:
-            outs.append(self._pinned(t.shape, t.dtype))
+        outs = [pool.take(t.shape, t.dtype) for t in ts]
         t1 = time.perf_counter()
         for h, t in zip(outs, ts):
             h.copy_(t, non_blocking=True)
@@ -117,27 +121,13 @@ class GCC(object):
         torch.cuda.current_stream(self.eris.device).synchronize()
         self.host_seconds["to_host_alloc"] += t1 - t0
         self.host_seconds["to_host_copy"] += time.perf_counter() - t1
-        arrs = [h.numpy() for h in outs]
-        for a, h, t in zip(arrs, outs, ts):
-            if a.nbytes >= self.TRACK_MIN_BYTES:
-                # the pinned block goes back to this object's pool when the caller drops the array
-                weakref.finalize(a, self._pool.setdefault((tuple(h.shape), h.dtype), []).append, h)
-                if self.track_outputs:
-                    a.setflags(write=False)
-                    key = id(a)
-                    self._tracked[key] = (weakref.ref(a, lambda _r, k=key, d=self._tracked: d.pop(k, None)), t)
+        arrs = [pool.hand_out(h) for h in outs]
+        for a, t in zip(arrs, ts):
+            if self.track_outputs and a.nbytes >= self.TRACK_MIN_BYTES:
+                a.setflags(write=False)
+                key = id(a)
+                self._tracked[key] = (weakref.ref(a, lambda _r, k=key, d=self._tracked: d.pop(k, None)), t)
         return arrs[0] if len(arrs) == 1 else tuple(arrs)
-
-    def _pinned(self, shape, dtype):
-        """A pinned host buffer for one result.  Page-locking gigabytes costs far more than the transfer itself
-        (cudaHostAlloc), so blocks of arrays the caller has dropped are reused (per shape, at most POOL_DEPTH kept)."""
-        torch = self._torch()
-        free = self._pool.get((tuple(shape), dtype))
-        if free:
-            h = free.pop()
-            del free[self.POOL_DEPTH:]
-            return h
-        return torch.empty(shape, dtype=dtype, pin_memory=True)
 
     def to_numpy(self, t):
         """Download a device tensor the way every method of this class returns its results (pinned, read-only,
@@ -150,24 +140,9 @@ class GCC(object):
         e = self.eris
         if o * o * v * v > self.STAGE_MAX_ELEMS or getattr(e, "world", 1) > 1:
             return None
-        st = getattr(self, "_stage_bufs", None)
-        if st is None:
-            torch = self._torch()
-            n = o + v
-            mk = lambda *shape: torch.empty(shape, dtype=torch.float64, device=e.device)      # noqa: E731
-            st = self._stage_bufs = dict(t1=mk(o, v), t2=mk(o, o, v, v), l1=mk(o, v), l2=mk(o, o, v, v), fsp=mk(n, n),
-                                         o1=mk(o, v), o2=mk(o, o, v, v), rdm1=mk(n, n), e=mk(1))
-        return st
-
-    @staticmethod
-    def _staged(st, **named):
-        """Copy the call's device arguments into the persistent blocks; returns the blocks in the same order."""
-        out = []
-        for k, t in named.items():
-            if t.data_ptr() != st[k].data_ptr():
-                st[k].copy_(t)
-            out.append(st[k])
-        return out
+        if self._blocks is None:
+            self._blocks = ArgBlocks(e.device, **self._shapes)
+        return self._blocks
 
     def antisym_stats(self, d_x):
         """(max |x[ijab]+x[jiab]|, |x[ijab]+x[ijba]|, max |x|) of a device doubles amplitude."""
@@ -198,41 +173,44 @@ class GCC(object):
             return self.eris.fock_dev, True
         return self._to_dev("fsp", fsp, (n, n))
 
-    # -- rdm1 (CCSD.py:204-208 -> :136-182) -------------------------------------
-    def gamma(self, t1, t2, l1, l2):
+    def _call(self, func, launch, inputs, outputs, antisym=(), alpha=None, equation=False):
+        """The sequence of the four entry points: upload `inputs` (name -> array; the first one decides between device
+        and host results; "fsp" may be None = the Fock matrix), measure the antisymmetry of the doubles named in
+        `antisym`, stage everything into the persistent blocks when the shape allows, allocate the `outputs`, and run
+        launch(flags, pointers by name) through the guarded executor.  Returns (device results?, [outputs])."""
         torch = self._torch()
-        o, v = self.nocc, self.nvir
         e = self.eris
-        d_t1, dev = self._to_dev("t1", t1, (o, v))
-        d_t2, _ = self._to_dev("t2", t2, (o, o, v, v))
-        d_l1, _ = self._to_dev("l1", l1, (o, v))
-        d_l2, _ = self._to_dev("l2", l2, (o, o, v, v))
+        shapes = self._shapes
+        args, dev = {}, None
+        for k, x in inputs.items():
+            args[k], d = self._fsp(x) if k == "fsp" else self._to_dev(k, x, shapes[k])
+            dev = d if dev is None else dev
+        fl = _flags(alpha, equation, bool(antisym) and self._is_antisym(*(args[k] for k in antisym)))
         st = self._stage()
         if st is not None:
-            d_t1, d_t2, d_l1, d_l2 = self._staged(st, t1=d_t1, t2=d_t2, l1=d_l1, l2=d_l2)
-        out = st["rdm1"] if st is not None else torch.empty((o + v, o + v), dtype=torch.float64, device=e.device)
-        e.execute("gamma", 0, lambda: lib.ecw_ccsd_gamma(e._h, d_t1.data_ptr(), d_t2.data_ptr(), d_l1.data_ptr(),
-                                                         d_l2.data_ptr(), out.data_ptr(), e.stream()), "ecw_ccsd_gamma")
+            args = dict(zip(args, st.put(**args)))
+            outs = [st[k] for k in outputs]
+        else:
+            outs = [torch.empty(shapes[k], dtype=torch.float64, device=e.device) for k in outputs]
+        p = {k: t.data_ptr() for k, t in list(args.items()) + list(zip(outputs, outs))}
+        e.execute(func, fl, lambda: launch(fl, p), "ecw_ccsd_" + func)
         if st is not None:
-            out = out.clone()
-        return out if dev else self._to_host(out)
+            outs = [t.clone() for t in outs]
+        return dev, outs
+
+    # -- rdm1 (CCSD.py:204-208 -> :136-182) -------------------------------------
+    def gamma(self, t1, t2, l1, l2):
+        e = self.eris
+        dev, outs = self._call("gamma", lambda fl, p: lib.ecw_ccsd_gamma(
+            e._h, p["t1"], p["t2"], p["l1"], p["l2"], p["rdm1"], e.stream()),
+            dict(t1=t1, t2=t2, l1=l1, l2=l2), ("rdm1",))
+        return outs[0] if dev else self._to_host(*outs)
 
     # -- energy (CCSD.py:224-242) -------------------------------------------------
     def energy(self, t1, t2, fsp):
-        torch = self._torch()
-        o, v = self.nocc, self.nvir
         e = self.eris
-        d_t1, dev = self._to_dev("t1", t1, (o, v))
-        d_t2, _ = self._to_dev("t2", t2, (o, o, v, v))
-        d_f, _ = self._fsp(fsp)
-        st = self._stage()
-        if st is not None:
-            d_t1, d_t2, d_f = self._staged(st, t1=d_t1, t2=d_t2, fsp=d_f)
-        out = st["e"] if st is not None else torch.empty(1, dtype=torch.float64, device=e.device)
-        e.execute("energy", 0, lambda: lib.ecw_ccsd_energy(e._h, d_t1.data_ptr(), d_t2.data_ptr(), d_f.data_ptr(),
-                                                           out.data_ptr(), e.stream()), "ecw_ccsd_energy")
-        if st is not None:
-            out = out.clone()
+        dev, (out,) = self._call("energy", lambda fl, p: lib.ecw_ccsd_energy(
+            e._h, p["t1"], p["t2"], p["fsp"], p["e"], e.stream()), dict(t1=t1, t2=t2, fsp=fsp), ("e",))
         if dev:
             return out[0]
         self.d2h_bytes += 8
@@ -240,82 +218,27 @@ class GCC(object):
 
     # -- T1/T2 (CCSD.py:248-338) ---------------------------------------------------
     def tupdate(self, t1, t2, fsp=None, alpha=None, equation=False):
-        torch = self._torch()
-        o, v = self.nocc, self.nvir
         e = self.eris
-        d_t1, dev = self._to_dev("t1", t1, (o, v))
-        d_t2, _ = self._to_dev("t2", t2, (o, o, v, v))
-        d_f, _ = self._fsp(fsp)
-        st = self._stage()
-        if st is not None:
-            d_t1, d_t2, d_f = self._staged(st, t1=d_t1, t2=d_t2, fsp=d_f)
-            o1, o2 = st["o1"], st["o2"]
-        else:
-            o1 = torch.empty((o, v), dtype=torch.float64, device=e.device)
-            o2 = torch.empty((o, o, v, v), dtype=torch.float64, device=e.device)
-        fl = _flags(alpha, equation, self._is_antisym(d_t2))
-        e.execute("tupdate", fl, lambda: lib.ecw_ccsd_tupdate(
-            e._h, d_t1.data_ptr(), d_t2.data_ptr(), d_f.data_ptr(), e.fock_dev.data_ptr(), fl, float(alpha or 0.0),
-            o1.data_ptr(), o2.data_ptr(), e.stream()), "ecw_ccsd_tupdate")
-        if st is not None:
-            o1, o2 = o1.clone(), o2.clone()
-        if dev:
-            return o1, o2
-        return self._to_host(o1, o2)
+        dev, outs = self._call("tupdate", lambda fl, p: lib.ecw_ccsd_tupdate(
+            e._h, p["t1"], p["t2"], p["fsp"], e.fock_dev.data_ptr(), fl, float(alpha or 0.0), p["o1"], p["o2"],
+            e.stream()), dict(t1=t1, t2=t2, fsp=fsp), ("o1", "o2"), ("t2",), alpha, equation)
+        return tuple(outs) if dev else self._to_host(*outs)
 
     # -- L1/L2 (CCSD.py:419-535, Linter :543-623) --------------------------------------
     def lupdate(self, t1, t2, l1, l2, fsp=None, alpha=None, equation=False):
-        torch = self._torch()
-        o, v = self.nocc, self.nvir
         e = self.eris
-        d_t1, dev = self._to_dev("t1", t1, (o, v))
-        d_t2, _ = self._to_dev("t2", t2, (o, o, v, v))
-        d_l1, _ = self._to_dev("l1", l1, (o, v))
-        d_l2, _ = self._to_dev("l2", l2, (o, o, v, v))
-        d_f, _ = self._fsp(fsp)
-        st = self._stage()
-        if st is not None:
-            d_t1, d_t2, d_l1, d_l2, d_f = self._staged(st, t1=d_t1, t2=d_t2, l1=d_l1, l2=d_l2, fsp=d_f)
-            o1, o2 = st["o1"], st["o2"]
-        else:
-            o1 = torch.empty((o, v), dtype=torch.float64, device=e.device)
-            o2 = torch.empty((o, o, v, v), dtype=torch.float64, device=e.device)
-        fl = _flags(alpha, equation, self._is_antisym(d_t2, d_l2))
-        e.execute("lupdate", fl, lambda: lib.ecw_ccsd_lupdate(
-            e._h, d_t1.data_ptr(), d_t2.data_ptr(), d_l1.data_ptr(), d_l2.data_ptr(), d_f.data_ptr(),
-            e.fock_dev.data_ptr(), fl, float(alpha or 0.0), o1.data_ptr(), o2.data_ptr(), e.stream()),
-            "ecw_ccsd_lupdate")
-        if st is not None:
-            o1, o2 = o1.clone(), o2.clone()
-        if dev:
-            return o1, o2
-        return self._to_host(o1, o2)
+        dev, outs = self._call("lupdate", lambda fl, p: lib.ecw_ccsd_lupdate(
+            e._h, p["t1"], p["t2"], p["l1"], p["l2"], p["fsp"], e.fock_dev.data_ptr(), fl, float(alpha or 0.0),
+            p["o1"], p["o2"], e.stream()), dict(t1=t1, t2=t2, l1=l1, l2=l2, fsp=fsp), ("o1", "o2"), ("t2", "l2"),
+            alpha, equation)
+        return tuple(outs) if dev else self._to_host(*outs)
 
     # -- intermediates of the reference API (CCSD.py:207-208, 346-413, 543-623) ------------------
     # Not used by the fused tupdate/lupdate plans (which never form Wvvvv / wvvvo); provided so
     # that every public GCC method exists.  numpy in -> numpy out, arithmetic on the device
     # through the primitive ops (same index strings as the reference, canonical integral blocks).
-    def _dev_ops(self):
-        if getattr(self, "_ops", None) is None:
-            from .devops import DevOps
-            o, v = self.nocc, self.nvir
-            b = self.eris.buf
-            self._ops = DevOps(self.eris)
-            self._oooo = b["oooo"][: o ** 4].view(o, o, o, o)
-            self._ooov = b["ooov"][: o * o * o * v].view(o, o, o, v)
-            self._oovv = b["oovv"][: o * o * v * v].view(o, o, v, v)
-            self._ovvv = b["ovvv"][: o * v ** 3].view(o, v, v, v)
-            self._ovov_ph = b["ovov_ph"][: o * v * o * v].view(o, v, o, v)
-        return self._ops
-
-    def _fblocks(self, fsp):
-        ops = self._dev_ops()
-        o = self.nocc
-        F = self.eris.fock_dev if fsp is None else ops.to_dev(fsp)
-        return F[:o, :o], F[:o, o:], F[o:, :o], F[o:, o:]
-
     def _tau_dev(self, t2, t1a, t1b, fac=1.):
-        ops = self._dev_ops()
+        ops = self.ops
         x = ops.contract('ia,jb->ijab', t1a, t1b, alpha=0.5 * fac)          # CCSD.py:348
         y = ops.copy(x)
         ops.axpby(-1.0, x, 'jiab', 1.0, y, 'ijab')                          # :349
@@ -325,11 +248,11 @@ class GCC(object):
         return tau
 
     def make_tau(self, t2, t1a, t1b, fac=1.):
-        ops = self._dev_ops()
+        ops = self.ops
         return ops.to_host(self._tau_dev(ops.to_dev(t2), ops.to_dev(t1a), ops.to_dev(t1b), fac))
 
     def gamma_inter(self, t1, t2, l1, l2):                                  # CCSD.py:165-182
-        ops = self._dev_ops()
+        ops = self.ops
         t1, t2, l1, l2 = (ops.to_dev(x) for x in (t1, t2, l1, l2))
         doo = ops.contract('ie,je->ij', l1, t1, alpha=-1.0)
         ops.contract('imef,jmef->ij', l2, t2, alpha=-0.5, out=doo, beta=1.0)
@@ -345,48 +268,48 @@ class GCC(object):
         return ops.to_host(doo), ops.to_host(l1), ops.to_host(dvo), ops.to_host(dvv)
 
     def cc_Fvv(self, t1, t2, fsp):                                          # CCSD.py:355-368
-        ops = self._dev_ops()
+        ops, B = self.ops, self.eris.block
         t1, t2 = ops.to_dev(t1), ops.to_dev(t2)
-        foo, fov, fvo, fvv = self._fblocks(fsp)
+        foo, fov, fvo, fvv = self.eris.fock_blocks(fsp)
         tt = self._tau_dev(t2, t1, t1, fac=0.5)
         Fae = ops.copy(fvv)
         ops.contract('me,ma->ae', fov, t1, alpha=-0.5, out=Fae, beta=1.0)
-        ops.contract('mf,maef->ae', t1, self._ovvv, alpha=-1.0, out=Fae, beta=1.0)     # vovv[amef] = -ovvv[maef]
-        ops.contract('mnaf,mnef->ae', tt, self._oovv, alpha=-0.5, out=Fae, beta=1.0)
+        ops.contract('mf,maef->ae', t1, B("ovvv"), alpha=-1.0, out=Fae, beta=1.0)      # vovv[amef] = -ovvv[maef]
+        ops.contract('mnaf,mnef->ae', tt, B("oovv"), alpha=-0.5, out=Fae, beta=1.0)
         return ops.to_host(Fae)
 
     def cc_Foo(self, t1, t2, fsp):                                          # CCSD.py:370-381
-        ops = self._dev_ops()
+        ops, B = self.ops, self.eris.block
         t1, t2 = ops.to_dev(t1), ops.to_dev(t2)
-        foo, fov, fvo, fvv = self._fblocks(fsp)
+        foo, fov, fvo, fvv = self.eris.fock_blocks(fsp)
         tt = self._tau_dev(t2, t1, t1, fac=0.5)
         Fmi = ops.copy(foo)
         ops.contract('me,ie->mi', fov, t1, alpha=0.5, out=Fmi, beta=1.0)
-        ops.contract('ne,mnie->mi', t1, self._ooov, out=Fmi, beta=1.0)
-        ops.contract('inef,mnef->mi', tt, self._oovv, alpha=0.5, out=Fmi, beta=1.0)
+        ops.contract('ne,mnie->mi', t1, B("ooov"), out=Fmi, beta=1.0)
+        ops.contract('inef,mnef->mi', tt, B("oovv"), alpha=0.5, out=Fmi, beta=1.0)
         return ops.to_host(Fmi)
 
     def cc_Fov(self, t1, t2, fsp):                                          # CCSD.py:383-387
-        ops = self._dev_ops()
+        ops, B = self.ops, self.eris.block
         t1 = ops.to_dev(t1)
-        foo, fov, fvo, fvv = self._fblocks(fsp)
+        foo, fov, fvo, fvv = self.eris.fock_blocks(fsp)
         Fme = ops.copy(fov)
-        ops.contract('nf,mnef->me', t1, self._oovv, out=Fme, beta=1.0)
+        ops.contract('nf,mnef->me', t1, B("oovv"), out=Fme, beta=1.0)
         return ops.to_host(Fme)
 
     def cc_Woooo(self, t1, t2):                                             # CCSD.py:389-394
-        ops = self._dev_ops()
+        ops, B = self.ops, self.eris.block
         t1, t2 = ops.to_dev(t1), ops.to_dev(t2)
         tau = self._tau_dev(t2, t1, t1)
-        tmp = ops.contract('je,mnie->mnij', t1, self._ooov)
-        W = ops.copy(self._oooo)
+        tmp = ops.contract('je,mnie->mnij', t1, B("ooov"))
+        W = ops.copy(B("oooo"))
         ops.add(W, tmp)
         ops.axpby(-1.0, tmp, 'mnji', 1.0, W, 'mnij')
-        ops.contract('ijef,mnef->mnij', tau, self._oovv, alpha=0.25, out=W, beta=1.0)
+        ops.contract('ijef,mnef->mnij', tau, B("oovv"), alpha=0.25, out=W, beta=1.0)
         return ops.to_host(W)
 
     def _vvvv_dense(self):
-        ops = self._dev_ops()
+        ops = self.ops
         v = self.nvir
         if self.eris.world != 1:
             raise EcwError("dense vvvv is not available on a sharded context")
@@ -397,77 +320,77 @@ class GCC(object):
         return ops.unpack(self.eris.buf["vvvv_p"][: pv * pv].view(pv, pv), 3, ops.empty(v, v, v, v))
 
     def cc_Wvvvv(self, t1, t2):                                             # CCSD.py:396-402 (small sizes only: v^4)
-        ops = self._dev_ops()
+        ops, B = self.ops, self.eris.block
         t1, t2 = ops.to_dev(t1), ops.to_dev(t2)
         tau = self._tau_dev(t2, t1, t1)
-        tmp = ops.contract('mb,mafe->bafe', t1, self._ovvv)
+        tmp = ops.contract('mb,mafe->bafe', t1, B("ovvv"))
         W = self._vvvv_dense()
         ops.add(W, tmp, -1.0)
         ops.axpby(1.0, tmp, 'bafe', 1.0, W, 'abfe')
-        ops.contract('mnab,mnef->abef', tau, self._oovv, alpha=0.25, out=W, beta=1.0)
+        ops.contract('mnab,mnef->abef', tau, B("oovv"), alpha=0.25, out=W, beta=1.0)
         return ops.to_host(W)
 
     def _wovvo_dev(self, t1, t2):
-        ops = self._dev_ops()
-        W = ops.contract('jf,mbef->mbej', t1, self._ovvv)                                   # CCSD.py:408
-        ops.contract('nb,mnje->mbej', t1, self._ooov, out=W, beta=1.0)                      # -(oovo = -ooov)
-        ops.contract('jnfb,mnef->mbej', t2, self._oovv, alpha=-0.5, out=W, beta=1.0)
-        x = ops.contract('jf,mnef->mnej', t1, self._oovv)
+        ops, B = self.ops, self.eris.block
+        W = ops.contract('jf,mbef->mbej', t1, B("ovvv"))                                    # CCSD.py:408
+        ops.contract('nb,mnje->mbej', t1, B("ooov"), out=W, beta=1.0)                       # -(oovo = -ooov)
+        ops.contract('jnfb,mnef->mbej', t2, B("oovv"), alpha=-0.5, out=W, beta=1.0)
+        x = ops.contract('jf,mnef->mnej', t1, B("oovv"))
         ops.contract('nb,mnej->mbej', t1, x, alpha=-1.0, out=W, beta=1.0)
-        ops.axpby(-1.0, self._ovov_ph, 'jbme', 1.0, W, 'mbej')                              # ovvo[mbej] = -ovov[mbje]
+        ops.axpby(-1.0, B("ovov_ph"), 'jbme', 1.0, W, 'mbej')                               # ovvo[mbej] = -ovov[mbje]
         return W
 
     def cc_Wovvo(self, t1, t2):                                             # CCSD.py:404-413
-        ops = self._dev_ops()
+        ops = self.ops
         return ops.to_host(self._wovvo_dev(ops.to_dev(t1), ops.to_dev(t2)))
 
     def Linter(self, t1, t2, fsp=None):                                     # CCSD.py:543-623
-        ops = self._dev_ops()
+        ops, B = self.ops, self.eris.block
         t1, t2 = ops.to_dev(t1), ops.to_dev(t2)
-        foo, fov, fvo, fvv = self._fblocks(fsp)
+        foo, fov, fvo, fvv = self.eris.fock_blocks(fsp)
         tau = ops.contract('ia,jb->ijab', t1, t1, alpha=2.0)
         ops.add(tau, t2)
         v1 = ops.copy(fvv)
         ops.contract('ja,jb->ba', fov, t1, alpha=-1.0, out=v1, beta=1.0)
-        ops.contract('jbac,jc->ba', self._ovvv, t1, alpha=-1.0, out=v1, beta=1.0)
-        ops.contract('jkca,jkbc->ba', self._oovv, tau, alpha=0.5, out=v1, beta=1.0)
+        ops.contract('jbac,jc->ba', B("ovvv"), t1, alpha=-1.0, out=v1, beta=1.0)
+        ops.contract('jkca,jkbc->ba', B("oovv"), tau, alpha=0.5, out=v1, beta=1.0)
         v2 = ops.copy(foo)
         ops.contract('ib,jb->ij', fov, t1, out=v2, beta=1.0)
-        ops.contract('kijb,kb->ij', self._ooov, t1, alpha=-1.0, out=v2, beta=1.0)
-        ops.contract('ikbc,jkbc->ij', self._oovv, tau, alpha=0.5, out=v2, beta=1.0)
-        v3 = ops.contract('ijcd,klcd->ijkl', self._oovv, tau)
-        v4 = ops.contract('ljdb,klcd->jcbk', self._oovv, t2)
-        ops.axpby(-1.0, self._ovov_ph, 'kcjb', 1.0, v4, 'jcbk')                             # ovvo[jcbk] = -ovov[jckb]
+        ops.contract('kijb,kb->ij', B("ooov"), t1, alpha=-1.0, out=v2, beta=1.0)
+        ops.contract('ikbc,jkbc->ij', B("oovv"), tau, alpha=0.5, out=v2, beta=1.0)
+        v3 = ops.contract('ijcd,klcd->ijkl', B("oovv"), tau)
+        v4 = ops.contract('ljdb,klcd->jcbk', B("oovv"), t2)
+        ops.axpby(-1.0, B("ovov_ph"), 'kcjb', 1.0, v4, 'jcbk')                              # ovvo[jcbk] = -ovov[jckb]
         v5 = ops.copy(fvo)
         ops.contract('kc,jkbc->bj', fov, t2, out=v5, beta=1.0)
         tmp = ops.copy(fov)
-        ops.contract('kldc,ld->kc', self._oovv, t1, alpha=-1.0, out=tmp, beta=1.0)
+        ops.contract('kldc,ld->kc', B("oovv"), t1, alpha=-1.0, out=tmp, beta=1.0)
         q = ops.contract('kc,jc->kj', tmp, t1)                                              # 'kc,kb,jc->bj'
         ops.contract('kb,kj->bj', t1, q, out=v5, beta=1.0)
-        ops.contract('kljc,klbc->bj', self._ooov, t2, alpha=-0.5, out=v5, beta=1.0)
-        ops.contract('kbdc,jkcd->bj', self._ovvv, t2, alpha=0.5, out=v5, beta=1.0)
+        ops.contract('kljc,klbc->bj', B("ooov"), t2, alpha=-0.5, out=v5, beta=1.0)
+        ops.contract('kbdc,jkcd->bj', B("ovvv"), t2, alpha=0.5, out=v5, beta=1.0)
         w3 = ops.copy(v5)
         ops.contract('jcbk,jb->ck', v4, t1, out=w3, beta=1.0)
         ops.contract('cb,jb->cj', v1, t1, out=w3, beta=1.0)
         ops.contract('jk,jb->bk', v2, t1, alpha=-1.0, out=w3, beta=1.0)
-        woooo = ops.copy(self._oooo, alpha=0.5)
+        woooo = ops.copy(B("oooo"), alpha=0.5)
         ops.add(woooo, v3, 0.25)
-        ops.contract('jilc,kc->jilk', self._ooov, t1, out=woooo, beta=1.0)
+        ops.contract('jilc,kc->jilk', B("ooov"), t1, out=woooo, beta=1.0)
         wovvo = ops.copy(v4)
-        s1 = ops.contract('ljdb,kd->ljbk', self._oovv, t1)                                  # 'ljdb,lc,kd->jcbk'
+        s1 = ops.contract('ljdb,kd->ljbk', B("oovv"), t1)                                   # 'ljdb,lc,kd->jcbk'
         ops.contract('ljbk,lc->jcbk', s1, t1, alpha=-1.0, out=wovvo, beta=1.0)
-        ops.contract('ljkb,lc->jcbk', self._ooov, t1, alpha=-1.0, out=wovvo, beta=1.0)
-        ops.contract('jcbd,kd->jcbk', self._ovvv, t1, out=wovvo, beta=1.0)
-        wovoo = ops.contract('icdb,jkdb->icjk', self._ovvv, tau, alpha=0.25)
-        ops.axpby(0.5, self._ooov, 'jkic', 1.0, wovoo, 'icjk')
+        ops.contract('ljkb,lc->jcbk', B("ooov"), t1, alpha=-1.0, out=wovvo, beta=1.0)
+        ops.contract('jcbd,kd->jcbk', B("ovvv"), t1, out=wovvo, beta=1.0)
+        wovoo = ops.contract('icdb,jkdb->icjk', B("ovvv"), tau, alpha=0.25)
+        ops.axpby(0.5, B("ooov"), 'jkic', 1.0, wovoo, 'icjk')
         ops.contract('icbk,jb->icjk', v4, t1, out=wovoo, beta=1.0)
-        ops.contract('lijb,klcb->icjk', self._ooov, t2, alpha=-1.0, out=wovoo, beta=1.0)
+        ops.contract('lijb,klcb->icjk', B("ooov"), t2, alpha=-1.0, out=wovoo, beta=1.0)
         wvvvo = ops.contract('jcak,jb->bcak', v4, t1)
-        ops.contract('jlka,jlbc->bcak', self._ooov, tau, alpha=0.25, out=wvvvo, beta=1.0)
-        ops.axpby(-0.5, self._ovvv, 'jacb', 1.0, wvvvo, 'bcaj')
-        ops.contract('kbad,jkcd->bcaj', self._ovvv, t2, out=wvvvo, beta=1.0)
-        G = ops.contract('menf,nf->me', self.eris.buf["oovv_ph"][: t1.numel() ** 2].view(*t1.shape, *t1.shape), t1)
-        E = ops.dot(fov, t1) + 0.25 * ops.dot(t2, self._oovv) + 0.5 * ops.dot(t1, G)
+        ops.contract('jlka,jlbc->bcak', B("ooov"), tau, alpha=0.25, out=wvvvo, beta=1.0)
+        ops.axpby(-0.5, B("ovvv"), 'jacb', 1.0, wvvvo, 'bcaj')
+        ops.contract('kbad,jkcd->bcaj', B("ovvv"), t2, out=wvvvo, beta=1.0)
+        G = ops.contract('menf,nf->me', B("oovv_ph"), t1)
+        E = ops.dot(fov, t1) + 0.25 * ops.dot(t2, B("oovv")) + 0.5 * ops.dot(t1, G)
 
         class _IMDS:
             pass

@@ -45,9 +45,8 @@ class Solver_CCSD(object):
         self.tsini = up(tsini, (o, v)) if tsini is not None else torch.zeros((o, v), dtype=torch.float64, device=dev)
         self.lsini = up(lsini, (o, v)) if lsini is not None else torch.zeros((o, v), dtype=torch.float64, device=dev)
         if tdini is None:                                  # MP2 start (Solver_GS.py:554-559), formed on the device
-            ops = mycc._dev_ops()
-            oovv = mycc._oovv
-            tdini = ops.denom(oovv, oovv)                  # oovv / (e_i - e_a + e_j - e_b), bare Fock (amp unused)
+            oovv = mycc.eris.block("oovv")
+            tdini = mycc.eris.ops.denom(oovv, oovv)       # oovv / (e_i - e_a + e_j - e_b), bare Fock (amp unused)
             ldini = tdini.clone()
         self.tdini = up(tdini, (o, o, v, v))
         self.ldini = up(ldini, (o, o, v, v)) if ldini is not None else self.tdini.clone()
@@ -115,7 +114,7 @@ class Solver_CCSD(object):
             adiis = DIIS()
             adiis.space, adiis.min_space = self.maxdiis, 2
         if 'tl' in diis:
-            tl_diis = DIIS(mycc._dev_ops())
+            tl_diis = DIIS(mycc.eris.ops)
             tl_diis.space, tl_diis.min_space = self.maxdiis, 2
         # a single density-matrix target (ecw_vexp_mat), structure-factor target (ecw_vexp_sf) or amplitude target
         # (ecw_vexp_sfobs) of our own Exp class is evaluated on the device: then nothing but scalars crosses PCIe inside

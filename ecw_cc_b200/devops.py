@@ -5,10 +5,11 @@ Torch only allocates the memory and provides the stream; every arithmetic
 operation is one of this repo's kernels.
 """
 import ctypes
+import weakref
 
 import numpy as np
 
-from ._lib import lib, EcwError
+from ._lib import lib
 
 
 class _TensorDesc(ctypes.Structure):
@@ -37,13 +38,63 @@ def _ref(d):
     return ctypes.byref(d) if d is not None else None
 
 
+class PinnedPool(object):
+    """Pinned host blocks for device -> host downloads (a pageable D2H runs at ~2.5 GB/s).  Page-locking gigabytes
+    costs far more than the transfer itself (cudaHostAlloc), so the block of a returned array of MIN_BYTES or more
+    goes back to the pool when the caller drops the array (per shape and dtype, at most DEPTH kept); smaller ones come
+    from torch's caching host allocator."""
+    MIN_BYTES = 1 << 20
+    DEPTH = 4
+
+    def __init__(self):
+        self._free = {}
+
+    def take(self, shape, dtype):
+        import torch
+        free = self._free.get((tuple(shape), dtype))
+        if free:
+            h = free.pop()
+            del free[self.DEPTH:]
+            return h
+        return torch.empty(shape, dtype=dtype, pin_memory=True)
+
+    def hand_out(self, h):
+        """numpy view of a filled block; a large block returns to the pool when the array is dropped."""
+        a = h.numpy()
+        if a.nbytes >= self.MIN_BYTES:
+            weakref.finalize(a, self._free.setdefault((tuple(h.shape), h.dtype), []).append, h)
+        return a
+
+
+class ArgBlocks(object):
+    """Persistent device argument blocks, name -> tensor.  A C entry point that always receives the same pointers
+    replays its CUDA graph (include/ecw_b200.h, ecw_ctx_set_graphs) instead of launching its kernels one by one."""
+
+    def __init__(self, device, **shapes):
+        import torch
+        self.blocks = {k: torch.empty(s, dtype=torch.float64, device=device) for k, s in shapes.items()}
+
+    def __getitem__(self, name):
+        return self.blocks[name]
+
+    def put(self, **named):
+        """Copy device tensors into the blocks of the same names (device to device); returns the blocks in order."""
+        out = []
+        for k, t in named.items():
+            b = self.blocks[k]
+            if t.data_ptr() != b.data_ptr():
+                b.copy_(t)
+            out.append(b)
+        return out
+
+
 class DevOps(object):
     def __init__(self, eris):
         import torch
         self.torch = torch
         self.e = eris
         self.dev = eris.device
-        self.launches = 0
+        self.pinned = PinnedPool()
 
     # -- memory -----------------------------------------------------------------
     def to_dev(self, x):
@@ -55,50 +106,32 @@ class DevOps(object):
     def empty(self, *shape):
         return self.torch.empty(shape, dtype=self.torch.float64, device=self.dev)
 
-    POOL_MIN_BYTES = 1 << 20    # larger downloads go through pooled pinned blocks (a pageable D2H runs at ~2.5 GB/s)
-    POOL_DEPTH = 3
-
     def to_host(self, t):
-        """device -> fresh numpy array.  Large results (the o^2v^2 intermediates Wbija / Wakic) are DMA'd into pinned
-        blocks that return to a per-shape pool when the caller drops the array, as in GCC._to_host."""
-        if t.numel() * 8 < self.POOL_MIN_BYTES:
-            return t.cpu().numpy()
-        import weakref
-        torch = self.torch
-        pool = self.__dict__.setdefault("_pool", {})
-        key = tuple(t.shape)
-        free = pool.setdefault(key, [])
-        if free:
-            h = free.pop()
-            del free[self.POOL_DEPTH:]
-        else:
-            h = torch.empty(key, dtype=torch.float64, pin_memory=True)
+        """device -> fresh numpy array in a pinned block of `self.pinned`."""
+        h = self.pinned.take(t.shape, t.dtype)
         h.copy_(t, non_blocking=True)
-        torch.cuda.current_stream(self.dev).synchronize()
-        a = h.numpy()
-        weakref.finalize(a, free.append, h)
-        return a
+        self.torch.cuda.current_stream(self.dev).synchronize()
+        return self.pinned.hand_out(h)
 
     def scalar(self, t):
         """Device scalar -> Python float (one synchronising D2H read)."""
         return float(t.cpu().reshape(-1)[0])
 
     # -- dispatch with workspace growth ---------------------------------------------
-    def _call(self, fn, *args):
+    def _launch(self, fn, *args):
+        """fn(ctx, *args, stream) -> rc; a call that needs more workspace than the context has (rc -2) is repeated
+        with the workspace grown to what the library asks for."""
         e = self.e
         if e._ws is None:
-            e._ws = self.torch.empty(1 << 20, dtype=self.torch.uint8, device=self.dev)
-            e.check(lib.ecw_set_workspace(e._h, e._ws.data_ptr(), e._ws.numel()), "ecw_set_workspace")
+            e.grow_workspace(1 << 20)
         rc = fn(e._h, *args, e.stream())
         if rc == -2:
-            need = int(lib.ecw_op_workspace_needed(e._h))
-            self.torch.cuda.current_stream(self.dev).synchronize()
-            e._ws = None
-            e._ws = self.torch.empty(max(need, 256) + 4096, dtype=self.torch.uint8, device=self.dev)
-            e.check(lib.ecw_set_workspace(e._h, e._ws.data_ptr(), e._ws.numel()), "ecw_set_workspace")
+            e.grow_workspace(max(int(lib.ecw_op_workspace_needed(e._h)), 256) + 4096)
             rc = fn(e._h, *args, e.stream())
-        e.check(rc, getattr(fn, "__name__", "ecw_op"))
-        self.launches += 1
+        return rc
+
+    def _call(self, fn, *args):
+        self.e.check(self._launch(fn, *args), getattr(fn, "__name__", "ecw_op"))
 
     # -- ops ---------------------------------------------------------------------------
     def contract(self, spec, A, B, alpha=1.0, out=None, beta=0.0):
@@ -114,21 +147,13 @@ class DevOps(object):
             beta = 0.0
         da, db, dc = _desc(A), _desc(B), _desc(out)
         args = (_scalar(alpha), _ref(da), sa.encode(), _ref(db), sb.encode(), _scalar(beta), _ref(dc), sc.encode())
-        self._call(lib.ecw_op_contract, *args)
         e = self.e
-        if e.int8_digits and e.int8_tol > 0.0 and 2.0 * A.numel() * B.numel() >= e.int8_min_flops >= 0.0:
+        if 2.0 * A.numel() * B.numel() >= e.int8_min_flops >= 0.0:
             # a contraction this large may have taken the INT8 route (2MNK <= 2|A||B|): accuracy guard (eris.py)
-            b = e.last_bound = e.int8_bound()
-            if b == b and b > e.int8_tol:
-                e.guard_trips += 1
-                if _scalar(beta) != 0.0:
-                    raise EcwError("ecw_op_contract: INT8 error bound %.2e > %.1e on an accumulating contraction; "
-                                   "use more digits (int8_digits) or gemm='dmma'" % (b, e.int8_tol))
-                e.check(lib.ecw_ctx_set_engine_override(e._h, 1), "ecw_ctx_set_engine_override")
-                try:
-                    self._call(lib.ecw_op_contract, *args)
-                finally:
-                    lib.ecw_ctx_set_engine_override(e._h, 0)
+            e.guarded(lambda: self._launch(lib.ecw_op_contract, *args), "ecw_op_contract",
+                      repeat=_scalar(beta) == 0.0)
+        else:
+            self._call(lib.ecw_op_contract, *args)
         return out
 
     def axpby(self, alpha, A, sa, beta, C, sc):
@@ -180,12 +205,16 @@ class DevOps(object):
                    _scalar(shift), _ref(do))
         return out
 
+    def dot_into(self, out, A, B, alpha=1.0, beta=1.0):
+        """out[0] = alpha * <A, B> + beta * out[0] on the device, without synchronising (out: one-element tensor)."""
+        da, db = _desc(A), _desc(B)
+        self._call(lib.ecw_op_dot, _scalar(alpha), _ref(da), _ref(db), _scalar(beta), ctypes.c_void_p(out.data_ptr()))
+        return out
+
     def dot(self, A, B, alpha=1.0):
         """alpha * <A, B> as a Python float."""
         out = self.torch.zeros(1, dtype=self.torch.float64, device=self.dev)
-        da, db = _desc(A), _desc(B)
-        self._call(lib.ecw_op_dot, _scalar(alpha), _ref(da), _ref(db), 0.0, ctypes.c_void_p(out.data_ptr()))
-        return self.scalar(out)
+        return self.scalar(self.dot_into(out, A, B, alpha, 0.0))
 
     def trace(self, M):
         """sum_i M[i,i] through the dot kernel (diagonal view x ones)."""

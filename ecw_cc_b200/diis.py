@@ -14,12 +14,7 @@ Gram matrix are projected out).  PySCF itself is outside the reference tree: DII
 restatement in oracle/pyscf_stub and to the fixed point of the plain iteration, not to PySCF ("parity unpinned").
 HBM need on the device: (2*space + 1) vectors — 2*(ov + o^2v^2) doubles each; choose `maxdiis` accordingly.
 """
-import ctypes
-
 import numpy as np
-
-from ._lib import lib
-from .devops import _desc, _ref
 
 
 def solve_coefficients(h):
@@ -98,10 +93,8 @@ class _DeviceStore(object):
         ops = self.ops
         ops.fill(self.gram, 0.0)
         for i in range(nd):
-            out = ctypes.c_void_p(self.gram.data_ptr() + 8 * i)
             for a, b in zip(self._segments(self.e[slot]), self._segments(self.e[i])):
-                da, db = _desc(a), _desc(b)
-                ops._call(lib.ecw_op_dot, 1.0, _ref(da), _ref(db), 1.0, out)
+                ops.dot_into(self.gram[i:i + 1], a, b)
         return self.gram[:nd].cpu().numpy()                      # nd doubles: the only D2H of an update
 
     def combine(self, c):

@@ -8,6 +8,7 @@ molecule (PySCF ao2mo, Eris.py:47-128) is out of scope.
 """
 import ctypes
 import os
+import weakref
 
 import numpy as np
 
@@ -16,6 +17,7 @@ from ._lib import lib, EcwError
 _LAYOUTS = ("oooo", "ooov", "oovv", "ovvv", "oovv_ph", "ovov_ph", "oooo_p", "oovv_p", "ovvv_p", "vvvv_p")
 SYNTH_KIND = dict(oooo=0, ooov=1, oovv=2, oovv_ph=3, ovov_ph=4, ovvv=5, oooo_p=6, oovv_p=7, ovvv_p=8, vvvv_p=9,
                   fock=10, fsp=11, t1=12, l1=13, t2=14, l2=15)
+_BLOCK_INDEX = dict(oooo="oooo", ooov="ooov", oovv="oovv", ovvv="ovvv", ovov_ph="ovov", oovv_ph="ovov")
 
 
 # GEMM engine of the contraction plans (include/ecw_b200.h, ecw_ctx_set_gemm):
@@ -114,9 +116,11 @@ class DeviceEris(object):
         self.use_ovvv_planes = bool(ovvv_planes and self.int8_digits and self.nocc % 8 == 0 and self.nvir % 8 == 0)
         self.int8_tol = float(os.environ.get("ECW_INT8_TOL", INT8_TOL) if int8_tol is None else int8_tol)
         self.guard_trips = 0      # calls whose INT8 error bound exceeded int8_tol (each was repeated on DMMA)
-        self.last_bound = 0.0     # bound of the last guarded call / the largest one seen so far
-        self.max_bound = 0.0
+        self.last_bound = 0.0     # bound of the last guarded call (a plan or a primitive contraction)
+        self.max_bound = 0.0      # the largest finite bound of those calls that stayed within int8_tol
         self.buf = {}
+        self._views = {}          # block(): shaped views of the canonical integral blocks
+        self._ops = None
         self._ws = None
         self._scal = torch.zeros(16, dtype=torch.float64, device=self.device)
         self._bind("scal", self._scal)
@@ -155,15 +159,23 @@ class DeviceEris(object):
         self._bind(name, t)
         return t
 
-    def ensure_workspace(self, func, flags):
+    def grow_workspace(self, nbytes):
+        """Give the context a workspace of at least `nbytes` (never shrinks).  The stream is synchronised before the
+        old buffer is dropped: work already enqueued may still read it."""
+        if self._ws is not None and self._ws.numel() >= nbytes:
+            return
         torch = _torch()
+        if self._ws is not None:
+            torch.cuda.current_stream(self.device).synchronize()
+        self._ws = None
+        self._ws = torch.empty(int(nbytes), dtype=torch.uint8, device=self.device)
+        self.check(lib.ecw_set_workspace(self._h, self._ws.data_ptr(), self._ws.numel()), "ecw_set_workspace")
+
+    def ensure_workspace(self, func, flags):
         need = lib.ecw_workspace_bytes(self._h, func.encode(), flags)
         if need < 0:
             self.check(-1, "ecw_workspace_bytes(%s)" % func)
-        if self._ws is None or self._ws.numel() < need:
-            self._ws = None
-            self._ws = torch.empty(max(int(need), 256), dtype=torch.uint8, device=self.device)
-            self.check(lib.ecw_set_workspace(self._h, self._ws.data_ptr(), self._ws.numel()), "ecw_set_workspace")
+        self.grow_workspace(max(int(need), 256))
 
     def run(self, rc, what):
         """Drive a (possibly distributed) call to completion: while the library reports a pending
@@ -228,9 +240,19 @@ class DeviceEris(object):
         return "vvvv_p" in self.buf and "ovvv_p" in self.buf
 
     def execute(self, func, flags, launch, what):
-        """ensure_workspace + launch() (a closure around the C entry point, returns its rc) + the INT8 accuracy
-        guard: when the bound of the call exceeds int8_tol the same call is repeated without the INT8 route."""
-        self.ensure_workspace(func, flags)
+        """One plan call: `launch` (a closure around the C entry point) through `guarded`, with the workspace sized
+        for the plan of `func` / `flags` before every launch."""
+        self.guarded(launch, what, prepare=lambda: self.ensure_workspace(func, flags))
+
+    def guarded(self, launch, what, prepare=None, repeat=True):
+        """prepare() + launch() (a closure around a C entry point, returns its rc) + the INT8 accuracy guard: when the
+        bound of the call exceeds int8_tol the same call is repeated without the INT8 route.  repeat=False: the call
+        accumulates into its output (beta != 0), so a repeat would count its product twice; it raises instead.  A plan
+        call (the calls with a prepare step) reads the FP64 integral layouts when it runs on DMMA: without them it
+        raises too.  The primitive contractions only guard calls large enough for the INT8 route (DevOps.contract):
+        on a sharded context reading the bound is a collective."""
+        if prepare is not None:
+            prepare()
         self.run(launch(), what)
         if not self.int8_digits or not self.int8_tol > 0.0:
             return
@@ -239,14 +261,18 @@ class DeviceEris(object):
             self.max_bound = max(self.max_bound, b) if b == b else self.max_bound
             return
         self.guard_trips += 1
-        if not self.can_dmma():
+        if not repeat:
+            raise EcwError("%s: INT8 error bound %.2e > %.1e on an accumulating contraction; use more digits "
+                           "(int8_digits) or gemm='dmma'" % (what, b, self.int8_tol))
+        if prepare is not None and not self.can_dmma():
             raise EcwError("%s: the INT8 engine cannot guarantee its accuracy for these operands (worst-case error "
                            "bound %.2e > %.1e with %d digits) and the FP64 integral layouts are not on the device: "
                            "build the container with int8_digits=%d or gemm='dmma'"
                            % (what, b, self.int8_tol, self.int8_digits, min(self.int8_digits + 1, 8)))
         self.check(lib.ecw_ctx_set_engine_override(self._h, 1), "ecw_ctx_set_engine_override")
         try:
-            self.ensure_workspace(func, flags)
+            if prepare is not None:
+                prepare()
             self.run(launch(), what + " (FP64 DMMA after the INT8 guard)")
         finally:
             lib.ecw_ctx_set_engine_override(self._h, 0)
@@ -407,26 +433,43 @@ class DeviceEris(object):
             raise EcwError("ecw_synth_tensor(%s) failed" % kind)
         return out
 
-    # -- reference attribute surface (host views on demand) ----------------------
-    def _host(self, name, shape):
-        return self.buf[name][: int(np.prod(shape))].reshape(shape).cpu().numpy()
+    # -- device views, the primitive ops, the Fock blocks ---------------------------
+    def block(self, name):
+        """Device view of a canonical integral block in its index shape (ovov_ph / oovv_ph: [ia, jb] as (o, v, o, v))."""
+        t = self._views.get(name)
+        if t is None:
+            shape = tuple(self.nocc if c == "o" else self.nvir for c in _BLOCK_INDEX[name])
+            t = self._views[name] = self.buf[name][: int(np.prod(shape))].view(shape)
+        return t
 
     @property
+    def ops(self):
+        """The primitive device ops of this context (one DevOps, shared by every class built on it)."""
+        if self._ops is None:
+            from .devops import DevOps
+            self._ops = DevOps(weakref.proxy(self))    # no reference cycle: the context is freed with its last owner
+        return self._ops
+
+    def fock_blocks(self, fsp=None):
+        """oo, ov, vo, vv views of the device one-body operator: fsp (uploaded when it is a host array) or the Fock
+        matrix."""
+        o = self.nocc
+        F = self.fock_dev if fsp is None else self.ops.to_dev(fsp)
+        return F[:o, :o], F[:o, o:], F[o:, :o], F[o:, o:]
+
+    # -- reference attribute surface (host copies on demand) ----------------------
+    @property
     def oovv(self):
-        o, v = self.nocc, self.nvir
-        return self._host("oovv", (o, o, v, v))
+        return self.block("oovv").cpu().numpy()
 
     @property
     def ooov(self):
-        o, v = self.nocc, self.nvir
-        return self._host("ooov", (o, o, o, v))
+        return self.block("ooov").cpu().numpy()
 
     @property
     def oooo(self):
-        o = self.nocc
-        return self._host("oooo", (o, o, o, o))
+        return self.block("oooo").cpu().numpy()
 
     @property
     def ovvv(self):
-        o, v = self.nocc, self.nvir
-        return self._host("ovvv", (o, v, v, v))
+        return self.block("ovvv").cpu().numpy()
