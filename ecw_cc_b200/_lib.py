@@ -5,8 +5,8 @@ import subprocess
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libecw_b200.so")
-_SRC = ["gemm.cu", "gemm_tma.cu", "ewise.cu", "ozaki.cu", "synth.cu", "ftao.cu", "maps.cu", "capi.cu", "plan.cpp", "ccsd_plan.cpp",
-        "ccsd_plan_slab.cpp", "ccs_plan.cpp"]
+_SRC = ["gemm.cu", "gemm_tma.cu", "ewise.cu", "ozaki.cu", "synth.cu", "ftao.cu", "maps.cu", "capi.cu", "exec.cu", "plan.cpp",
+        "ccsd_plan.cpp", "ccsd_plan_slab.cpp", "ccs_plan.cpp"]
 
 ECW_HAS_ALPHA = 1
 ECW_EQUATION = 2
@@ -22,7 +22,8 @@ def build(force=False, verbose=False):
     """Compile the CUDA library in-tree for sm_100a (nvcc cross-compiles without a GPU).
     One object per source under csrc/build/ (recompiled only when stale), then one link."""
     csrc = os.path.join(_HERE, "csrc")
-    hdrs = [os.path.join(csrc, h) for h in ("plan.h", "kernels.h", "ccsd_plan.h", "ccsd_plan_detail.h")]
+    hdrs = [os.path.join(csrc, h) for h in ("plan.h", "kernels.h", "ccsd_plan.h", "ccsd_plan_detail.h", "exec.h",
+                                            "ozaki_layout.h")]
     hdrs.append(os.path.join(_HERE, "..", "include", "ecw_b200.h"))
     hdr_mt = max(os.path.getmtime(h) for h in hdrs)
     nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")

@@ -42,8 +42,7 @@ struct Slots {
     ovvv_p = make_tensor(S_OVVV_P, 0, {o, v, pv});
     ovvv_p2 = make_tensor(S_OVVV_P, 0, {o * v, pv});
     nshmax = (pv + world - 1) / world;
-    n0 = std::min<int64_t>(pv, (int64_t)rank * nshmax);
-    nsh = std::min<int64_t>(pv, n0 + nshmax) - n0;
+    shard_range(pv, rank, world, &n0, &nsh);
     vvvv_p = make_tensor(S_VVVV_P, 0, {nsh, pv});   // local shard (all of it when world == 1)
   }
 };
@@ -87,7 +86,8 @@ inline void emit_wovvo_rows(Plan& P, const Slots& s, const Tensor& t1, const Ten
 // whole Wph, rows distributed over the ranks and all-gathered once
 inline void emit_wovvo(Plan& P, const Slots& s, const Tensor& t1, const Tensor& t2x, double c2, const Tensor& Wph) {
   const int64_t L = s.o, chunk = P.lead_chunk(L);
-  const int64_t m0 = std::min<int64_t>(L, (int64_t)P.rank * chunk), nm = std::min<int64_t>(L, m0 + chunk) - m0;
+  int64_t m0, nm;
+  P.my_range(L, &m0, &nm);
   if (P.world == 1) {
     emit_wovvo_rows(P, s, t1, t2x, c2, Wph, 0, L);
     return;
@@ -190,8 +190,8 @@ inline void ladder_dist(Plan& P, const Slots& s, const Tensor& X, const Tensor& 
   }
   P.allgather(accL, rows * s.nshmax, G, note);
   for (int r = 0; r < s.world; ++r) {
-    const int64_t c0 = std::min<int64_t>(s.pv, (int64_t)r * s.nshmax);
-    const int64_t nc = std::min<int64_t>(s.pv, c0 + s.nshmax) - c0;
+    int64_t c0, nc;
+    shard_range(s.pv, r, s.world, &c0, &nc);
     if (nc <= 0) continue;
     Tensor src = make_tensor(G.slot, G.off + (int64_t)r * rows * s.nshmax, {rows, nc});
     src.str[0] = s.nshmax;

@@ -3,6 +3,8 @@
 #include <cuda_runtime.h>
 #include <cstdint>
 
+#include "ozaki_layout.h"
+
 namespace ecw {
 
 struct GemmArgs {
@@ -26,10 +28,7 @@ cudaError_t launch_gemm_tma(const GemmArgs& a, cudaStream_t st, int cfg);
 // FP64 GEMM by error-free splitting on the INT8 tcgen05 tensor pipe (ozaki.cu).
 // An operand X[R,K] (element (r,k) at X[r*rs + k*ks], one of rs/ks == 1) is cut into `ns` int8 digit
 // planes (ozaki_plane_bytes) plus row statistics `scale` = [2^e scales | row sums / scale], each
-// ozaki_padded_rows doubles long.
-int ozaki_tile_n(int ns);
-int64_t ozaki_padded_rows(int64_t R);
-int64_t ozaki_plane_bytes(int64_t R, int64_t K, int ns);
+// ozaki_padded_rows doubles long (sizes: ozaki_layout.h).
 // row0/total_rows: X holds rows [row0, row0+R) of an operand of total_rows rows whose plane set is cut chunk
 // by chunk (row0 a multiple of 128; every chunk but the last a multiple of 128 rows)
 cudaError_t launch_ozaki_split(const double* X, int64_t R, int64_t K, int64_t rs, int64_t ks, int ns, int8_t* planes,
@@ -38,9 +37,6 @@ cudaError_t launch_ozaki_split(const double* X, int64_t R, int64_t K, int64_t rs
 // to a multiple of 32 per k1 (k-block index k1*ceil(K2/32) + k2/32), and the statistics also hold the row sums per k1:
 // stats = [scales | row sums | row sums of k1 = 0 | ... ] (ozaki_stat_elems doubles).  A contiguous range of k1
 // values of such a plane set is itself a valid operand (OzBatch::*_kb0/_kbb/_t0/_tb).
-int64_t ozaki_kblocks(int64_t K1, int64_t K2);
-int64_t ozaki_plane_bytes2(int64_t R, int64_t K1, int64_t K2, int ns);
-int64_t ozaki_stat_elems(int64_t R, int64_t K1);
 cudaError_t launch_ozaki_split2(const double* X, int64_t R, int64_t K1, int64_t K2, int64_t rs, int64_t ks1, int64_t ks2,
                                 int ns, int8_t* planes, double* stats, cudaStream_t st, int64_t row0 = 0,
                                 int64_t total_rows = 0);

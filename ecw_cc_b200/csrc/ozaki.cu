@@ -52,8 +52,6 @@ namespace ecw {
 
 namespace {
 
-constexpr int OZ_BK = 32;        // k per stage = K of one kind::i8 MMA
-constexpr int OZ_TM = 128;       // tile rows  (MMA M)
 // int32 accumulators are drained to FP64 every oz_kflush(NS) k.  The accumulator of weight NS-1 sums NS digit products
 // per k, each at most 128 * 128 = 2^14 in magnitude: NS * K * 2^14 < 2^31 needs K < 2^17 / NS.  8192 keeps a factor of
 // two of headroom for every digit count (16384 is admissible up to seven digits and was measured: no gain — the drain
@@ -141,9 +139,6 @@ struct OzGemmParams {
   // batch b = 0..batch-1 of independent products (OzBatch, kernels.h)
   OzBatch bt;
 };
-
-// tile columns: NS accumulators of TN int32 columns must fit the 512 TMEM columns; every MMA needs N % 16 == 0
-template <int NS> struct OzTile { static constexpr int TN = NS <= 5 ? 96 : (NS == 6 ? 80 : 64); };
 
 template <int NS, int TN>
 struct OzCfg {
@@ -602,26 +597,10 @@ cudaError_t launch_gemm_ns_tn(OzGemmParams p, cudaStream_t st, int sm_count) {
 }
 template <int NS>
 cudaError_t launch_gemm_ns(OzGemmParams p, cudaStream_t st, int sm_count) {
-  return launch_gemm_ns_tn<NS, OzTile<NS>::TN>(p, st, sm_count);
+  return launch_gemm_ns_tn<NS, ozaki_tile_n(NS)>(p, st, sm_count);
 }
 
 }  // namespace
-
-int ozaki_tile_n(int ns) {
-  switch (ns) {
-    case 3: return OzTile<3>::TN; case 4: return OzTile<4>::TN; case 5: return OzTile<5>::TN;
-    case 6: return OzTile<6>::TN; case 7: return OzTile<7>::TN; case 8: return OzTile<8>::TN;
-  }
-  return 64;
-}
-int64_t ozaki_padded_rows(int64_t R) { return (R + 127) / 128 * 128; }
-int64_t ozaki_kblocks(int64_t K1, int64_t K2) { return K1 * ((K2 + OZ_BK - 1) / OZ_BK); }
-// + one tile of slack: the last tile of the last slab may start inside the padded rows and run past them
-int64_t ozaki_plane_bytes2(int64_t R, int64_t K1, int64_t K2, int ns) {
-  return ozaki_padded_rows(R) * ozaki_kblocks(K1, K2) * OZ_BK * ns + 4096;
-}
-int64_t ozaki_plane_bytes(int64_t R, int64_t K, int ns) { return ozaki_plane_bytes2(R, 1, K, ns); }
-int64_t ozaki_stat_elems(int64_t R, int64_t K1) { return (K1 > 1 ? 2 + K1 : 2) * ozaki_padded_rows(R); }
 
 cudaError_t launch_ozaki_split2(const double* X, int64_t R, int64_t K1, int64_t K2, int64_t rs, int64_t ks1, int64_t ks2,
                                 int ns, int8_t* planes, double* stats, cudaStream_t st, int64_t row0, int64_t total_rows) {

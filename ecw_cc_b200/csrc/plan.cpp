@@ -873,14 +873,6 @@ void Plan::contract(double alpha, const Tensor& A, const char* sa, const Tensor&
 }
 
 // ---------------------------------------------------------------- INT8-pipe GEMM
-// sizes mirror ozaki.cu (ozaki_padded_rows / ozaki_plane_bytes2 / ozaki_stat_elems / ozaki_tile_n); this file stays
-// CUDA-free
-static int64_t oz_pad_rows(int64_t r) { return (r + 127) / 128 * 128; }
-static int64_t oz_plane_elems(int64_t R, int64_t K1, int64_t K2, int ns) {
-  return (oz_pad_rows(R) * K1 * ((K2 + 31) / 32 * 32) * ns + 4096 + 7) / 8;
-}
-static int64_t oz_stat_elems(int64_t R, int64_t K1) { return (K1 > 1 ? 2 + K1 : 2) * oz_pad_rows(R); }
-static int oz_tile_n(int ns) { return ns <= 5 ? 96 : (ns == 6 ? 80 : 64); }
 
 // Seconds (model) of one INT8-route GEMM for both role assignments; tile = 128 rows of the first operand x TN rows
 // of the second.  Main loop: padded product at ~100 TFLOP/s FP64-equivalent for 7 digits (scaled by the digit-pair
@@ -889,7 +881,7 @@ static int oz_tile_n(int ns) { return ns <= 5 ? 96 : (ns == 6 ? 80 : 64); }
 static double oz_time(int ns, int sm_count, int64_t M, int64_t N, int64_t K, int64_t crs, int64_t ccs, double beta,
                       bool* swap_out, int64_t splits) {
   auto pad = [](int64_t x, int64_t g) { return (x + g - 1) / g * g; };
-  const int TN = oz_tile_n(ns);
+  const int TN = ozaki_tile_n(ns);
   const double rate = 1.0e14 * 28.0 / (0.5 * ns * (ns + 1));
   double best = 1e300;
   for (int sw = 0; sw < 2; ++sw) {
@@ -908,7 +900,7 @@ static double oz_time(int ns, int sm_count, int64_t M, int64_t N, int64_t K, int
 // chunk, partial results summed by a reduce op).  S = the divisor of K/32 up to 64 that fills the SMs best.
 static int64_t oz_pick_splits(int ns, int sm_count, int64_t M, int64_t N, int64_t K, int64_t min_k) {
   auto pad = [](int64_t x, int64_t g) { return (x + g - 1) / g * g; };
-  const int TN = oz_tile_n(ns);
+  const int TN = ozaki_tile_n(ns);
   const int64_t tiles = std::min((pad(M, 128) / 128) * (pad(N, TN) / TN), (pad(N, 128) / 128) * (pad(M, TN) / TN));
   if (min_k <= 0 || K < min_k || K % 32 != 0 || tiles * 2 > sm_count) return 1;
   int64_t best = 1;
@@ -1028,8 +1020,8 @@ OzSet Plan::oz_cut(const Tensor& X, int64_t R, int64_t rs, int64_t K1, int64_t k
   s.R = R; s.K1 = K1; s.K2 = K2;
   s.owned = !cacheable;
   s.cached = cacheable;
-  s.planes = tmp({oz_plane_elems(R, K1, K2, oz_ns)});
-  s.stats = tmp({oz_stat_elems(R, K1)});
+  s.planes = tmp({ozaki_plane_elems(R, K1, K2, oz_ns)});
+  s.stats = tmp({ozaki_stat_elems(R, K1)});
   Op sp;
   sp.kind = OP_OZ_SPLIT;
   sp.a = X;
@@ -1075,24 +1067,24 @@ OzSet Plan::oz_const_vvvv(int64_t rows) const {
   const int64_t pv = npair(nvir);
   OzSet s;
   s.R = rows; s.K1 = 1; s.K2 = pv;
-  s.planes = make_tensor(S_VVVV_OZ, 0, {oz_plane_elems(rows, 1, pv, oz_ns)});
-  s.stats = make_tensor(S_VVVV_OZS, 0, {oz_stat_elems(rows, 1)});
+  s.planes = make_tensor(S_VVVV_OZ, 0, {ozaki_plane_elems(rows, 1, pv, oz_ns)});
+  s.stats = make_tensor(S_VVVV_OZS, 0, {ozaki_stat_elems(rows, 1)});
   return s;
 }
 OzSet Plan::oz_const_ovvv1() const {
   const int64_t pv = npair(nvir);
   OzSet s;
   s.R = nocc * nvir; s.K1 = 1; s.K2 = pv;
-  s.planes = make_tensor(S_OVVV_OZ1, 0, {oz_plane_elems(s.R, 1, pv, oz_ns)});
-  s.stats = make_tensor(S_OVVV_OZ1S, 0, {oz_stat_elems(s.R, 1)});
+  s.planes = make_tensor(S_OVVV_OZ1, 0, {ozaki_plane_elems(s.R, 1, pv, oz_ns)});
+  s.stats = make_tensor(S_OVVV_OZ1S, 0, {ozaki_stat_elems(s.R, 1)});
   return s;
 }
 OzSet Plan::oz_const_ovvv2() const {
   const int64_t pv = npair(nvir);
   OzSet s;
   s.R = pv; s.K1 = nocc; s.K2 = nvir;
-  s.planes = make_tensor(S_OVVV_OZ2, 0, {oz_plane_elems(pv, nocc, nvir, oz_ns)});
-  s.stats = make_tensor(S_OVVV_OZ2S, 0, {oz_stat_elems(pv, nocc)});
+  s.planes = make_tensor(S_OVVV_OZ2, 0, {ozaki_plane_elems(pv, nocc, nvir, oz_ns)});
+  s.stats = make_tensor(S_OVVV_OZ2S, 0, {ozaki_stat_elems(pv, nocc)});
   return s;
 }
 
@@ -1190,10 +1182,16 @@ static void dump_tensor(std::ostringstream& o, const char* key, const Tensor& t)
   o << "]}";
 }
 
+const char* op_kind_name(int kind) {
+  static const char* names[] = {"gemm", "reduce", "permute", "fill", "tau", "pack", "unpack", "finish",
+                                "dot", "scale_dev", "diag_add", "rdm1", "ewise", "allgather", "oz_split", "oz_gemm",
+                                "asym4", "alltoall"};
+  static_assert(sizeof(names) / sizeof(names[0]) == OP_ALLTOALL + 1, "one name per OpKind");
+  if (kind < 0 || kind > OP_ALLTOALL) return "?";
+  return names[kind];
+}
+
 std::string Plan::dump_json() const {
-  static const char* kn[] = {"gemm", "reduce", "permute", "fill", "tau", "pack", "unpack", "finish",
-                             "dot", "scale_dev", "diag_add", "rdm1", "ewise", "allgather", "oz_split", "oz_gemm",
-                             "asym4", "alltoall"};
   std::ostringstream o;
   o.precision(17);
   o << "{\"workspace_elems\":" << arena.peak << ",\"gemm_flops\":" << gemm_flops << ",\"oz_flops\":" << oz_flops
@@ -1201,7 +1199,7 @@ std::string Plan::dump_json() const {
   for (size_t i = 0; i < ops.size(); ++i) {
     const Op& p = ops[i];
     if (i) o << ",";
-    o << "\n{\"kind\":\"" << kn[p.kind] << "\",";
+    o << "\n{\"kind\":\"" << op_kind_name(p.kind) << "\",";
     dump_tensor(o, "a", p.a); o << ",";
     dump_tensor(o, "b", p.b); o << ",";
     dump_tensor(o, "c", p.c); o << ",";

@@ -17,6 +17,8 @@
 #include <stdexcept>
 #include <algorithm>
 
+#include "ozaki_layout.h"
+
 namespace ecw {
 
 constexpr int MAXD = 6;
@@ -40,6 +42,21 @@ enum Slot : int {
   S_COUNT
 };
 const char* slot_name(int s);
+
+// the device scalars of slot S_SCAL
+enum Scalar : int {
+  SC_RESULT = 0,        // the scalar result of a plan (energy-like), copied out by the entry points
+  SC_DOT = 1,           // ecw_op_dot
+  SC_INT8_BOUND = 15,   // run-time error bound of the INT8-route products of the last call (ecw_int8_error_bound)
+  SC_COUNT = 16
+};
+
+// this rank's part [*i0, *i0 + *ni) of an index of extent L that is distributed in chunks of ceil(L / world)
+inline void shard_range(int64_t L, int rank, int world, int64_t* i0, int64_t* ni) {
+  const int64_t ch = (L + world - 1) / world;
+  *i0 = std::min<int64_t>(L, (int64_t)rank * ch);
+  *ni = std::min<int64_t>(L, *i0 + ch) - *i0;
+}
 
 struct Tensor {
   int slot = -1;
@@ -79,6 +96,7 @@ enum OpKind : int {
   OP_ASYM4,       // c[ijab] = alpha b[ijab] + a[ijab] - a[jiab] - a[ijba] + a[jiba] + beta c[ijab]  (b may be unset)
   OP_ALLTOALL,    // collective: block q (i0 elements) of `a` goes to rank q; block q of `c` comes from rank q
 };
+const char* op_kind_name(int kind);
 
 struct Op {
   int kind = 0;
@@ -102,8 +120,8 @@ struct OzSet {
   int64_t R = 0, K1 = 1, K2 = 0;
   bool owned = false;          // lives in the workspace arena and is released by oz_release
   bool cached = false;         // lives in the workspace arena, owned by the cut cache of the plan
-  int64_t rp() const { return (R + 127) / 128 * 128; }
-  int64_t nkb2() const { return (K2 + 31) / 32; }
+  int64_t rp() const { return ozaki_padded_rows(R); }
+  int64_t nkb2() const { return ozaki_kblocks(1, K2); }
 };
 // The part of a plane set one product of a batch reads: rows [row0 + b*rowb, +M|N), k1 values [k10 + b*k1b, +nk1)
 // (nk1 = K1: the whole contraction index; otherwise nk1 must be 1).
@@ -154,11 +172,7 @@ class Plan {
   // bit-identical replicas).  world == 1: C += part.
   void sum_ranks_add(const Tensor& part, const Tensor& C, const char* note = "");
   // this rank's range of an index of extent L that is distributed in chunks of lead_chunk(L)
-  void my_range(int64_t L, int64_t* i0, int64_t* ni) const {
-    const int64_t ch = lead_chunk(L);
-    *i0 = std::min<int64_t>(L, (int64_t)rank * ch);
-    *ni = std::min<int64_t>(L, *i0 + ch) - *i0;
-  }
+  void my_range(int64_t L, int64_t* i0, int64_t* ni) const { shard_range(L, rank, world, i0, ni); }
   // C (contiguous) += alpha * sum_K A.B with the range of the contracted label `lab` split across ranks
   // (partial sums are all-gathered and added in rank order on every rank: bit-identical replicas)
   void contract_split(double alpha, const Tensor& A, const char* sa, const Tensor& B, const char* sb,
